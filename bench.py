@@ -2,6 +2,7 @@
 """bench.py — self-play hot path throughput on B200 (contract: see the task statement / DESIGN.md §Measurement).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload selfplay|perft|tree]
+                    [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[2]: 8x8 Othello self-play, 100 sims/move, 4096 concurrent games per GPU,
 random-init OthelloNNet (C=512) evaluated in bf16 on the tcgen05 tower.  One "step" = 100 engine steps (one tree
@@ -204,14 +205,44 @@ def l2_bandwidth(E, device, mb=32, passes=50):
     return {"read_gbs": best, "what": f"oz_probe_l2_read: {passes} sweeps of 16-byte .cg loads over a {mb} MB L2-resident buffer, best of 3"}
 
 
+DUMP_MAX_BYTES = 60 << 20   # --dump-outputs stays under 64 MB, .npy headers included
+
+
+def bits64(a):
+    """uint64 bitboards -> float64 [..., 2]: the low and the high 32 bits, each exact in float64."""
+    a = np.asarray(a, dtype=np.uint64)
+    return np.stack([a & np.uint64(0xFFFFFFFF), a >> np.uint64(32)], axis=-1).astype(np.float64)
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array of `arrays` (float32 / float64, one row per game) as out_dir/<name>.npy, plus row_index.npy:
+    the game index of every row.  When all of it exceeds DUMP_MAX_BYTES, the same fixed, seeded sample of games is kept
+    in every array."""
+    rows = len(next(iter(arrays.values())))
+    per_row = sum(a.nbytes for a in arrays.values()) / max(1, rows) + 8
+    keep = min(rows, int(DUMP_MAX_BYTES // per_row))
+    idx = np.arange(rows) if keep == rows else np.sort(np.random.default_rng(0).choice(rows, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in dict(arrays, row_index=np.arange(rows, dtype=np.float64)).items():
+        assert a.dtype in (np.float32, np.float64) and len(a) == rows, name
+        np.save(os.path.join(out_dir, name + ".npy"), a[idx])
+
+
+def selfplay_arrays(rec, rows):
+    """The first `rows` games' self-play records (engine.Engine.selfplay_records) as float arrays."""
+    return {"black": bits64(rec["black"][:rows]), "white": bits64(rec["white"][:rows]),
+            **{k: rec[k][:rows].astype(np.float32) for k in ("action", "player", "n_moves", "winner")}}
+
+
 class Ctx:
     pass
 
 
-def selfplay_leg(cx, *, games, sims, vl, cache_log2, window, steps, warmup, mode):
+def selfplay_leg(cx, *, games, sims, vl, cache_log2, window, steps, warmup, mode, dump_dir=None):
     """One timed leg of the self-play hot path: `steps` x (STEPS_PER_MOVE engine steps) with `games` slots in flight.
     window = "steady": slots start at every game phase and finished slots take queued games (steady-state mix);
-             "opening": every game starts within its first 8 plies (round 1's default window)."""
+             "opening": every game starts within its first 8 plies (round 1's default window).
+    dump_dir: where rank 0 writes the records of the job's first generation of games, each played to its end."""
     torch, dist, E, oznet, args = cx.torch, cx.dist, cx.E, cx.oznet, cx.args
     n, C, G = 8, args.channels, games
     spm = (sims + max(1, vl) - 1) // max(1, vl)
@@ -273,6 +304,16 @@ def selfplay_leg(cx, *, games, sims, vl, cache_log2, window, steps, warmup, mode
             c1 = eng.counters()
         l1 = eng.launches()
         lt = eng.layer_times() if mode == E.PRIOR_NET else np.zeros(8, dtype=np.float32)
+        if dump_dir and cx.rank == 0:
+            rows = total
+            if not tree_only:
+                # how far a game has got when the timed steps end varies by a move from run to run, so the records are
+                # not comparable then; the job's first generation (the games that started in the G slots) is played on,
+                # untimed, until each of its games has ended - at most one game's length, whatever --steps is
+                rows = min(G, total)
+                while (eng.selfplay_records()["winner"][:rows] < 0).any() and eng.selfplay_run(spm) > 0:
+                    pass
+            dump_outputs(dump_dir, selfplay_arrays(eng.selfplay_records(), rows))
         d = {k: c1[k] - c0[k] for k in zero}
         d_evals = d["nodes"] - d["cache_hits"] - d["cache_aliases"]   # positions that actually went through the network
         t = torch.tensor([ms, d["sims"], d_evals, d["moves"], l1 - l0, d["cache_hits"], d["cache_aliases"]],
@@ -373,7 +414,7 @@ def run_ours(args):
         torch.cuda.synchronize()
 
     if args.workload == "perft":
-        line = perft_leg(args, E, peaks, rank, world, local, barrier, args.steps, args.warmup)
+        line = perft_leg(args, E, peaks, rank, world, local, barrier, args.steps, args.warmup, dump_dir=args.dump_outputs)
         if world > 1:
             dist.barrier(); dist.destroy_process_group()
         if rank == 0:
@@ -400,7 +441,7 @@ def run_ours(args):
         cx.l2 = l2_bandwidth(E, local)
     tree_only = mode == E.PRIOR_HASH
     leg = selfplay_leg(cx, games=G, sims=sims, vl=args.vl, cache_log2=args.eval_cache_log2, window=args.window,
-                       steps=args.steps, warmup=args.warmup, mode=mode)
+                       steps=args.steps, warmup=args.warmup, mode=mode, dump_dir=args.dump_outputs)
     ms = leg["ms"]
     sims_per_s = leg["sims"] / (ms / 1e3)
 
@@ -592,9 +633,10 @@ def perft_cpu_sample(games_per_proc=4000, procs=None):
                        f"restatement: {plies} plies in {wall:.1f}s")
 
 
-def perft_leg(args, E, peaks, rank, world, local, barrier, steps, warmup):
+def perft_leg(args, E, peaks, rank, world, local, barrier, steps, warmup, dump_dir=None):
     """configs[1]: random-playout perft, 1M concurrent games per launch.  Returns the JSON line as a dict (rank 0) after the
-    max/sum over ranks; the caller owns the process group."""
+    max/sum over ranks; the caller owns the process group.  dump_dir: where rank 0 writes the final positions of the last
+    timed launch's games."""
     import ctypes as C
     import torch
     n_games = args.games if args.games > 4096 else (1 << 20)
@@ -637,6 +679,12 @@ def perft_leg(args, E, peaks, rank, world, local, barrier, steps, warmup):
     for i in range(steps):
         launch(100 + i)
         plies += int((info & 0xFF).sum().item())
+    if dump_dir and rank == 0:
+        # the loop above ended with the last timed launch's seed
+        fields = E.decode_perft_info(info.cpu().numpy().view(np.uint32))
+        dump_outputs(dump_dir, dict({"black": bits64(b.cpu().numpy().view(np.uint64)),
+                                     "white": bits64(w.cpu().numpy().view(np.uint64))},
+                                    **{k: v.astype(np.float32) for k, v in fields.items()}))
     # e2e: the host-buffer entry point (results D2H inside the timed region), one launch
     E.perft_playouts(n_games, 8, seed=6, first_game_id=rank * n_games, device=local)  # warm: sizes the staging buffers
     e_calls, e_plies = 3, 0
@@ -748,10 +796,17 @@ def main():
                          "--steps/--warmup); opening: every game within its first plies (round 1's window)")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the short extra legs (opening window, cache off, configs[3] waves, tree only, perft) of the N=1 line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path computed as DIR/<name>.npy in float32/float64, "
+                         "at most 64 MB (a fixed, seeded sample of games beyond that): self-play, the records of the "
+                         "games that started in the slots, each played to its end untimed; tree, the last job's records; "
+                         "perft, the last launch's final positions.  With several GPUs, rank 0's games")
     args = ap.parse_args()
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3  # timing rule: W >= 3
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes what the CUDA path computed: it needs --impl ours")
         return run_reference(args)
     os.environ["OZ_NET_CONV2"] = args.conv2  # read by the engine when it is created
     os.environ["OZ_NET_CONV3"] = args.conv3 if args.conv2 == "table" else "direct"

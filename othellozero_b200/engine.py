@@ -63,9 +63,15 @@ def perft_playouts(n_games: int, board_size: int = 8, seed: int = 0, first_game_
     moves = np.zeros((n_games, 64), dtype=np.uint8) if want_moves else None
     check(_lib.load().oz_perft_playouts_host(device, board_size, seed & M64, first_game_id & M64, n_games, max_moves,
                                              ptr(black, u64p), ptr(white, u64p), ptr(info, u32p), ptr(moves, u8p)))
-    return dict(black=black, white=white, plies=(info & 0xFF).astype(np.int32),
-                player=((info >> 8) & 1).astype(np.int32), finished=((info >> 9) & 1).astype(bool),
-                passes=(info >> 16).astype(np.int32), moves=moves)
+    return dict(black=black, white=white, **decode_perft_info(info), moves=moves)
+
+
+def decode_perft_info(info) -> dict:
+    """The per-game info word of oz_perft_playouts_*: plies in bits 0-7, side to move in bit 8, finished in bit 9, passes
+    in bits 16-31."""
+    info = np.asarray(info, dtype=np.uint32)
+    return dict(plies=(info & 0xFF).astype(np.int32), player=((info >> 8) & 1).astype(np.int32),
+                finished=((info >> 9) & 1).astype(bool), passes=(info >> 16).astype(np.int32))
 
 
 def probe_l2_read(megabytes: int = 32, passes: int = 50, device: int = 0) -> float:

@@ -1,4 +1,6 @@
 """Replay buffer semantics (main.py:21-53) - against the reference's own CircularArray when it is importable."""
+import json
+import os
 import random
 
 import numpy as np
@@ -32,16 +34,21 @@ def test_circular_array_overwrites_oldest(max_, count):
     assert sorted(map(str, ca)) == sorted(map(str, _model(max_, list(range(count)) + ["x"])))
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference not present")
 def test_circular_array_equals_reference():
-    main = ref_loader.load_main()
-    rng = random.Random(3)
-    for max_ in (1, 4, 7):
-        a, b = CircularArray(max_), main.CircularArray(max_)
-        for _ in range(40):
-            chunk = [rng.random() for _ in range(rng.randrange(0, 6))]
-            a.extend(chunk); b.extend(chunk)
-            assert list(a) == list(b) and len(a) == len(b) and str(a) == str(b)
+    """list() and str() after each extend of a seeded sequence, as stored in tests/golden/reference_checks.json
+    (tools/gen_reference_checks.py); where the reference is importable its own CircularArray must match them too."""
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_checks.json")) as f:
+        stored = json.load(f)["circular_array"]
+    main = ref_loader.load_main() if ref_loader.available() else None
+    for case in stored:
+        arrays = [CircularArray(case["max"])] + ([main.CircularArray(case["max"])] if main else [])
+        items = []
+        for step in case["steps"]:
+            items += step["chunk"]
+            assert step["list"] == _model(case["max"], items)
+            for a in arrays:
+                a.extend(step["chunk"])
+                assert list(a) == step["list"] and len(a) == len(step["list"]) and str(a) == step["str"]
 
 
 def test_record_buffer_matches_circular_array():

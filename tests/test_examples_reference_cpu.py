@@ -1,16 +1,19 @@
 """Example stream (SURVEY 8f rank 1) against the REFERENCE: `selfplay.records_to_examples*` must reproduce
 training.execute_episode's list (training.py:58-72: 8 symmetries per move in the order of :13-23, one-hot policies,
 z, dtypes) element for element.  The committed digests (tests/golden/examples.json) were produced by running the
-reference's own execute_episode (tools/gen_golden.py examples); with /root/reference present the comparison is repeated
-element-wise against the live reference."""
+reference's own execute_episode (tools/gen_golden.py examples); one of those streams is stored in full
+(tests/golden/examples_reference_stream.npz, its bytes checked against the reference's digest) for the element-wise
+comparison."""
+import os
+
 import numpy as np
-import pytest
 
 import oracle
 import prior_fns
 from example_digest import examples_digest, oracle_episode_as_records
 from othellozero_b200 import selfplay
-from tools import ref_loader
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def _oracle_records(g):
@@ -35,13 +38,11 @@ def test_example_stream_digests(golden_examples):
         assert all(type(z) is int for _, _, z in aliased + snap + batch)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference not present")
 def test_example_stream_elementwise_vs_live_reference(golden_examples):
-    from tools import gen_golden as G
     g = golden_examples[1]  # 6x6, T = 0, e_greedy 0.7: every draw site is exercised
-    prior = G.hash_prior if g["prior"] == "hash" else prior_fns.sha_prior
-    ref, _, _ = G.reference_episode_with_engine_rng(g["n"], g["sims"], prior, 1, g["T"], g["e_greedy"], g["seed"],
-                                                    g["game_id"])
+    with np.load(os.path.join(GOLDEN, "examples_reference_stream.npz")) as f:
+        ref = [(b, p, int(z)) for b, p, z in zip(f["board"], f["policy"], f["z"])]
+    assert examples_digest(ref) == g["sha256_reference_stream"]  # the stored stream is the reference's, byte for byte
     rec = _oracle_records(g)
     ours = selfplay.records_to_examples(rec, 0, g["n"], reference_aliasing=True)
     assert len(ours) == len(ref)
