@@ -18,6 +18,20 @@
  *     in HBM and a cudaStream_t passed as void*.
  *   - There is no CPU fallback: without a CUDA device every compute entry point fails
  *     with OZ_ERR_CUDA.
+ *   - Rules.  By default every move is played with the reference's flip rule: a move also flips
+ *     opponent discs that lie beyond the bracketing own disc (Othello/__init__.py:216-235 has no
+ *     `break`).  OR-ing OZ_RULES_STANDARD into a board_size argument selects standard Othello
+ *     flipping (a run flips only up to the first own disc) for oz_rules_apply_*,
+ *     oz_perft_playouts_* and oz_engine_config.board_size (search and self-play).  Legal moves, the
+ *     initial position, the automatic pass, the terminal test and the scoring (a draw counts as a
+ *     BLACK win) are the same under both rule sets; oz_rules_legal_moves_* and oz_net_blob_floats
+ *     accept the flag and ignore it, so one value can be passed everywhere.  Any other bit above
+ *     the size is OZ_ERR_INVALID.
+ *   - Passes and perft.  A side with no legal move passes automatically inside the move that left
+ *     it without one: a pass is not a move of its own and does not use up a ply.  A full-tree perft
+ *     counted with these calls therefore treats a finished game as a leaf and a pass as free, e.g.
+ *     8x8 depths 1-9 under standard rules: 4, 12, 56, 244, 1396, 8200, 55092, 390216, 3005320
+ *     (reference rules first differ at depth 7: 55032, 389164, 2994476).
  */
 #ifndef OZ_B200_H
 #define OZ_B200_H
@@ -35,6 +49,9 @@ extern "C" {
 #define OZ_ERR_STATE (-4)   /* call sequence error (reference: RuntimeError) */
 
 #define OZ_ABI_VERSION 1
+
+/* OR-ed into a board_size argument: standard Othello flipping instead of the reference's (see Conventions) */
+#define OZ_RULES_STANDARD 0x100
 
 /* flags returned by oz_rules_apply_* (one uint32 per position) */
 #define OZ_MOVE_SWAPPED 1u  /* opponent moves next; outputs are in HIS frame (own/opp swapped) */
@@ -57,7 +74,8 @@ typedef struct oz_engine oz_engine;
 
 typedef struct oz_engine_config {
     int32_t device;          /* CUDA ordinal */
-    int32_t board_size;      /* 4, 6 or 8 (Othello/__init__.py:29-36; the net needs 6 or 8) */
+    int32_t board_size;      /* 4, 6 or 8 (Othello/__init__.py:29-36; the net needs 6 or 8), | OZ_RULES_STANDARD for
+                                standard flipping in simulations and self-play moves */
     int32_t max_games;       /* concurrent game slots (one warp each) */
     int32_t nodes_per_game;  /* node-pool capacity per game; reference keeps every node of an episode
                                 (training.py:32), i.e. <= sims * plies */

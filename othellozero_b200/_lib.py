@@ -12,6 +12,16 @@ OZ_OK, OZ_ERR_INVALID, OZ_ERR_CUDA, OZ_ERR_NOMEM, OZ_ERR_STATE = 0, -1, -2, -3, 
 PRIOR_HASH, PRIOR_HOST, PRIOR_NET = 0, 1, 2
 MOVE_SWAPPED, MOVE_PASSED, MOVE_FINISHED = 1, 2, 4
 GAME_IDLE, GAME_ACTIVE, GAME_WAIT_LEAF, GAME_FINISHED, GAME_POOL_FULL = 0, 1, 2, 3, 4
+RULES_STANDARD = 0x100  # OZ_RULES_STANDARD, OR-ed into a board_size argument
+RULES = ("reference", "standard")
+
+
+def board_arg(board_size: int, rules: str = "reference") -> int:
+    """The C-ABI board_size argument for a rule set: "reference" (the reference's flip rule, the default) or
+    "standard" (standard Othello flipping).  Anything else raises ValueError."""
+    if rules not in RULES:
+        raise ValueError(f"rules must be one of {RULES}, got {rules!r}")
+    return board_size | (RULES_STANDARD if rules == "standard" else 0)
 
 
 class EngineConfig(C.Structure):

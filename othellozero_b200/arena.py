@@ -11,6 +11,8 @@
 
 The reference's own drivers ``training.duel_between_neural_networks`` / ``evaluate_neural_network`` are broken
 (SURVEY §0.8); ``pit`` follows the working semantics of main.py:165-197 (who won, counted per game).
+``rules="standard"`` plays every game of a batched driver under standard Othello flipping; the per-game agents take the
+rule set from their game (``othello.StandardOthelloGame``).
 """
 from __future__ import annotations
 
@@ -48,7 +50,7 @@ class NeuralNetworkOthelloAgent(OthelloAgent):
         self.temperature = 0
         self.neural_network = neural_network
         self.num_simulations = num_simulations
-        self.mcts = OthelloMCTS(game.board_size, neural_network, degree_exploration)
+        self.mcts = OthelloMCTS(game.board_size, neural_network, degree_exploration, rules=game.rules)
         super().__init__(game)
 
     def play(self):
@@ -108,14 +110,15 @@ def _draw_indices(rng, counts: np.ndarray) -> np.ndarray:
 
 
 def pit(board_size, net_black, net_white, num_simulations, degree_exploration=1, n_games=64, device=0, rng=None,
-        start_black=None, start_white=None, start_player=None):
+        start_black=None, start_white=None, start_player=None, rules="reference"):
     """n_games simultaneous duels, net_black playing BLACK.  Returns dict(winner [n_games] 0/1, black, white, plies).
     Every step is one kernel chain over all games whose turn it is: one search launch per network side
     (NeuralNetworkOthelloAgent.play, agents.py:52-68, always temperature 0), one move-generator launch for a
     ``RANDOM_AGENT`` side (RandomOthelloAgent.play, agents.py:20-24; main.py:165-197 evaluates the network against it),
     one rules launch to apply the moves.  Ties in the visit counts and the random agent's moves are drawn from ``rng``
     (Python's ``random`` like the reference, or a numpy Generator for fully vectorised draws) over the candidates in
-    row-major order."""
+    row-major order.  Both sides search, and every move is applied, under ``rules``."""
+    _e.board_arg(board_size, rules)
     rng = rng or random
     n = board_size
     nodes = num_simulations * (n * n) + 64
@@ -126,7 +129,7 @@ def pit(board_size, net_black, net_white, num_simulations, degree_exploration=1,
             continue
         mode = _mode_for(net)
         e = _e.Engine(n, max_games=n_games, nodes_per_game=nodes, prior_mode=mode, c_puct=float(degree_exploration),
-                      device=device)
+                      device=device, rules=rules)
         if mode == _e.PRIOR_NET:
             e.load_weights(net.blob, net.channels)
         engines.append(e)
@@ -166,7 +169,7 @@ def pit(board_size, net_black, net_white, num_simulations, degree_exploration=1,
                     tied = visits == visits.max(axis=1, keepdims=True)             # othelo_mcts.py:58: the arg-max set
                     pick = _draw_indices(rng, tied.sum(axis=1))                    # a unique maximum needs no draw
                     sq = np.argmax(tied & ((np.cumsum(tied, axis=1) - 1) == pick[:, None]), axis=1).astype(np.int32)
-                o2, p2, fl, _ = _e.apply_moves(own, opp, sq, n, device)
+                o2, p2, fl, _ = _e.apply_moves(own, opp, sq, n, device, rules=rules)
                 assert not (fl & 0x80000000).any()
                 swapped = (fl & 1).astype(bool)
                 npl = np.where(swapped, 1 - player[idx], player[idx]).astype(np.int32)
@@ -185,21 +188,23 @@ def pit(board_size, net_black, net_white, num_simulations, degree_exploration=1,
 
 # ---- batched arena drivers (the worker work types of workers.py:18-21,72-79) -----------------------------------------
 def duels_between_neural_networks(n_duels, board_size, neural_network_1, neural_network_2, degree_exploration,
-                                  num_simulations, device=0, rng=None):
+                                  num_simulations, device=0, rng=None, rules="reference"):
     """``n_duels`` x training.duel_between_neural_networks (training.py:75-89) as one batch: network 1 plays BLACK
     (agent_1 of duel_between_agents, agents.py:71-74); each entry is 0 if network 1 won, else 1."""
     out = pit(board_size, neural_network_1, neural_network_2, num_simulations, degree_exploration, n_games=n_duels,
-              device=device, rng=rng)
+              device=device, rng=rng, rules=rules)
     return [int(w) for w in out["winner"]]
 
 
 def evaluate_neural_network(board_size, total_iterations, neural_network, num_simulations, degree_exploration,
-                            agent_class=RandomOthelloAgent, agent_arguments=(), device=0, rng=None, repeats=1):
+                            agent_class=RandomOthelloAgent, agent_arguments=(), device=0, rng=None, repeats=1,
+                            rules="reference"):
     """training.evaluate_neural_network (training.py:92-115) with the working semantics of main.py:165-197: the network
     meets ``agent_class`` (RandomOthelloAgent) in ``total_iterations`` games, colours shuffled per game; returns the
     network's wins.  ``repeats`` > 1 plays that many evaluations in the same batch and returns a list of win counts."""
     if agent_class is not RandomOthelloAgent:
         raise TypeError("the batched evaluation plays against RandomOthelloAgent (main.py:165-197)")
+    _e.board_arg(board_size, rules)
     rng = rng or random
     games = total_iterations * repeats
     net_is_black = np.array([rng.random() < 0.5 for _ in range(games)], dtype=bool)   # random.shuffle of two agents
@@ -209,7 +214,8 @@ def evaluate_neural_network(board_size, total_iterations, neural_network, num_si
         if sel.size == 0:
             continue
         a, b = (neural_network, RANDOM_AGENT) if black_side else (RANDOM_AGENT, neural_network)
-        out = pit(board_size, a, b, num_simulations, degree_exploration, n_games=int(sel.size), device=device, rng=rng)
+        out = pit(board_size, a, b, num_simulations, degree_exploration, n_games=int(sel.size), device=device, rng=rng,
+                  rules=rules)
         net_won[sel] = out["winner"] == (0 if black_side else 1)
     wins = net_won.reshape(repeats, total_iterations).sum(axis=1)
     return int(wins[0]) if repeats == 1 else [int(w) for w in wins]

@@ -14,6 +14,11 @@
 //                 occupied square and flips opponent discs beyond own discs too)
 //   turn logic    Othello/__init__.py:147-159, othelo_mcts.py:43-49
 //   terminal      Othello/__init__.py:249-252;  winner :254-260 (draw -> BLACK / ch0)
+//
+// Standard Othello flipping (a run of opponent discs flips only when the FIRST own disc beyond it brackets it) is
+// offered next to the reference quirk: flip_mask_standard / flip_mask_standard_compact, and apply_move / play_move
+// take the rule set as a template parameter (RULES_REFERENCE by default).  Legal moves, the initial position, the
+// pass and terminal logic and the scoring are the same under both rule sets.
 #pragma once
 #include <stdint.h>
 
@@ -144,6 +149,38 @@ OZ_HD oz_u64 flip_mask(oz_u64 m, oz_u64 own, oz_u64 opp) {
     return f;
 }
 
+// ---- flips (standard Othello) ----------------------------------------------------------------------------
+// Along +D: the contiguous OPPONENT run behind the move (occluded fill through opponent discs only), kept iff the square
+// right after it is an own disc.  `wrap` as in flips_up: shifting by D must not wrap across a column edge.
+template <int D>
+OZ_HD oz_u64 flips_up_standard(oz_u64 m, oz_u64 own, oz_u64 opp, oz_u64 wrap) {
+    oz_u64 pro = opp & wrap;
+    oz_u64 run = fill_up<D>((m << D) & pro, pro);
+    return ((run << D) & wrap & own) ? run : 0ull;
+}
+template <int D>
+OZ_HD oz_u64 flips_down_standard(oz_u64 m, oz_u64 own, oz_u64 opp, oz_u64 wrap) {
+    oz_u64 pro = opp & wrap;
+    oz_u64 run = fill_down<D>((m >> D) & pro, pro);
+    return ((run >> D) & wrap & own) ? run : 0ull;
+}
+
+OZ_HD oz_u64 flip_mask_standard(oz_u64 m, oz_u64 own, oz_u64 opp) {
+    oz_u64 f = 0;
+    f |= flips_up_standard<1>(m, own, opp, NOT_A);
+    f |= flips_up_standard<9>(m, own, opp, NOT_A);
+    f |= flips_up_standard<8>(m, own, opp, ~0ull);
+    f |= flips_up_standard<7>(m, own, opp, NOT_H);
+    f |= flips_down_standard<1>(m, own, opp, NOT_H);
+    f |= flips_down_standard<9>(m, own, opp, NOT_H);
+    f |= flips_down_standard<8>(m, own, opp, ~0ull);
+    f |= flips_down_standard<7>(m, own, opp, NOT_A);
+    return f;
+}
+
+// Rule sets of apply_move / play_move (and of the kernels instantiated per rule set).
+enum : int { RULES_REFERENCE = 0, RULES_STANDARD = 1 };
+
 // ---- compact forms -------------------------------------------------------------------------------------
 // The same arithmetic with the four axes walked by a loop with run-time shift counts (a 64-bit shift costs two
 // instructions either way): about a quarter of the code.  For callers whose instruction FOOTPRINT matters more than
@@ -211,9 +248,46 @@ OZ_HD oz_u64 flip_mask_compact(oz_u64 m, oz_u64 own, oz_u64 opp) {
     return f;
 }
 
+// flip_mask_standard in the compact form (same footprint constraints as flip_mask_compact).
+OZ_HD oz_u64 flip_mask_standard_compact(oz_u64 m, oz_u64 own, oz_u64 opp) {
+    oz_u64 f = 0;
+#if defined(__CUDA_ARCH__)
+#pragma unroll 1
+#endif
+    for (int a = 0; a < 4; ++a) {
+        const int D = (a == 0) ? 1 : 6 + a;  // 1, 7, 8, 9
+        const oz_u64 wu = (D == 8) ? ~0ull : (D == 7 ? NOT_H : NOT_A);
+        const oz_u64 wd = (D == 8) ? ~0ull : (D == 7 ? NOT_A : NOT_H);
+        {   // flips_up_standard<D>
+            oz_u64 pro = opp & wu;
+            oz_u64 gen = (m << D) & pro;
+            gen |= pro & (gen << D);
+            pro &= pro << D;
+            gen |= pro & (gen << (2 * D));
+            pro &= pro << (2 * D);
+            gen |= pro & (gen << (4 * D));
+            f |= ((gen << D) & wu & own) ? gen : 0ull;
+        }
+        {   // flips_down_standard<D>
+            oz_u64 pro = opp & wd;
+            oz_u64 gen = (m >> D) & pro;
+            gen |= pro & (gen >> D);
+            pro &= pro >> D;
+            gen |= pro & (gen >> (2 * D));
+            pro &= pro >> (2 * D);
+            gen |= pro & (gen >> (4 * D));
+            f |= ((gen >> D) & wd & own) ? gen : 0ull;
+        }
+    }
+    return f;
+}
+
 // flip_board_squares, Othello/__init__.py:237-247: mover = own.
+template <int RULES = RULES_REFERENCE>
 OZ_HD void apply_move(oz_u64 m, oz_u64* own, oz_u64* opp) {
-    oz_u64 f = flip_mask(m, *own, *opp);
+    oz_u64 f;
+    if constexpr (RULES == RULES_STANDARD) f = flip_mask_standard(m, *own, *opp);
+    else f = flip_mask(m, *own, *opp);
     *own |= f | m;
     *opp &= ~f;
 }
@@ -224,8 +298,9 @@ enum : unsigned { MOVE_SWAPPED = 1u, MOVE_PASSED = 2u, MOVE_FINISHED = 4u };
 // Move + turn logic (OthelloGame.play :147-159 == get_next_state othelo_mcts.py:43-49).
 // On return (*own,*opp) is in the frame of the side to move NEXT (swapped iff the opponent
 // can move); *next_legal = that side's legal moves (0 iff finished).
+template <int RULES = RULES_REFERENCE>
 OZ_HD unsigned play_move(oz_u64 m, oz_u64* own, oz_u64* opp, oz_u64 full, oz_u64* next_legal) {
-    apply_move(m, own, opp);
+    apply_move<RULES>(m, own, opp);
     oz_u64 lo = legal_moves(*opp, *own, full);
     if (lo) {
         oz_u64 t = *own; *own = *opp; *opp = t;

@@ -63,13 +63,13 @@ __global__ void validate_starts_kernel(int n_games, const u64* __restrict__ blac
 extern "C" int oz_engine_create(const oz_engine_config* cfg, oz_engine** out) {
     OZ_REQUIRE(cfg && out, "null argument");
     *out = nullptr;
-    OZ_REQUIRE(cfg->board_size == 4 || cfg->board_size == 6 || cfg->board_size == 8,
-               "board_size must be 4, 6 or 8 (got %d)", cfg->board_size);
+    int size, rules;
+    if (oz_decode_board(cfg->board_size, &size, &rules)) return OZ_ERR_INVALID;
     OZ_REQUIRE(cfg->max_games >= 1 && cfg->max_games <= (1 << 20), "max_games out of range: %d", cfg->max_games);
     OZ_REQUIRE(cfg->nodes_per_game >= 2 && cfg->nodes_per_game <= (1 << 22), "nodes_per_game out of range: %d",
                cfg->nodes_per_game);
     OZ_REQUIRE(cfg->prior_mode >= OZ_PRIOR_HASH && cfg->prior_mode <= OZ_PRIOR_NET, "bad prior_mode %d", cfg->prior_mode);
-    OZ_REQUIRE(cfg->prior_mode != OZ_PRIOR_NET || cfg->board_size >= 6, "the network needs board_size 6 or 8");
+    OZ_REQUIRE(cfg->prior_mode != OZ_PRIOR_NET || size >= 6, "the network needs board_size 6 or 8");
     OZ_REQUIRE(cfg->vl_width >= 0 && cfg->vl_width <= 64, "vl_width out of range: %d", cfg->vl_width);
     int ndev = 0;
     int rc = oz_device_count(&ndev);
@@ -81,6 +81,8 @@ extern "C" int oz_engine_create(const oz_engine_config* cfg, oz_engine** out) {
     OZ_CUDA(cudaSetDevice(cfg->device));
     oz_engine* e = new oz_engine();
     e->cfg = *cfg;
+    e->cfg.board_size = size;
+    e->rules = rules;
     cudaError_t err = cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking);
     if (err != cudaSuccess) {
         oz_set_error("cudaStreamCreate failed: %s", cudaGetErrorString(err));
@@ -495,7 +497,9 @@ extern "C" int oz_selfplay_get_positions(oz_engine* e, uint64_t* black, uint64_t
 
 // ---- network ----------------------------------------------------------------------------------------
 extern "C" int64_t oz_net_blob_floats(int32_t board_size, int32_t channels) {
-    return oz_net_blob_floats_impl(board_size, channels);
+    int size;  // the network does not depend on the rule set: the rules flag is accepted and ignored
+    if (oz_decode_board(board_size, &size, nullptr)) return -1;
+    return oz_net_blob_floats_impl(size, channels);
 }
 
 extern "C" int oz_net_load_weights(oz_engine* e, const float* blob, int64_t n_floats, int32_t channels) {

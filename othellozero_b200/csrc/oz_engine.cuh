@@ -29,6 +29,19 @@ void oz_set_error(const char* fmt, ...);
         }                            \
     } while (0)
 
+// The board_size argument of the C-ABI: N (4, 6 or 8), optionally | OZ_RULES_STANDARD.  -> N and the ozbb rule set
+// (either output may be null); any other bit is OZ_ERR_INVALID.  Only the C-ABI entry points see the flag.
+inline int oz_decode_board(int32_t board_size, int* n, int* rules) {
+    const int size = board_size & ~OZ_RULES_STANDARD;
+    if (size != 4 && size != 6 && size != 8) {
+        oz_set_error("board_size must be 4, 6 or 8, optionally | OZ_RULES_STANDARD (got %d)", board_size);
+        return OZ_ERR_INVALID;
+    }
+    if (n) *n = size;
+    if (rules) *rules = (board_size & OZ_RULES_STANDARD) ? ozbb::RULES_STANDARD : ozbb::RULES_REFERENCE;
+    return OZ_OK;
+}
+
 // ---- tree node pool layout (HBM) -----------------------------------------------------------------
 // Node = 48-byte header followed by SoA child rows, k = popcount(legal):
 //   double P[k]; double Q[k]; int N[k]; int child[k];        (48 + 24k bytes, rounded up to 16)
@@ -100,7 +113,8 @@ struct OzTreeParams {
 struct OzNet;  // oz_net.cu
 
 struct oz_engine {
-    oz_engine_config cfg;
+    oz_engine_config cfg;      // cfg.board_size holds plain N; the rules flag of the caller's value is in `rules`
+    int rules = ozbb::RULES_REFERENCE;
     cudaStream_t stream = nullptr;
     OzTreeParams tp{};
     int n_games = 0;

@@ -20,6 +20,7 @@ __global__ void __launch_bounds__(256) rules_legal_kernel(const u64* __restrict_
         moves[i] = legal_moves(own[i], opp[i], full);
 }
 
+template <int RULES>
 __global__ void __launch_bounds__(256)
 rules_apply_kernel(const u64* __restrict__ own, const u64* __restrict__ opp, const int* __restrict__ sq,
                    u64* __restrict__ own_out, u64* __restrict__ opp_out, u32* __restrict__ flags,
@@ -34,7 +35,7 @@ rules_apply_kernel(const u64* __restrict__ own, const u64* __restrict__ opp, con
         if (!(m & legal_moves(o, p, full))) {
             fl = 0x80000000u;  // not a legal move: position returned unchanged
         } else {
-            fl = play_move(m, &o, &p, full, &nl);
+            fl = play_move<RULES>(m, &o, &p, full, &nl);
         }
         own_out[i] = o;
         opp_out[i] = p;
@@ -54,6 +55,7 @@ __global__ void __launch_bounds__(256) rules_score_kernel(const u64* __restrict_
 }
 
 // One thread = one whole random game; nothing but the final position touches memory.
+template <int RULES>
 __global__ void __launch_bounds__(256)
 perft_playout_kernel(int n, u64 full, u64 seed, u64 first_id, long long n_games, int max_moves,
                      u64* __restrict__ black, u64* __restrict__ white, u32* __restrict__ info,
@@ -71,7 +73,7 @@ perft_playout_kernel(int n, u64 full, u64 seed, u64 first_id, long long n_games,
             u32 k = pick_index(sm64(base + (u64)plies), cnt);
             int s = kth_set_bit(legal, (int)k);
             if (mv && plies < 64) mv[plies] = (unsigned char)s;
-            u32 fl = play_move(1ull << s, &own, &opp, full, &legal);
+            u32 fl = play_move<RULES>(1ull << s, &own, &opp, full, &legal);
             ++plies;
             if (fl & MOVE_SWAPPED) player ^= 1u;
             if (fl & MOVE_PASSED) ++passes;
@@ -96,20 +98,13 @@ static int grid_for(long long n, int block) {
     return (int)b;
 }
 
-static int check_board_size(int n) {
-    if (n != 4 && n != 6 && n != 8) {
-        oz_set_error("board_size must be 4, 6 or 8 (got %d)", n);
-        return OZ_ERR_INVALID;
-    }
-    return OZ_OK;
-}
-
 extern "C" int oz_rules_legal_moves_dev(int32_t board_size, const uint64_t* own, const uint64_t* opp,
                                         uint64_t* moves, int64_t n, void* stream) {
-    if (check_board_size(board_size)) return OZ_ERR_INVALID;
+    int size;  // legal moves are the same under both rule sets: the flag is accepted and ignored
+    if (oz_decode_board(board_size, &size, nullptr)) return OZ_ERR_INVALID;
     if (n <= 0) return OZ_OK;
     rules_legal_kernel<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>((const u64*)own, (const u64*)opp,
-                                                                            (u64*)moves, n, full_mask(board_size));
+                                                                            (u64*)moves, n, full_mask(size));
     OZ_CUDA(cudaGetLastError());
     return OZ_OK;
 }
@@ -117,11 +112,12 @@ extern "C" int oz_rules_legal_moves_dev(int32_t board_size, const uint64_t* own,
 extern "C" int oz_rules_apply_dev(int32_t board_size, const uint64_t* own, const uint64_t* opp, const int32_t* sq,
                                   uint64_t* own_out, uint64_t* opp_out, uint32_t* flags, uint64_t* next_legal,
                                   int64_t n, void* stream) {
-    if (check_board_size(board_size)) return OZ_ERR_INVALID;
+    int size, rules;
+    if (oz_decode_board(board_size, &size, &rules)) return OZ_ERR_INVALID;
     if (n <= 0) return OZ_OK;
-    rules_apply_kernel<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(
-        (const u64*)own, (const u64*)opp, sq, (u64*)own_out, (u64*)opp_out, flags, (u64*)next_legal, n,
-        full_mask(board_size));
+    auto kernel = rules == RULES_STANDARD ? rules_apply_kernel<RULES_STANDARD> : rules_apply_kernel<RULES_REFERENCE>;
+    kernel<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>((const u64*)own, (const u64*)opp, sq, (u64*)own_out,
+                                                               (u64*)opp_out, flags, (u64*)next_legal, n, full_mask(size));
     OZ_CUDA(cudaGetLastError());
     return OZ_OK;
 }
@@ -138,15 +134,16 @@ extern "C" int oz_rules_score_dev(const uint64_t* black, const uint64_t* white, 
 extern "C" int oz_perft_playouts_dev(int32_t board_size, uint64_t seed, uint64_t first_game_id, int64_t n_games,
                                      int32_t max_moves, uint64_t* black, uint64_t* white, uint32_t* info,
                                      uint8_t* moves, void* stream) {
-    if (check_board_size(board_size)) return OZ_ERR_INVALID;
+    int size, rules;
+    if (oz_decode_board(board_size, &size, &rules)) return OZ_ERR_INVALID;
     if (n_games <= 0) return OZ_OK;
     // 128-thread CTAs: games end at different plies, smaller CTAs retire sooner (less tail per SM).
     long long blocks = (n_games + 127) / 128;
     long long cap = 148LL * 16 * 8;
     if (blocks > cap) blocks = cap;
-    perft_playout_kernel<<<(int)blocks, 128, 0, (cudaStream_t)stream>>>(board_size, full_mask(board_size), seed,
-                                                                        first_game_id, n_games, max_moves,
-                                                                        (u64*)black, (u64*)white, info, moves);
+    auto kernel = rules == RULES_STANDARD ? perft_playout_kernel<RULES_STANDARD> : perft_playout_kernel<RULES_REFERENCE>;
+    kernel<<<(int)blocks, 128, 0, (cudaStream_t)stream>>>(size, full_mask(size), seed, first_game_id, n_games, max_moves,
+                                                          (u64*)black, (u64*)white, info, moves);
     OZ_CUDA(cudaGetLastError());
     return OZ_OK;
 }
@@ -202,7 +199,7 @@ inline size_t up256(size_t x) { return (x + 255) & ~(size_t)255; }
 
 extern "C" int oz_rules_legal_moves_host(int32_t device, int32_t board_size, const uint64_t* own,
                                          const uint64_t* opp, uint64_t* moves, int64_t n) {
-    if (check_board_size(board_size)) return OZ_ERR_INVALID;
+    if (oz_decode_board(board_size, nullptr, nullptr)) return OZ_ERR_INVALID;
     OZ_REQUIRE(n >= 0 && (n == 0 || (own && opp && moves)), "null buffer");
     if (n == 0) return OZ_OK;
     HostScratch& S = g_scratch;
@@ -224,7 +221,7 @@ extern "C" int oz_rules_legal_moves_host(int32_t device, int32_t board_size, con
 extern "C" int oz_rules_apply_host(int32_t device, int32_t board_size, const uint64_t* own, const uint64_t* opp,
                                    const int32_t* sq, uint64_t* own_out, uint64_t* opp_out, uint32_t* flags,
                                    uint64_t* next_legal, int64_t n) {
-    if (check_board_size(board_size)) return OZ_ERR_INVALID;
+    if (oz_decode_board(board_size, nullptr, nullptr)) return OZ_ERR_INVALID;
     OZ_REQUIRE(n >= 0 && (n == 0 || (own && opp && sq && own_out && opp_out && flags)), "null buffer");
     if (n == 0) return OZ_OK;
     HostScratch& S = g_scratch;
@@ -275,7 +272,7 @@ extern "C" int oz_rules_score_host(int32_t device, const uint64_t* black, const 
 extern "C" int oz_perft_playouts_host(int32_t device, int32_t board_size, uint64_t seed, uint64_t first_game_id,
                                       int64_t n_games, int32_t max_moves, uint64_t* black, uint64_t* white,
                                       uint32_t* info, uint8_t* moves) {
-    if (check_board_size(board_size)) return OZ_ERR_INVALID;
+    if (oz_decode_board(board_size, nullptr, nullptr)) return OZ_ERR_INVALID;
     OZ_REQUIRE(n_games >= 0 && (n_games == 0 || (black && white && info)), "null buffer");
     if (n_games == 0) return OZ_OK;
     HostScratch& S = g_scratch;

@@ -63,12 +63,19 @@ __device__ __forceinline__ u64 key_hash(u64 own, u64 opp) {
 // which is what keeps the kernel's hot loops inside the instruction cache (round 1: ~10.3 K SASS instructions, fetch
 // stalls on top of the stall list).
 // ... and they use the looped compact forms of oz_bitboard.cuh (a quarter of the unrolled templates' code, same issue count).
-__device__ __noinline__ u64 flip_mask_call(u64 m, u64 own, u64 opp) { return flip_mask_compact(m, own, opp); }
+// The rule set is a template parameter of the kernel (one instantiation per rule set, chosen at launch), never a
+// run-time branch, so the reference instantiation carries no cost for the standard rule (tools/sass_compare.py).
+template <int RULES>
+__device__ __noinline__ u64 flip_mask_call(u64 m, u64 own, u64 opp) {
+    if constexpr (RULES == RULES_STANDARD) return flip_mask_standard_compact(m, own, opp);
+    else return flip_mask_compact(m, own, opp);
+}
 __device__ __noinline__ u64 legal_moves_call(u64 own, u64 opp, u64 full) { return legal_moves_compact(own, opp, full); }
 
 // play_move (oz_bitboard.cuh) over the out-of-line helpers.
+template <int RULES>
 __device__ __forceinline__ unsigned play_move_dev(u64 m, u64& own, u64& opp, u64 full, u64& next_legal) {
-    const u64 f = flip_mask_call(m, own, opp);
+    const u64 f = flip_mask_call<RULES>(m, own, opp);
     own |= f | m;
     opp &= ~f;
     const u64 lo = legal_moves_call(opp, own, full);
@@ -417,6 +424,7 @@ __device__ __noinline__ double ucb_value_call(int nraw, double q, double pj, dou
 #ifndef OZ_TREE_MIN_CTAS
 #define OZ_TREE_MIN_CTAS 7
 #endif
+template <int RULES>
 __global__ void __launch_bounds__(TREE_WARPS * 32, OZ_TREE_MIN_CTAS) tree_step_kernel(const OzTreeParams P) {
     __shared__ double s_a[TREE_WARPS][72];  // [0,64): masked priors of the node being expanded, [64,72): its partial sums
     const int lane = threadIdx.x & 31;
@@ -562,7 +570,7 @@ __global__ void __launch_bounds__(TREE_WARPS * 32, OZ_TREE_MIN_CTAS) tree_step_k
                     }
                 }
                 u64 nl;
-                const unsigned fl = play_move_dev(1ull << sq, own, opp, P.full, nl);
+                const unsigned fl = play_move_dev<RULES>(1ull << sq, own, opp, P.full, nl);
                 if (fl & MOVE_SWAPPED) player ^= 1;
                 black = player ? opp : own;
                 white = player ? own : opp;
@@ -675,7 +683,7 @@ __global__ void __launch_bounds__(TREE_WARPS * 32, OZ_TREE_MIN_CTAS) tree_step_k
                 u64 own = h->own, opp = h->opp;
                 const int sq = warp_kth_set_bit(h->legal, bj, lane);
                 u64 nl;
-                const unsigned fl = play_move_dev(1ull << sq, own, opp, P.full, nl);
+                const unsigned fl = play_move_dev<RULES>(1ull << sq, own, opp, P.full, nl);
                 if (fl & MOVE_FINISHED) {
                     // is_terminal_state -> return -reward; reward = +1 iff ch0 count >= ch1 count (draw -> BLACK)
                     int reward = (popc(own) >= popc(opp)) ? 1 : -1;
@@ -1053,7 +1061,8 @@ int oz_tree_reset(oz_engine* e, int n_games, const u64* black, const u64* white,
 int oz_tree_step(oz_engine* e) {
     OzTreeParams& P = e->tp;
     int blocks = (P.G + TREE_WARPS - 1) / TREE_WARPS;
-    tree_step_kernel<<<blocks, TREE_WARPS * 32, 0, e->stream>>>(P);
+    auto kernel = e->rules == RULES_STANDARD ? tree_step_kernel<RULES_STANDARD> : tree_step_kernel<RULES_REFERENCE>;
+    kernel<<<blocks, TREE_WARPS * 32, 0, e->stream>>>(P);
     OZ_CUDA(cudaGetLastError());
     e->launches++;
     return OZ_OK;

@@ -7,7 +7,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import (PRIOR_HASH, PRIOR_HOST, PRIOR_NET, check, f32p, f64p, i32p, ptr, u8p, u32p, u64p)
+from ._lib import (PRIOR_HASH, PRIOR_HOST, PRIOR_NET, board_arg, check, f32p, f64p, i32p, ptr, u8p, u32p, u64p)
 
 M64 = (1 << 64) - 1
 
@@ -21,25 +21,28 @@ def _i32(a):
 
 
 # ---- stateless rules (Othello/__init__.py) ------------------------------------------------------
-def legal_moves(own, opp, board_size: int = 8, device: int = 0) -> np.ndarray:
-    """get_player_valid_actions as masks (Othello/__init__.py:208-214). own/opp: uint64 arrays."""
+def legal_moves(own, opp, board_size: int = 8, device: int = 0, rules: str = "reference") -> np.ndarray:
+    """get_player_valid_actions as masks (Othello/__init__.py:208-214). own/opp: uint64 arrays.  Legal moves are the
+    same under both rule sets; `rules` is checked and otherwise ignored."""
+    bs = board_arg(board_size, rules)
     own, opp = _u64(np.atleast_1d(own)), _u64(np.atleast_1d(opp))
     assert own.shape == opp.shape
     out = np.zeros(own.shape, dtype=np.uint64)
-    check(_lib.load().oz_rules_legal_moves_host(device, board_size, ptr(own, u64p), ptr(opp, u64p), ptr(out, u64p),
-                                                own.size))
+    check(_lib.load().oz_rules_legal_moves_host(device, bs, ptr(own, u64p), ptr(opp, u64p), ptr(out, u64p), own.size))
     return out
 
 
-def apply_moves(own, opp, sq, board_size: int = 8, device: int = 0):
-    """flip_board_squares + turn logic (Othello/__init__.py:237-247,147-159).
-    Returns (own', opp', flags, next_legal) in the frame of the side to move next."""
+def apply_moves(own, opp, sq, board_size: int = 8, device: int = 0, rules: str = "reference"):
+    """flip_board_squares + turn logic (Othello/__init__.py:237-247,147-159), with the reference's flip rule or, for
+    rules="standard", standard Othello flipping.  Returns (own', opp', flags, next_legal) in the frame of the side to
+    move next."""
+    bs = board_arg(board_size, rules)
     own, opp, sq = _u64(np.atleast_1d(own)), _u64(np.atleast_1d(opp)), _i32(np.atleast_1d(sq))
     assert own.shape == opp.shape == sq.shape
     o2, p2 = np.zeros_like(own), np.zeros_like(own)
     fl = np.zeros(own.shape, dtype=np.uint32)
     nl = np.zeros_like(own)
-    check(_lib.load().oz_rules_apply_host(device, board_size, ptr(own, u64p), ptr(opp, u64p), ptr(sq, i32p),
+    check(_lib.load().oz_rules_apply_host(device, bs, ptr(own, u64p), ptr(opp, u64p), ptr(sq, i32p),
                                           ptr(o2, u64p), ptr(p2, u64p), ptr(fl, u32p), ptr(nl, u64p), own.size))
     return o2, p2, fl, nl
 
@@ -55,13 +58,14 @@ def score(black, white, device: int = 0):
 
 
 def perft_playouts(n_games: int, board_size: int = 8, seed: int = 0, first_game_id: int = 0, max_moves: int = -1,
-                   want_moves: bool = False, device: int = 0):
-    """Random playouts (agents.py:20-24,71-84) with the engine RNG.  Returns dict of arrays."""
+                   want_moves: bool = False, device: int = 0, rules: str = "reference"):
+    """Random playouts (agents.py:20-24,71-84) with the engine RNG under `rules`.  Returns dict of arrays."""
+    bs = board_arg(board_size, rules)
     black = np.zeros(n_games, dtype=np.uint64)
     white = np.zeros(n_games, dtype=np.uint64)
     info = np.zeros(n_games, dtype=np.uint32)
     moves = np.zeros((n_games, 64), dtype=np.uint8) if want_moves else None
-    check(_lib.load().oz_perft_playouts_host(device, board_size, seed & M64, first_game_id & M64, n_games, max_moves,
+    check(_lib.load().oz_perft_playouts_host(device, bs, seed & M64, first_game_id & M64, n_games, max_moves,
                                              ptr(black, u64p), ptr(white, u64p), ptr(info, u32p), ptr(moves, u8p)))
     return dict(black=black, white=white, **decode_perft_info(info), moves=moves)
 
@@ -82,13 +86,16 @@ def probe_l2_read(megabytes: int = 32, passes: int = 50, device: int = 0) -> flo
 
 
 class Engine:
-    """oz_engine handle: node pools + per-game state for `max_games` concurrent games on one GPU."""
+    """oz_engine handle: node pools + per-game state for `max_games` concurrent games on one GPU.  `rules` is the rule
+    set of every simulation and self-play move: "reference" (default) or "standard" Othello flipping."""
 
     def __init__(self, board_size: int = 8, max_games: int = 1, nodes_per_game: int = 8192,
                  prior_mode: int = PRIOR_HASH, c_puct: float = 1.0, seed: int = 0, device: int = 0,
-                 log_visits: bool = False, eval_cache_log2: int = 0, vl_width: int = 1):
+                 log_visits: bool = False, eval_cache_log2: int = 0, vl_width: int = 1, rules: str = "reference"):
+        bs = board_arg(board_size, rules)
         self._L = _lib.load()
         self.board_size = board_size
+        self.rules = rules
         self.nsq = board_size * board_size
         self.max_games = max_games
         self.prior_mode = prior_mode
@@ -96,7 +103,7 @@ class Engine:
         self.log_visits = log_visits
         self.vl_width = max(1, int(vl_width))
         self.max_leaves = max_games * self.vl_width
-        cfg = _lib.EngineConfig(device, board_size, max_games, nodes_per_game, prior_mode, int(log_visits),
+        cfg = _lib.EngineConfig(device, bs, max_games, nodes_per_game, prior_mode, int(log_visits),
                                 int(eval_cache_log2), int(vl_width), float(c_puct), seed & M64)
         h = C.c_void_p()
         check(self._L.oz_engine_create(C.byref(cfg), C.byref(h)))

@@ -44,6 +44,7 @@ class IterationConfig:
     arena_simulations: int = 25
     max_concurrent: int = 4096
     seed: int = 0
+    rules: str = "reference"         # "standard": self-play and arena under standard Othello flipping
 
 
 def unpack_rows(rows: np.ndarray):
@@ -116,7 +117,8 @@ class Trainer:
         rec = None
         if ids.size:
             sp = selfplay.SelfPlay(n, net_now, cfg.degree_exploration, max_games=min(int(ids.size), cfg.max_concurrent),
-                                   num_simulations=cfg.num_simulations, device=self.local, seed=cfg.seed)
+                                   num_simulations=cfg.num_simulations, device=self.local, seed=cfg.seed,
+                                   rules=cfg.rules)
             rec = sp.play(int(ids.size), cfg.temperature, cfg.e_greedy, game_ids=ids)
             info["selfplay_sims_this_rank"] = sp.engine.counters()["sims"]
             sp.close()
@@ -145,10 +147,10 @@ class Trainer:
         rng = np.random.default_rng(cfg.seed * 1000 + self.iteration * 64 + self.rank)
         if mine_a:
             wins += int((arena.pit(n, new_net, old_net, cfg.arena_simulations, cfg.degree_exploration, n_games=mine_a,
-                                   device=self.local, rng=rng)["winner"] == 0).sum())
+                                   device=self.local, rng=rng, rules=cfg.rules)["winner"] == 0).sum())
         if mine_b:
             wins += int((arena.pit(n, old_net, new_net, cfg.arena_simulations, cfg.degree_exploration, n_games=mine_b,
-                                   device=self.local, rng=rng)["winner"] == 1).sum())
+                                   device=self.local, rng=rng, rules=cfg.rules)["winner"] == 1).sum())
         if self.world > 1:
             t = torch.tensor([wins], dtype=torch.int64, device=dev)
             dist.all_reduce(t)
@@ -178,9 +180,10 @@ class Trainer:
 
 
 def main(argv=None):
+    from ._lib import RULES
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     for f, v in asdict(IterationConfig()).items():
-        ap.add_argument("--" + f.replace("_", "-"), type=type(v), default=v)
+        ap.add_argument("--" + f.replace("_", "-"), type=type(v), default=v, **({"choices": RULES} if f == "rules" else {}))
     ap.add_argument("--iterations", type=int, default=1)
     args = ap.parse_args(argv)
     import torch

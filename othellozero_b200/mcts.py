@@ -13,6 +13,7 @@ the CUDA tree kernel.  Same constructor and method names as the reference:
   * anything with ``.predict`` (e.g. the reference's Keras NNetWrapper) -> leaves are handed to the host and
     ``predict`` is called once per expanded node, exactly as the reference does (OZ_PRIOR_HOST).
 Aliases ``search`` / ``getActionProb`` are the alpha-zero-general names used in BASELINE.json.
+``rules="standard"`` searches under standard Othello flipping instead of the reference's flip rule.
 """
 from __future__ import annotations
 
@@ -22,7 +23,7 @@ import numpy as np
 
 from . import engine as _e
 from .net import B200NNet, NeuralNets, bits_to_board
-from .othello import OthelloGame, OthelloPlayer, _bits
+from .othello import OthelloGame, OthelloPlayer, StandardOthelloGame, _bits
 
 
 class HashPriorNet:
@@ -34,7 +35,8 @@ class HashPriorNet:
 
 
 class OthelloMCTS:
-    def __init__(self, board_size, neural_network, degree_exploration, nodes: int = 65536, device: int = 0):
+    def __init__(self, board_size, neural_network, degree_exploration, nodes: int = 65536, device: int = 0,
+                 rules: str = "reference"):
         self._board_size = board_size
         self._neural_network = neural_network
         self.degree_explorarion = degree_exploration  # (sic) MCTS/__init__.py:27
@@ -49,7 +51,8 @@ class OthelloMCTS:
             mode = _e.PRIOR_HOST
         self._mode = mode
         self._eng = _e.Engine(board_size, max_games=1, nodes_per_game=nodes, prior_mode=mode,
-                              c_puct=float(degree_exploration), device=device)
+                              c_puct=float(degree_exploration), device=device, rules=rules)
+        self._game = StandardOthelloGame if rules == "standard" else OthelloGame
         if mode == _e.PRIOR_NET:
             self._eng.load_weights(neural_network.blob, neural_network.channels)
         self._eng.reset(1)
@@ -101,7 +104,7 @@ class OthelloMCTS:
 
     def get_next_state(self, state, action):
         board = np.copy(state)
-        OthelloGame.flip_board_squares(board, OthelloPlayer.BLACK, *action)
+        self._game.flip_board_squares(board, OthelloPlayer.BLACK, *action)
         if OthelloGame.has_player_actions_on_board(board, OthelloPlayer.WHITE):
             board = OthelloGame.invert_board(board)
         return board

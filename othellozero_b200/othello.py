@@ -11,6 +11,10 @@ inside the kernels (csrc/oz_bitboard.cuh).
 
 Deliberate deviations are listed in INTEGRATION.md (e.g. ``is_square_free`` works here; the reference's
 version raises NameError, Othello/__init__.py:88-98).
+
+``OthelloGame`` plays the reference's rules, including its flip rule (a move also flips opponent discs beyond the
+bracketing own disc).  ``StandardOthelloGame`` is the same class with standard Othello flipping; the class attribute
+``rules`` selects the rule set of ``play``, ``get_action_flip_squares``, ``flip_board_squares`` and ``getNextState``.
 """
 from __future__ import annotations
 
@@ -62,6 +66,7 @@ def _mask_to_squares(mask: int, n: int):
 class OthelloGame:
     PLAYER_CHANNELS = {OthelloPlayer.BLACK: 0, OthelloPlayer.WHITE: 1}
     device = 0  # CUDA ordinal used by the static rule calls
+    rules = "reference"  # flip rule of play / get_action_flip_squares / flip_board_squares / getNextState
 
     def __init__(self, board_size=8, initial_board=None, current_player=OthelloPlayer.BLACK):
         """Othello/__init__.py:29-59: same arguments, same assertions; a supplied board is adopted (not copied)."""
@@ -119,7 +124,7 @@ class OthelloGame:
         n = self._board_size
         black, white = _bits(self._board)
         own, opp = (black, white) if self.current_player is OthelloPlayer.BLACK else (white, black)
-        o2, p2, fl, _ = _e.apply_moves([own], [opp], [int(row) * 8 + int(col)], n, self.device)
+        o2, p2, fl, _ = _e.apply_moves([own], [opp], [int(row) * 8 + int(col)], n, self.device, rules=self.rules)
         fl = int(fl[0])
         if fl & 0x80000000:
             # the reference does not validate: it places the disc and flips nothing (:237-247)
@@ -198,27 +203,27 @@ class OthelloGame:
     def is_valid_player_action(board, player, row, col):
         return bool((OthelloGame.legal_mask(board, player) >> (int(row) * 8 + int(col))) & 1)
 
-    @staticmethod
-    def get_action_flip_squares(board, player, row, col):
+    @classmethod
+    def get_action_flip_squares(cls, board, player, row, col):
         """The SET of flipped squares in row-major order (the reference's generator also yields duplicates,
-        :216-235; every consumer only uses membership)."""
+        :216-235; every consumer only uses membership), under ``cls.rules``."""
         n = np.asarray(board).shape[0]
         own, opp = OthelloGame._own_opp(board, player)
         sq = int(row) * 8 + int(col)
         if (own | opp) >> sq & 1:
             return iter(())
-        o2, p2, fl, _ = _e.apply_moves([own], [opp], [sq], n, OthelloGame.device)
+        o2, p2, fl, _ = _e.apply_moves([own], [opp], [sq], n, cls.device, rules=cls.rules)
         if int(fl[0]) & 0x80000000:
             return iter(())
         mover = int(p2[0]) if int(fl[0]) & MOVE_SWAPPED else int(o2[0])
         flipped = mover & ~own & ~(1 << sq)
         return iter(_mask_to_squares(flipped, n))
 
-    @staticmethod
-    def flip_board_squares(board, player, row, col):
+    @classmethod
+    def flip_board_squares(cls, board, player, row, col):
         """:237-247, in place: the flipped squares and the played square go to `player`'s channel."""
-        mine = OthelloGame.PLAYER_CHANNELS[player]
-        squares = list(OthelloGame.get_action_flip_squares(board, player, row, col)) + [(row, col)]
+        mine = cls.PLAYER_CHANNELS[player]
+        squares = list(cls.get_action_flip_squares(board, player, row, col)) + [(row, col)]
         rr, cc = zip(*squares)
         board[rr, cc, mine] = True
         board[rr, cc, 1 - mine] = False
@@ -266,11 +271,11 @@ class OthelloGame:
             out[r, c] = 1
         return out
 
-    @staticmethod
-    def getNextState(board, player, action):
-        """-> (next_board, next_player) with OthelloGame.play's pass handling."""
+    @classmethod
+    def getNextState(cls, board, player, action):
+        """-> (next_board, next_player) with OthelloGame.play's pass handling, under ``cls.rules``."""
         b = np.array(board, copy=True)
-        g = OthelloGame(b.shape[0], initial_board=b, current_player=player)
+        g = cls(b.shape[0], initial_board=b, current_player=player)
         g._has_finished = False
         g.play(*action)
         return g.board(BoardView.TWO_CHANNELS), g.current_player
@@ -285,3 +290,9 @@ class OthelloGame:
     @staticmethod
     def getCanonicalForm(board, player):
         return OthelloGame.invert_board(board) if player is OthelloPlayer.WHITE else board
+
+
+class StandardOthelloGame(OthelloGame):
+    """OthelloGame with standard Othello flipping: a run of opponent discs flips only up to the first own disc beyond
+    it.  Legal moves, passes, the end of the game and the scoring (a draw counts as a BLACK win) are unchanged."""
+    rules = "standard"

@@ -8,6 +8,7 @@ returns the reference's list of ``(board (N,N,2) bool, one-hot policy (N,N) floa
 symmetries of training.py:13-23 in the reference's order.  Differences, all documented in INTEGRATION.md:
 boards are true per-move snapshots unless ``reference_aliasing=True`` (the reference aliases the live board,
 SURVEY §0.8); with e_greedy < 1 the random moves come from the engine's counter RNG, not CPython's.
+Every entry point takes ``rules="reference"`` (the reference's flip rule) or ``rules="standard"`` (standard Othello).
 """
 from __future__ import annotations
 
@@ -46,7 +47,7 @@ class SelfPlay:
 
     def __init__(self, board_size: int, neural_network, degree_exploration: float = 1.0, max_games: int = 4096,
                  num_simulations: int = 100, device: int = 0, seed: int = 0, log_visits: bool = False,
-                 eval_cache_log2: int = 22):
+                 eval_cache_log2: int = 22, rules: str = "reference"):
         self.board_size = board_size
         self.num_simulations = num_simulations
         if isinstance(neural_network, HashPriorNet):
@@ -61,7 +62,7 @@ class SelfPlay:
                                 c_puct=float(degree_exploration), seed=seed, device=device, log_visits=log_visits,
                                 # identical positions reached by different games are evaluated once (results unchanged:
                                 # tests/test_gpu_net.py::test_eval_cache_is_results_preserving); 272 B per entry
-                                eval_cache_log2=eval_cache_log2 if mode == _e.PRIOR_NET else 0)
+                                eval_cache_log2=eval_cache_log2 if mode == _e.PRIOR_NET else 0, rules=rules)
         if mode == _e.PRIOR_NET:
             self.engine.load_weights(neural_network.blob, neural_network.channels)
 
@@ -177,7 +178,7 @@ def allocate_game_ids(n: int) -> np.ndarray:
 
 def execute_episodes(n_episodes, board_size, neural_network, degree_exploration, num_simulations, policy_temperature,
                      e_greedy, device: int = 0, seed: int | None = None, reference_aliasing: bool = False, game_ids=None,
-                     max_concurrent: int = 4096):
+                     max_concurrent: int = 4096, rules: str = "reference"):
     """n_episodes x training.execute_episode as one GPU job; returns a list of example lists.  At most `max_concurrent`
     episodes are in flight (node pools are per slot); the others are queued on the device and start as slots free up.
     policy_temperature may be 0 (main.py:73-76 switches to it after `temperature_threshold` iterations)."""
@@ -186,7 +187,7 @@ def execute_episodes(n_episodes, board_size, neural_network, degree_exploration,
     if game_ids is None:
         game_ids = allocate_game_ids(n_episodes)
     sp = SelfPlay(board_size, neural_network, degree_exploration, max_games=min(n_episodes, max_concurrent),
-                  num_simulations=num_simulations, device=device, seed=seed)
+                  num_simulations=num_simulations, device=device, seed=seed, rules=rules)
     try:
         rec = sp.play(n_episodes, policy_temperature, e_greedy, game_ids=game_ids)
     finally:
@@ -236,17 +237,19 @@ class Worker:
         return f'{self.__class__.__name__}-{str(uuid.uuid4()).split("-", 1)[0]}'
 
 
-def make_b200_worker(worker_base=Worker, device: int = 0, seed: int | None = None):
+def make_b200_worker(worker_base=Worker, device: int = 0, seed: int | None = None, rules: str = "reference"):
     """Builds a ``B200Worker`` class deriving from ``worker_base`` — pass the reference's ``workers.Worker`` so that
     ``WorkerManager.add_worker``'s isinstance check (workers.py:186-190) accepts it.  seed=None (default): the
     process-wide OS-drawn seed; game ids always come from the process-wide allocator, so every run() of every worker
-    plays episodes nobody has played before (see allocate_game_ids)."""
+    plays episodes nobody has played before (see allocate_game_ids).  ``rules`` is the rule set of every work type."""
+    _e.board_arg(8, rules)  # unknown rule sets fail here, not in the worker thread
 
     class B200Worker(worker_base):
         def __init__(self):
             super().__init__()
             self.device = device
             self.seed = seed
+            self.rules = rules
 
         def _run(self, work_type, iterations, args, kwargs):
             # workers.py:57-65 runs the target once per iteration; here all iterations are one GPU batch and
@@ -255,30 +258,33 @@ def make_b200_worker(worker_base=Worker, device: int = 0, seed: int | None = Non
             # WorkType class must match too, hence ==)
             if work_type == WorkType.EXECUTE_EPISODE:
                 logging.info(f'Task {work_type}: {iterations} episodes as one GPU job on cuda:{self.device}')
-                results = execute_episodes(iterations, *args, device=self.device, seed=self.seed, **kwargs)
+                results = execute_episodes(iterations, *args, device=self.device, seed=self.seed, rules=self.rules,
+                                           **kwargs)
             elif work_type == WorkType.DUEL_BETWEEN_NEURAL_NETWORKS:
                 from . import arena
                 logging.info(f'Task {work_type}: {iterations} duels as one GPU batch on cuda:{self.device}')
-                results = arena.duels_between_neural_networks(iterations, *args, device=self.device, **kwargs)
+                results = arena.duels_between_neural_networks(iterations, *args, device=self.device, rules=self.rules,
+                                                              **kwargs)
             elif work_type == WorkType.EVALUATE_NEURAL_NETWORK:
                 from . import arena
                 logging.info(f'Task {work_type}: {iterations} evaluations as one GPU batch on cuda:{self.device}')
-                results = arena.evaluate_neural_network(*args, device=self.device, repeats=iterations, **kwargs)
+                results = arena.evaluate_neural_network(*args, device=self.device, repeats=iterations,
+                                                        rules=self.rules, **kwargs)
                 results = results if isinstance(results, list) else [results]
             else:
                 raise TypeError('expecting WorkType object')
             self._results.extend(results)
 
         def execute_episode(self, *args, **kwargs):
-            return execute_episode(*args, device=self.device, seed=self.seed, **kwargs)
+            return execute_episode(*args, device=self.device, seed=self.seed, rules=self.rules, **kwargs)
 
         def duel_between_neural_networks(self, *args, **kwargs):
             from . import arena
-            return arena.duels_between_neural_networks(1, *args, device=self.device, **kwargs)[0]
+            return arena.duels_between_neural_networks(1, *args, device=self.device, rules=self.rules, **kwargs)[0]
 
         def evaluate_neural_network(self, *args, **kwargs):
             from . import arena
-            return arena.evaluate_neural_network(*args, device=self.device, **kwargs)
+            return arena.evaluate_neural_network(*args, device=self.device, rules=self.rules, **kwargs)
 
     return B200Worker
 
