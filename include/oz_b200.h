@@ -23,10 +23,17 @@
  *     `break`).  OR-ing OZ_RULES_STANDARD into a board_size argument selects standard Othello
  *     flipping (a run flips only up to the first own disc) for oz_rules_apply_*,
  *     oz_perft_playouts_* and oz_engine_config.board_size (search and self-play).  Legal moves, the
- *     initial position, the automatic pass, the terminal test and the scoring (a draw counts as a
- *     BLACK win) are the same under both rule sets; oz_rules_legal_moves_* and oz_net_blob_floats
- *     accept the flag and ignore it, so one value can be passed everywhere.  Any other bit above
- *     the size is OZ_ERR_INVALID.
+ *     initial position, the automatic pass, the terminal test and the scoring are the same under
+ *     both rule sets; oz_rules_legal_moves_* and oz_net_blob_floats accept the flag and ignore it,
+ *     so one value can be passed everywhere.
+ *   - Scoring.  By default a finished game with equal disc counts counts as a BLACK win (the
+ *     reference's max() over {BLACK, WHITE}, Othello/__init__.py:254-256).  OR-ing
+ *     OZ_SCORING_STANDARD into oz_engine_config.board_size scores it as a draw, independently of the
+ *     rule set: the search backs a drawn terminal up as the integer 0, and self-play records winner
+ *     OZ_WINNER_DRAW.  Empty squares left over are not counted.  oz_rules_legal_moves_*,
+ *     oz_rules_apply_*, oz_perft_playouts_* and oz_net_blob_floats accept the flag and ignore it
+ *     (nothing they compute depends on the scoring).  Any other bit above the size is
+ *     OZ_ERR_INVALID.
  *   - Passes and perft.  A side with no legal move passes automatically inside the move that left
  *     it without one: a pass is not a move of its own and does not use up a ply.  A full-tree perft
  *     counted with these calls therefore treats a finished game as a leaf and a pass as free, e.g.
@@ -52,6 +59,11 @@ extern "C" {
 
 /* OR-ed into a board_size argument: standard Othello flipping instead of the reference's (see Conventions) */
 #define OZ_RULES_STANDARD 0x100
+/* OR-ed into a board_size argument: a finished game with equal disc counts is a draw, not a BLACK win (see Conventions).
+ * 0x200 is not used: it stays OZ_ERR_INVALID everywhere. */
+#define OZ_SCORING_STANDARD 0x400
+/* self-play winner code of a drawn game under OZ_SCORING_STANDARD (oz_selfplay_get_records) */
+#define OZ_WINNER_DRAW 2
 
 /* flags returned by oz_rules_apply_* (one uint32 per position) */
 #define OZ_MOVE_SWAPPED 1u  /* opponent moves next; outputs are in HIS frame (own/opp swapped) */
@@ -75,7 +87,8 @@ typedef struct oz_engine oz_engine;
 typedef struct oz_engine_config {
     int32_t device;          /* CUDA ordinal */
     int32_t board_size;      /* 4, 6 or 8 (Othello/__init__.py:29-36; the net needs 6 or 8), | OZ_RULES_STANDARD for
-                                standard flipping in simulations and self-play moves */
+                                standard flipping in simulations and self-play moves, | OZ_SCORING_STANDARD for drawn
+                                games scored as draws in the search and in self-play winners */
     int32_t max_games;       /* concurrent game slots (one warp each) */
     int32_t nodes_per_game;  /* node-pool capacity per game; reference keeps every node of an episode
                                 (training.py:32), i.e. <= sims * plies */
@@ -189,7 +202,8 @@ int oz_selfplay_begin(oz_engine* e, int32_t n_games, const uint64_t* black, cons
 int oz_selfplay_run(oz_engine* e, int32_t steps, int32_t* n_active);
 /* Per-move records of EVERY game of the job (queued ones included, indexed by game), HOST buffers sized [n_games][64]
  * (rec_visits [n_games][64][64], may be NULL unless log_visits): position before the move as black/white bitboards, action square bit, mover; n_moves,
- * winner (0 BLACK / 1 WHITE, draw -> BLACK, Othello/__init__.py:254-256; -1 unfinished) per game.
+ * winner (0 BLACK / 1 WHITE, draw -> BLACK, Othello/__init__.py:254-256; under OZ_SCORING_STANDARD a draw is
+ * OZ_WINNER_DRAW (2); -1 unfinished) per game.
  * Entry n_moves[g] (< 64) of rec_black/rec_white[g] holds the position the episode ended in (the board every example
  * of the reference aliases, training.py:63). */
 int oz_selfplay_get_records(oz_engine* e, uint64_t* rec_black, uint64_t* rec_white, uint8_t* rec_action,

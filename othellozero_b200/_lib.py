@@ -14,14 +14,20 @@ MOVE_SWAPPED, MOVE_PASSED, MOVE_FINISHED = 1, 2, 4
 GAME_IDLE, GAME_ACTIVE, GAME_WAIT_LEAF, GAME_FINISHED, GAME_POOL_FULL = 0, 1, 2, 3, 4
 RULES_STANDARD = 0x100  # OZ_RULES_STANDARD, OR-ed into a board_size argument
 RULES = ("reference", "standard")
+SCORING_STANDARD = 0x400  # OZ_SCORING_STANDARD, OR-ed into a board_size argument
+SCORINGS = ("reference", "standard")
+WINNER_DRAW = 2  # OZ_WINNER_DRAW: self-play winner code of a drawn game under standard scoring
 
 
-def board_arg(board_size: int, rules: str = "reference") -> int:
+def board_arg(board_size: int, rules: str = "reference", scoring: str = "reference") -> int:
     """The C-ABI board_size argument for a rule set: "reference" (the reference's flip rule, the default) or
-    "standard" (standard Othello flipping).  Anything else raises ValueError."""
+    "standard" (standard Othello flipping), and a scoring: "reference" (a draw counts as a BLACK win, the default) or
+    "standard" (a draw is a draw).  Anything else raises ValueError."""
     if rules not in RULES:
         raise ValueError(f"rules must be one of {RULES}, got {rules!r}")
-    return board_size | (RULES_STANDARD if rules == "standard" else 0)
+    if scoring not in SCORINGS:
+        raise ValueError(f"scoring must be one of {SCORINGS}, got {scoring!r}")
+    return board_size | (RULES_STANDARD if rules == "standard" else 0) | (SCORING_STANDARD if scoring == "standard" else 0)
 
 
 class EngineConfig(C.Structure):

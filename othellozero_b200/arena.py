@@ -12,7 +12,9 @@
 The reference's own drivers ``training.duel_between_neural_networks`` / ``evaluate_neural_network`` are broken
 (SURVEY §0.8); ``pit`` follows the working semantics of main.py:165-197 (who won, counted per game).
 ``rules="standard"`` plays every game of a batched driver under standard Othello flipping; the per-game agents take the
-rule set from their game (``othello.StandardOthelloGame``).
+rule set from their game (``othello.StandardOthelloGame``).  ``scoring="standard"`` scores a game with equal disc counts
+as a draw (winner code 2, no win for either side) in the search and in the result; the per-game agents take it from
+their game too (``othello.game_class``).
 """
 from __future__ import annotations
 
@@ -21,6 +23,7 @@ import random
 import numpy as np
 
 from . import engine as _e
+from ._lib import WINNER_DRAW
 from .mcts import HashPriorNet, OthelloMCTS
 from .net import B200NNet
 from .othello import BoardView, OthelloGame, OthelloPlayer
@@ -50,7 +53,8 @@ class NeuralNetworkOthelloAgent(OthelloAgent):
         self.temperature = 0
         self.neural_network = neural_network
         self.num_simulations = num_simulations
-        self.mcts = OthelloMCTS(game.board_size, neural_network, degree_exploration, rules=game.rules)
+        self.mcts = OthelloMCTS(game.board_size, neural_network, degree_exploration, rules=game.rules,
+                                scoring=game.scoring)
         super().__init__(game)
 
     def play(self):
@@ -65,12 +69,13 @@ class NeuralNetworkOthelloAgent(OthelloAgent):
 
 
 def duel_between_agents(game, agent_1, agent_2):
-    """agents.py:71-84: agent_1 is BLACK, agent_2 WHITE; returns (winning agent, points)."""
+    """agents.py:71-84: agent_1 is BLACK, agent_2 WHITE; returns (winning agent, points), the agent None for a draw
+    under standard scoring."""
     players_agents = {OthelloPlayer.BLACK: agent_1, OthelloPlayer.WHITE: agent_2}
     while not game.has_finished():
         players_agents[game.current_player].play()
     winner, points = game.get_winning_player()
-    return players_agents[winner], points
+    return players_agents.get(winner), points
 
 
 RANDOM_AGENT = "random"   # a side of pit() that plays RandomOthelloAgent's policy (agents.py:20-24)
@@ -110,15 +115,17 @@ def _draw_indices(rng, counts: np.ndarray) -> np.ndarray:
 
 
 def pit(board_size, net_black, net_white, num_simulations, degree_exploration=1, n_games=64, device=0, rng=None,
-        start_black=None, start_white=None, start_player=None, rules="reference"):
-    """n_games simultaneous duels, net_black playing BLACK.  Returns dict(winner [n_games] 0/1, black, white, plies).
+        start_black=None, start_white=None, start_player=None, rules="reference", scoring="reference"):
+    """n_games simultaneous duels, net_black playing BLACK.  Returns dict(winner [n_games] 0/1, black, white, plies,
+    points, draws [n_games] bool: equal final counts).  Under reference scoring a draw is a BLACK win (winner 0); under
+    ``scoring="standard"`` its winner is 2, and both searches value drawn terminals as 0.
     Every step is one kernel chain over all games whose turn it is: one search launch per network side
     (NeuralNetworkOthelloAgent.play, agents.py:52-68, always temperature 0), one move-generator launch for a
     ``RANDOM_AGENT`` side (RandomOthelloAgent.play, agents.py:20-24; main.py:165-197 evaluates the network against it),
     one rules launch to apply the moves.  Ties in the visit counts and the random agent's moves are drawn from ``rng``
     (Python's ``random`` like the reference, or a numpy Generator for fully vectorised draws) over the candidates in
     row-major order.  Both sides search, and every move is applied, under ``rules``."""
-    _e.board_arg(board_size, rules)
+    _e.board_arg(board_size, rules, scoring)
     rng = rng or random
     n = board_size
     nodes = num_simulations * (n * n) + 64
@@ -129,7 +136,7 @@ def pit(board_size, net_black, net_white, num_simulations, degree_exploration=1,
             continue
         mode = _mode_for(net)
         e = _e.Engine(n, max_games=n_games, nodes_per_game=nodes, prior_mode=mode, c_puct=float(degree_exploration),
-                      device=device, rules=rules)
+                      device=device, rules=rules, scoring=scoring)
         if mode == _e.PRIOR_NET:
             e.load_weights(net.blob, net.channels)
         engines.append(e)
@@ -183,28 +190,34 @@ def pit(board_size, net_black, net_white, num_simulations, degree_exploration=1,
             if e is not None:
                 e.close()
     cb, cw = _e.score(black, white, device)
-    return dict(winner=np.where(cb >= cw, 0, 1), black=black, white=white, plies=plies, points=np.maximum(cb, cw))
+    draws = cb == cw
+    winner = np.where(cb >= cw, 0, 1)
+    if scoring == "standard":
+        winner = np.where(draws, WINNER_DRAW, winner)
+    return dict(winner=winner, black=black, white=white, plies=plies, points=np.maximum(cb, cw), draws=draws)
 
 
 # ---- batched arena drivers (the worker work types of workers.py:18-21,72-79) -----------------------------------------
 def duels_between_neural_networks(n_duels, board_size, neural_network_1, neural_network_2, degree_exploration,
-                                  num_simulations, device=0, rng=None, rules="reference"):
+                                  num_simulations, device=0, rng=None, rules="reference", scoring="reference"):
     """``n_duels`` x training.duel_between_neural_networks (training.py:75-89) as one batch: network 1 plays BLACK
-    (agent_1 of duel_between_agents, agents.py:71-74); each entry is 0 if network 1 won, else 1."""
+    (agent_1 of duel_between_agents, agents.py:71-74); each entry is 0 if network 1 won, 1 if network 2 won, and 2 for a
+    draw under standard scoring."""
     out = pit(board_size, neural_network_1, neural_network_2, num_simulations, degree_exploration, n_games=n_duels,
-              device=device, rng=rng, rules=rules)
+              device=device, rng=rng, rules=rules, scoring=scoring)
     return [int(w) for w in out["winner"]]
 
 
 def evaluate_neural_network(board_size, total_iterations, neural_network, num_simulations, degree_exploration,
                             agent_class=RandomOthelloAgent, agent_arguments=(), device=0, rng=None, repeats=1,
-                            rules="reference"):
+                            rules="reference", scoring="reference"):
     """training.evaluate_neural_network (training.py:92-115) with the working semantics of main.py:165-197: the network
     meets ``agent_class`` (RandomOthelloAgent) in ``total_iterations`` games, colours shuffled per game; returns the
-    network's wins.  ``repeats`` > 1 plays that many evaluations in the same batch and returns a list of win counts."""
+    network's wins (a draw under standard scoring is not a win).  ``repeats`` > 1 plays that many evaluations in the
+    same batch and returns a list of win counts."""
     if agent_class is not RandomOthelloAgent:
         raise TypeError("the batched evaluation plays against RandomOthelloAgent (main.py:165-197)")
-    _e.board_arg(board_size, rules)
+    _e.board_arg(board_size, rules, scoring)
     rng = rng or random
     games = total_iterations * repeats
     net_is_black = np.array([rng.random() < 0.5 for _ in range(games)], dtype=bool)   # random.shuffle of two agents
@@ -215,7 +228,7 @@ def evaluate_neural_network(board_size, total_iterations, neural_network, num_si
             continue
         a, b = (neural_network, RANDOM_AGENT) if black_side else (RANDOM_AGENT, neural_network)
         out = pit(board_size, a, b, num_simulations, degree_exploration, n_games=int(sel.size), device=device, rng=rng,
-                  rules=rules)
+                  rules=rules, scoring=scoring)
         net_won[sel] = out["winner"] == (0 if black_side else 1)
     wins = net_won.reshape(repeats, total_iterations).sum(axis=1)
     return int(wins[0]) if repeats == 1 else [int(w) for w in wins]

@@ -63,8 +63,8 @@ __global__ void validate_starts_kernel(int n_games, const u64* __restrict__ blac
 extern "C" int oz_engine_create(const oz_engine_config* cfg, oz_engine** out) {
     OZ_REQUIRE(cfg && out, "null argument");
     *out = nullptr;
-    int size, rules;
-    if (oz_decode_board(cfg->board_size, &size, &rules)) return OZ_ERR_INVALID;
+    int size, rules, scoring;
+    if (oz_decode_board(cfg->board_size, &size, &rules, &scoring)) return OZ_ERR_INVALID;
     OZ_REQUIRE(cfg->max_games >= 1 && cfg->max_games <= (1 << 20), "max_games out of range: %d", cfg->max_games);
     OZ_REQUIRE(cfg->nodes_per_game >= 2 && cfg->nodes_per_game <= (1 << 22), "nodes_per_game out of range: %d",
                cfg->nodes_per_game);
@@ -83,6 +83,7 @@ extern "C" int oz_engine_create(const oz_engine_config* cfg, oz_engine** out) {
     e->cfg = *cfg;
     e->cfg.board_size = size;
     e->rules = rules;
+    e->scoring = scoring;
     cudaError_t err = cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking);
     if (err != cudaSuccess) {
         oz_set_error("cudaStreamCreate failed: %s", cudaGetErrorString(err));
@@ -497,7 +498,7 @@ extern "C" int oz_selfplay_get_positions(oz_engine* e, uint64_t* black, uint64_t
 
 // ---- network ----------------------------------------------------------------------------------------
 extern "C" int64_t oz_net_blob_floats(int32_t board_size, int32_t channels) {
-    int size;  // the network does not depend on the rule set: the rules flag is accepted and ignored
+    int size;  // the network depends on neither the rule set nor the scoring: both flags are accepted and ignored
     if (oz_decode_board(board_size, &size, nullptr)) return -1;
     return oz_net_blob_floats_impl(size, channels);
 }

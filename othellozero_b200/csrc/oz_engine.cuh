@@ -29,16 +29,23 @@ void oz_set_error(const char* fmt, ...);
         }                            \
     } while (0)
 
-// The board_size argument of the C-ABI: N (4, 6 or 8), optionally | OZ_RULES_STANDARD.  -> N and the ozbb rule set
-// (either output may be null); any other bit is OZ_ERR_INVALID.  Only the C-ABI entry points see the flag.
-inline int oz_decode_board(int32_t board_size, int* n, int* rules) {
-    const int size = board_size & ~OZ_RULES_STANDARD;
+// Scorings of the tree kernel (instantiated per scoring, chosen at launch): REFERENCE counts a draw as a BLACK win,
+// STANDARD scores it as a draw (value 0, winner code OZ_WINNER_DRAW).
+enum : int { SCORING_REFERENCE = 0, SCORING_STANDARD = 1 };
+
+// The board_size argument of the C-ABI: N (4, 6 or 8), optionally | OZ_RULES_STANDARD | OZ_SCORING_STANDARD.  -> N, the
+// ozbb rule set and the scoring (any output may be null); any other bit is OZ_ERR_INVALID.  Only the C-ABI entry points
+// see the flags.
+inline int oz_decode_board(int32_t board_size, int* n, int* rules, int* scoring = nullptr) {
+    const int size = board_size & ~(OZ_RULES_STANDARD | OZ_SCORING_STANDARD);
     if (size != 4 && size != 6 && size != 8) {
-        oz_set_error("board_size must be 4, 6 or 8, optionally | OZ_RULES_STANDARD (got %d)", board_size);
+        oz_set_error("board_size must be 4, 6 or 8, optionally | OZ_RULES_STANDARD | OZ_SCORING_STANDARD (got %d)",
+                     board_size);
         return OZ_ERR_INVALID;
     }
     if (n) *n = size;
     if (rules) *rules = (board_size & OZ_RULES_STANDARD) ? ozbb::RULES_STANDARD : ozbb::RULES_REFERENCE;
+    if (scoring) *scoring = (board_size & OZ_SCORING_STANDARD) ? SCORING_STANDARD : SCORING_REFERENCE;
     return OZ_OK;
 }
 
@@ -62,6 +69,7 @@ constexpr int OZ_CH_UNKNOWN = -1;   // edge never traversed
 constexpr int OZ_CH_TERM_NEG = -2;  // child is terminal, simulate() returns -1
 constexpr int OZ_CH_TERM_POS = -3;  // child is terminal, simulate() returns +1
 constexpr int OZ_CH_PENDING = -4;   // leaf emitted by the current virtual-loss wave, not expanded yet
+constexpr int OZ_CH_TERM_DRAW = -5; // child is a drawn terminal, simulate() returns 0 (standard scoring only)
 constexpr int OZ_MAX_DEPTH = 64;
 
 struct OzTreeParams {
@@ -113,8 +121,9 @@ struct OzTreeParams {
 struct OzNet;  // oz_net.cu
 
 struct oz_engine {
-    oz_engine_config cfg;      // cfg.board_size holds plain N; the rules flag of the caller's value is in `rules`
+    oz_engine_config cfg;      // cfg.board_size holds plain N; the flags of the caller's value are in `rules`, `scoring`
     int rules = ozbb::RULES_REFERENCE;
+    int scoring = SCORING_REFERENCE;
     cudaStream_t stream = nullptr;
     OzTreeParams tp{};
     int n_games = 0;

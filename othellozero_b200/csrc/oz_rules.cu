@@ -100,7 +100,7 @@ static int grid_for(long long n, int block) {
 
 extern "C" int oz_rules_legal_moves_dev(int32_t board_size, const uint64_t* own, const uint64_t* opp,
                                         uint64_t* moves, int64_t n, void* stream) {
-    int size;  // legal moves are the same under both rule sets: the flag is accepted and ignored
+    int size;  // legal moves are the same under every rule set and scoring: the flags are accepted and ignored
     if (oz_decode_board(board_size, &size, nullptr)) return OZ_ERR_INVALID;
     if (n <= 0) return OZ_OK;
     rules_legal_kernel<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>((const u64*)own, (const u64*)opp,

@@ -63,8 +63,9 @@ __device__ __forceinline__ u64 key_hash(u64 own, u64 opp) {
 // which is what keeps the kernel's hot loops inside the instruction cache (round 1: ~10.3 K SASS instructions, fetch
 // stalls on top of the stall list).
 // ... and they use the looped compact forms of oz_bitboard.cuh (a quarter of the unrolled templates' code, same issue count).
-// The rule set is a template parameter of the kernel (one instantiation per rule set, chosen at launch), never a
-// run-time branch, so the reference instantiation carries no cost for the standard rule (tools/sass_compare.py).
+// The rule set and the scoring are template parameters of the kernel (one instantiation per combination, chosen at
+// launch), never run-time branches, so the reference instantiations carry no cost for the standard variants
+// (tools/sass_compare.py).
 template <int RULES>
 __device__ __noinline__ u64 flip_mask_call(u64 m, u64 own, u64 opp) {
     if constexpr (RULES == RULES_STANDARD) return flip_mask_standard_compact(m, own, opp);
@@ -424,7 +425,7 @@ __device__ __noinline__ double ucb_value_call(int nraw, double q, double pj, dou
 #ifndef OZ_TREE_MIN_CTAS
 #define OZ_TREE_MIN_CTAS 7
 #endif
-template <int RULES>
+template <int RULES, int SCORING>
 __global__ void __launch_bounds__(TREE_WARPS * 32, OZ_TREE_MIN_CTAS) tree_step_kernel(const OzTreeParams P) {
     __shared__ double s_a[TREE_WARPS][72];  // [0,64): masked priors of the node being expanded, [64,72): its partial sums
     const int lane = threadIdx.x & 31;
@@ -579,7 +580,12 @@ __global__ void __launch_bounds__(TREE_WARPS * 32, OZ_TREE_MIN_CTAS) tree_step_k
                 const bool over = (fl & MOVE_FINISHED) != 0;
                 if (over || (P.max_moves >= 0 && ply >= P.max_moves)) {
                     if (lane == 0) {
-                        P.winner[gi] = over ? ((popc(black) >= popc(white)) ? 0 : 1) : -1;
+                        if constexpr (SCORING == SCORING_STANDARD) {
+                            const int nb = popc(black), nw = popc(white);
+                            P.winner[gi] = over ? (nb > nw ? 0 : (nb < nw ? 1 : OZ_WINNER_DRAW)) : -1;
+                        } else {
+                            P.winner[gi] = over ? ((popc(black) >= popc(white)) ? 0 : 1) : -1;
+                        }
                         if (ply < 64) {  // entry n_moves of a game's record row = the position the episode ended in
                             P.rec_black[(size_t)gi * 64 + ply] = black; P.rec_white[(size_t)gi * 64 + ply] = white;
                         }
@@ -679,6 +685,9 @@ __global__ void __launch_bounds__(TREE_WARPS * 32, OZ_TREE_MIN_CTAS) tree_step_k
                     outcome = 1;
                     break;
                 }
+                if constexpr (SCORING == SCORING_STANDARD) {
+                    if (ch == OZ_CH_TERM_DRAW) { term_val = 0; outcome = 1; break; }
+                }
                 // frontier: get_next_state (othelo_mcts.py:43-49)
                 u64 own = h->own, opp = h->opp;
                 const int sq = warp_kth_set_bit(h->legal, bj, lane);
@@ -686,9 +695,16 @@ __global__ void __launch_bounds__(TREE_WARPS * 32, OZ_TREE_MIN_CTAS) tree_step_k
                 const unsigned fl = play_move_dev<RULES>(1ull << sq, own, opp, P.full, nl);
                 if (fl & MOVE_FINISHED) {
                     // is_terminal_state -> return -reward; reward = +1 iff ch0 count >= ch1 count (draw -> BLACK)
-                    int reward = (popc(own) >= popc(opp)) ? 1 : -1;
-                    term_val = -reward;
-                    if (lane == 0) Cp[bj] = (term_val > 0) ? OZ_CH_TERM_POS : OZ_CH_TERM_NEG;
+                    if constexpr (SCORING == SCORING_STANDARD) {
+                        // ... except that equal counts are a draw: reward 0, backed up as the integer 0
+                        const int a = popc(own), b = popc(opp);
+                        term_val = (a > b) ? -1 : (a < b ? 1 : 0);
+                        if (lane == 0) Cp[bj] = (term_val > 0) ? OZ_CH_TERM_POS : (term_val < 0 ? OZ_CH_TERM_NEG : OZ_CH_TERM_DRAW);
+                    } else {
+                        int reward = (popc(own) >= popc(opp)) ? 1 : -1;
+                        term_val = -reward;
+                        if (lane == 0) Cp[bj] = (term_val > 0) ? OZ_CH_TERM_POS : OZ_CH_TERM_NEG;
+                    }
                     outcome = 1;
                     break;
                 }
@@ -1061,7 +1077,11 @@ int oz_tree_reset(oz_engine* e, int n_games, const u64* black, const u64* white,
 int oz_tree_step(oz_engine* e) {
     OzTreeParams& P = e->tp;
     int blocks = (P.G + TREE_WARPS - 1) / TREE_WARPS;
-    auto kernel = e->rules == RULES_STANDARD ? tree_step_kernel<RULES_STANDARD> : tree_step_kernel<RULES_REFERENCE>;
+    auto kernel = e->rules == RULES_STANDARD
+                      ? (e->scoring == SCORING_STANDARD ? tree_step_kernel<RULES_STANDARD, SCORING_STANDARD>
+                                                        : tree_step_kernel<RULES_STANDARD, SCORING_REFERENCE>)
+                      : (e->scoring == SCORING_STANDARD ? tree_step_kernel<RULES_REFERENCE, SCORING_STANDARD>
+                                                        : tree_step_kernel<RULES_REFERENCE, SCORING_REFERENCE>);
     kernel<<<blocks, TREE_WARPS * 32, 0, e->stream>>>(P);
     OZ_CUDA(cudaGetLastError());
     e->launches++;

@@ -87,15 +87,19 @@ def probe_l2_read(megabytes: int = 32, passes: int = 50, device: int = 0) -> flo
 
 class Engine:
     """oz_engine handle: node pools + per-game state for `max_games` concurrent games on one GPU.  `rules` is the rule
-    set of every simulation and self-play move: "reference" (default) or "standard" Othello flipping."""
+    set of every simulation and self-play move: "reference" (default) or "standard" Othello flipping.  `scoring` is how a
+    finished game with equal disc counts is scored: "reference" (default) counts it as a BLACK win, "standard" as a draw
+    (value 0 in the search, winner code 2 in self-play records)."""
 
     def __init__(self, board_size: int = 8, max_games: int = 1, nodes_per_game: int = 8192,
                  prior_mode: int = PRIOR_HASH, c_puct: float = 1.0, seed: int = 0, device: int = 0,
-                 log_visits: bool = False, eval_cache_log2: int = 0, vl_width: int = 1, rules: str = "reference"):
-        bs = board_arg(board_size, rules)
+                 log_visits: bool = False, eval_cache_log2: int = 0, vl_width: int = 1, rules: str = "reference",
+                 scoring: str = "reference"):
+        bs = board_arg(board_size, rules, scoring)
         self._L = _lib.load()
         self.board_size = board_size
         self.rules = rules
+        self.scoring = scoring
         self.nsq = board_size * board_size
         self.max_games = max_games
         self.prior_mode = prior_mode

@@ -45,14 +45,16 @@ class IterationConfig:
     max_concurrent: int = 4096
     seed: int = 0
     rules: str = "reference"         # "standard": self-play and arena under standard Othello flipping
+    scoring: str = "reference"       # "standard": a drawn game is a draw (z = 0; no arena win for either network)
 
 
 def unpack_rows(rows: np.ndarray):
-    """dist.pack_records rows -> (black, white, action square bit, z)."""
+    """dist.pack_records rows -> (black, white, action square bit, z); z = 0 for a drawn game (winner code 2)."""
+    from ._lib import WINNER_DRAW
     rows = np.asarray(rows, dtype=np.uint64).reshape(-1, 3)
     meta = rows[:, 2].astype(np.int64)
     action, player, winner = meta & 0xFF, (meta >> 8) & 0xFF, (meta >> 16) & 0xFF
-    return rows[:, 0], rows[:, 1], action, np.where(winner == player, 1, -1)
+    return rows[:, 0], rows[:, 1], action, np.where(winner == WINNER_DRAW, 0, np.where(winner == player, 1, -1))
 
 
 def training_arrays(rows: np.ndarray, board_size: int):
@@ -118,7 +120,7 @@ class Trainer:
         if ids.size:
             sp = selfplay.SelfPlay(n, net_now, cfg.degree_exploration, max_games=min(int(ids.size), cfg.max_concurrent),
                                    num_simulations=cfg.num_simulations, device=self.local, seed=cfg.seed,
-                                   rules=cfg.rules)
+                                   rules=cfg.rules, scoring=cfg.scoring)
             rec = sp.play(int(ids.size), cfg.temperature, cfg.e_greedy, game_ids=ids)
             info["selfplay_sims_this_rank"] = sp.engine.counters()["sims"]
             sp.close()
@@ -143,20 +145,20 @@ class Trainer:
         mine_b = len(range(self.rank, cfg.arena_games - half, self.world))
         new_net = oznet.B200NNet((n, n), C, device=self.local, max_batch=8, blob=new_blob)
         old_net = oznet.B200NNet((n, n), C, device=self.local, max_batch=8, blob=self.old_blob)
-        wins = 0
+        wins = draws = 0
         rng = np.random.default_rng(cfg.seed * 1000 + self.iteration * 64 + self.rank)
-        if mine_a:
-            wins += int((arena.pit(n, new_net, old_net, cfg.arena_simulations, cfg.degree_exploration, n_games=mine_a,
-                                   device=self.local, rng=rng, rules=cfg.rules)["winner"] == 0).sum())
-        if mine_b:
-            wins += int((arena.pit(n, old_net, new_net, cfg.arena_simulations, cfg.degree_exploration, n_games=mine_b,
-                                   device=self.local, rng=rng, rules=cfg.rules)["winner"] == 1).sum())
+        for games, black_net, white_net, new_side in ((mine_a, new_net, old_net, 0), (mine_b, old_net, new_net, 1)):
+            if games:
+                out = arena.pit(n, black_net, white_net, cfg.arena_simulations, cfg.degree_exploration, n_games=games,
+                                device=self.local, rng=rng, rules=cfg.rules, scoring=cfg.scoring)
+                wins += int((out["winner"] == new_side).sum())
+                draws += int(out["draws"].sum()) if cfg.scoring == "standard" else 0
         if self.world > 1:
-            t = torch.tensor([wins], dtype=torch.int64, device=dev)
+            t = torch.tensor([wins, draws], dtype=torch.int64, device=dev)
             dist.all_reduce(t)
-            wins = int(t.item())
+            wins, draws = int(t[0].item()), int(t[1].item())
         timed("arena_s", t0)
-        promoted = wins >= cfg.arena_threshold                       # main.py:135-146
+        promoted = wins >= cfg.arena_threshold                       # main.py:135-146 (wins only: a draw is not a win)
         if promoted:
             self.old_blob = new_blob.copy()
             self.blob = new_blob
@@ -174,16 +176,19 @@ class Trainer:
         return dict(iteration=self.iteration, phases=phases, episodes=cfg.episodes, positions_gathered=int(rows.shape[0]),
                     buffer_examples=len(self.buffer), train_examples=int(arrays[0].shape[0]),
                     train_steps=cfg.epochs * ((arrays[0].shape[0] + cfg.batch_size - 1) // cfg.batch_size),
-                    train_history=hist, arena_new_wins=wins, arena_games=cfg.arena_games, promoted=bool(promoted),
+                    train_history=hist, arena_new_wins=wins, arena_draws=draws, arena_games=cfg.arena_games,
+                    promoted=bool(promoted),
                     selfplay_sims=info["selfplay_sims"],
                     selfplay_sims_per_s=info["selfplay_sims"] / max(phases["selfplay_s"], 1e-9))
 
 
 def main(argv=None):
-    from ._lib import RULES
+    from ._lib import RULES, SCORINGS
+    choices = {"rules": RULES, "scoring": SCORINGS}
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     for f, v in asdict(IterationConfig()).items():
-        ap.add_argument("--" + f.replace("_", "-"), type=type(v), default=v, **({"choices": RULES} if f == "rules" else {}))
+        ap.add_argument("--" + f.replace("_", "-"), type=type(v), default=v,
+                        **({"choices": choices[f]} if f in choices else {}))
     ap.add_argument("--iterations", type=int, default=1)
     args = ap.parse_args(argv)
     import torch

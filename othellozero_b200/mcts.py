@@ -13,7 +13,8 @@ the CUDA tree kernel.  Same constructor and method names as the reference:
   * anything with ``.predict`` (e.g. the reference's Keras NNetWrapper) -> leaves are handed to the host and
     ``predict`` is called once per expanded node, exactly as the reference does (OZ_PRIOR_HOST).
 Aliases ``search`` / ``getActionProb`` are the alpha-zero-general names used in BASELINE.json.
-``rules="standard"`` searches under standard Othello flipping instead of the reference's flip rule.
+``rules="standard"`` searches under standard Othello flipping instead of the reference's flip rule, and
+``scoring="standard"`` values a drawn terminal as 0 instead of as a BLACK win.
 """
 from __future__ import annotations
 
@@ -23,7 +24,7 @@ import numpy as np
 
 from . import engine as _e
 from .net import B200NNet, NeuralNets, bits_to_board
-from .othello import OthelloGame, OthelloPlayer, StandardOthelloGame, _bits
+from .othello import OthelloGame, OthelloPlayer, _bits, game_class
 
 
 class HashPriorNet:
@@ -36,7 +37,7 @@ class HashPriorNet:
 
 class OthelloMCTS:
     def __init__(self, board_size, neural_network, degree_exploration, nodes: int = 65536, device: int = 0,
-                 rules: str = "reference"):
+                 rules: str = "reference", scoring: str = "reference"):
         self._board_size = board_size
         self._neural_network = neural_network
         self.degree_explorarion = degree_exploration  # (sic) MCTS/__init__.py:27
@@ -51,8 +52,8 @@ class OthelloMCTS:
             mode = _e.PRIOR_HOST
         self._mode = mode
         self._eng = _e.Engine(board_size, max_games=1, nodes_per_game=nodes, prior_mode=mode,
-                              c_puct=float(degree_exploration), device=device, rules=rules)
-        self._game = StandardOthelloGame if rules == "standard" else OthelloGame
+                              c_puct=float(degree_exploration), device=device, rules=rules, scoring=scoring)
+        self._game = game_class(rules, scoring)
         if mode == _e.PRIOR_NET:
             self._eng.load_weights(neural_network.blob, neural_network.channels)
         self._eng.reset(1)
@@ -100,7 +101,8 @@ class OthelloMCTS:
         return OthelloGame.has_board_finished(state)
 
     def get_state_reward(self, state):
-        return OthelloGame.get_board_winning_player(state)[0].value
+        winner = self._game.get_board_winning_player(state)[0]
+        return 0 if winner is None else winner.value  # None: a draw under standard scoring
 
     def get_next_state(self, state, action):
         board = np.copy(state)

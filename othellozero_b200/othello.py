@@ -15,6 +15,10 @@ version raises NameError, Othello/__init__.py:88-98).
 ``OthelloGame`` plays the reference's rules, including its flip rule (a move also flips opponent discs beyond the
 bracketing own disc).  ``StandardOthelloGame`` is the same class with standard Othello flipping; the class attribute
 ``rules`` selects the rule set of ``play``, ``get_action_flip_squares``, ``flip_board_squares`` and ``getNextState``.
+Both count a draw as a BLACK win, like the reference.  The class attribute ``scoring = "standard"`` scores it as a draw
+instead: ``get_board_winning_player`` / ``get_winning_player`` return ``(None, points)`` and ``getGameEnded`` returns
+1e-4 (alpha-zero-general's small non-zero value for a draw).  ``game_class(rules, scoring)`` returns the class for any
+combination.
 """
 from __future__ import annotations
 
@@ -23,7 +27,7 @@ from enum import Enum, auto
 import numpy as np
 
 from . import engine as _e
-from ._lib import MOVE_FINISHED, MOVE_SWAPPED
+from ._lib import MOVE_FINISHED, MOVE_SWAPPED, board_arg
 
 
 class BoardView(Enum):
@@ -67,6 +71,7 @@ class OthelloGame:
     PLAYER_CHANNELS = {OthelloPlayer.BLACK: 0, OthelloPlayer.WHITE: 1}
     device = 0  # CUDA ordinal used by the static rule calls
     rules = "reference"  # flip rule of play / get_action_flip_squares / flip_board_squares / getNextState
+    scoring = "reference"  # "standard": equal counts are a draw in get_board_winning_player / getGameEnded
 
     def __init__(self, board_size=8, initial_board=None, current_player=OthelloPlayer.BLACK):
         """Othello/__init__.py:29-59: same arguments, same assertions; a supplied board is adopted (not copied)."""
@@ -159,7 +164,7 @@ class OthelloGame:
         return OthelloGame.get_board_players_points(self._board)
 
     def get_winning_player(self):
-        return OthelloGame.get_board_winning_player(self._board)
+        return self.get_board_winning_player(self._board)
 
     # ---- static array API (Othello/__init__.py:177-274) -----------------------------------------
     @staticmethod
@@ -233,10 +238,14 @@ class OthelloGame:
         return not OthelloGame.has_player_actions_on_board(board, OthelloPlayer.BLACK) and \
             not OthelloGame.has_player_actions_on_board(board, OthelloPlayer.WHITE)
 
-    @staticmethod
-    def get_board_winning_player(board):
+    @classmethod
+    def get_board_winning_player(cls, board):
+        """-> (winning OthelloPlayer, its points).  A draw goes to BLACK (dict order, :254-256), or under standard scoring
+        is (None, points)."""
         points = OthelloGame.get_board_players_points(board)
         top = max(points.values())
+        if cls.scoring == "standard" and points[OthelloPlayer.BLACK] == points[OthelloPlayer.WHITE]:
+            return None, top
         return next((player, count) for player, count in points.items() if count == top)   # draw -> BLACK (dict order)
 
     @staticmethod
@@ -280,12 +289,13 @@ class OthelloGame:
         g.play(*action)
         return g.board(BoardView.TWO_CHANNELS), g.current_player
 
-    @staticmethod
-    def getGameEnded(board):
-        """0 if not ended, else the winner's OthelloPlayer.value (draw -> BLACK)."""
+    @classmethod
+    def getGameEnded(cls, board):
+        """0 if not ended, else the winner's OthelloPlayer.value (draw -> BLACK; under standard scoring a draw is 1e-4)."""
         if not OthelloGame.has_board_finished(board):
             return 0
-        return OthelloGame.get_board_winning_player(board)[0].value
+        winner = cls.get_board_winning_player(board)[0]
+        return 1e-4 if winner is None else winner.value
 
     @staticmethod
     def getCanonicalForm(board, player):
@@ -296,3 +306,20 @@ class StandardOthelloGame(OthelloGame):
     """OthelloGame with standard Othello flipping: a run of opponent discs flips only up to the first own disc beyond
     it.  Legal moves, passes, the end of the game and the scoring (a draw counts as a BLACK win) are unchanged."""
     rules = "standard"
+
+
+_game_classes = {("reference", "reference"): OthelloGame, ("standard", "reference"): StandardOthelloGame}
+
+
+def game_class(rules: str = "reference", scoring: str = "reference") -> type:
+    """The game class for a rule set and a scoring: ``OthelloGame`` or ``StandardOthelloGame`` under reference scoring,
+    otherwise a subclass of one of them with ``scoring = "standard"`` (made once, then cached).  Unknown values raise
+    ValueError."""
+    board_arg(8, rules, scoring)
+    key = (rules, scoring)
+    if key not in _game_classes:
+        base = _game_classes[(rules, "reference")]
+        _game_classes[key] = type(base.__name__ + "StandardScoring", (base,), {
+            "scoring": scoring, "__module__": __name__,
+            "__doc__": f"{base.__name__} with standard scoring: a finished game with equal disc counts is a draw."})
+    return _game_classes[key]

@@ -8,7 +8,9 @@ returns the reference's list of ``(board (N,N,2) bool, one-hot policy (N,N) floa
 symmetries of training.py:13-23 in the reference's order.  Differences, all documented in INTEGRATION.md:
 boards are true per-move snapshots unless ``reference_aliasing=True`` (the reference aliases the live board,
 SURVEY §0.8); with e_greedy < 1 the random moves come from the engine's counter RNG, not CPython's.
-Every entry point takes ``rules="reference"`` (the reference's flip rule) or ``rules="standard"`` (standard Othello).
+Every entry point takes ``rules="reference"`` (the reference's flip rule) or ``rules="standard"`` (standard Othello),
+and ``scoring="reference"`` (a draw counts as a BLACK win) or ``scoring="standard"`` (a draw is a draw: winner code 2,
+z = 0 for every example of the game).
 """
 from __future__ import annotations
 
@@ -20,6 +22,7 @@ import uuid
 import numpy as np
 
 from . import engine as _e
+from ._lib import WINNER_DRAW
 from .mcts import HashPriorNet
 from .net import B200NNet
 
@@ -47,7 +50,7 @@ class SelfPlay:
 
     def __init__(self, board_size: int, neural_network, degree_exploration: float = 1.0, max_games: int = 4096,
                  num_simulations: int = 100, device: int = 0, seed: int = 0, log_visits: bool = False,
-                 eval_cache_log2: int = 22, rules: str = "reference"):
+                 eval_cache_log2: int = 22, rules: str = "reference", scoring: str = "reference"):
         self.board_size = board_size
         self.num_simulations = num_simulations
         if isinstance(neural_network, HashPriorNet):
@@ -62,7 +65,8 @@ class SelfPlay:
                                 c_puct=float(degree_exploration), seed=seed, device=device, log_visits=log_visits,
                                 # identical positions reached by different games are evaluated once (results unchanged:
                                 # tests/test_gpu_net.py::test_eval_cache_is_results_preserving); 272 B per entry
-                                eval_cache_log2=eval_cache_log2 if mode == _e.PRIOR_NET else 0, rules=rules)
+                                eval_cache_log2=eval_cache_log2 if mode == _e.PRIOR_NET else 0, rules=rules,
+                                scoring=scoring)
         if mode == _e.PRIOR_NET:
             self.engine.load_weights(neural_network.blob, neural_network.channels)
 
@@ -82,7 +86,8 @@ class SelfPlay:
 
 def records_to_examples(rec: dict, game: int, board_size: int, reference_aliasing: bool = False):
     """One game's records -> the reference's example list (training.py:58-72): per move the 8 symmetries of
-    (board (N,N,2) bool, one-hot policy (N,N) float64) in the order of training.py:13-23, with z = +1 iff the mover won.
+    (board (N,N,2) bool, one-hot policy (N,N) float64) in the order of training.py:13-23, with z = +1 iff the mover won
+    (z = 0 for every example of a drawn game, winner code 2, which only standard scoring records).
 
     reference_aliasing=True reproduces the reference's stream byte for byte: its examples hold VIEWS of the live board
     (training.py:63 appends np.rot90 / np.fliplr views of game.board()), so once the episode is over every example shows
@@ -100,7 +105,7 @@ def records_to_examples(rec: dict, game: int, board_size: int, reference_aliasin
         a = int(rec["action"][game][p])
         policy = np.zeros((n, n))
         policy[a >> 3][a & 7] = 1
-        z = 1 if winner == int(rec["player"][game][p]) else -1
+        z = 0 if winner == WINNER_DRAW else (1 if winner == int(rec["player"][game][p]) else -1)
         for b, pol in training_example_symmetries(board, policy):
             examples.append((b, pol, z))
     return examples
@@ -147,7 +152,8 @@ def records_to_examples_batch(rec: dict, board_size: int, games=None):
     P = int(gsel.size)
     b8, p8 = expand_symmetries(np.asarray(rec["black"])[gsel, psel], np.asarray(rec["white"])[gsel, psel],
                                np.asarray(rec["action"])[gsel, psel], n)
-    z = np.where(np.asarray(rec["winner"])[gsel] == np.asarray(rec["player"])[gsel, psel], 1, -1)
+    w = np.asarray(rec["winner"])[gsel]
+    z = np.where(w == WINNER_DRAW, 0, np.where(w == np.asarray(rec["player"])[gsel, psel], 1, -1))
     # one (board view, policy view, z) tuple per example, made by C-level iteration over the leading axis
     flat = list(zip(b8.reshape(P * 8, n, n, 2), p8.reshape(P * 8, n, n), np.repeat(np.asarray(z, dtype=np.int64), 8).tolist()))
     out, row = [], 0
@@ -178,7 +184,7 @@ def allocate_game_ids(n: int) -> np.ndarray:
 
 def execute_episodes(n_episodes, board_size, neural_network, degree_exploration, num_simulations, policy_temperature,
                      e_greedy, device: int = 0, seed: int | None = None, reference_aliasing: bool = False, game_ids=None,
-                     max_concurrent: int = 4096, rules: str = "reference"):
+                     max_concurrent: int = 4096, rules: str = "reference", scoring: str = "reference"):
     """n_episodes x training.execute_episode as one GPU job; returns a list of example lists.  At most `max_concurrent`
     episodes are in flight (node pools are per slot); the others are queued on the device and start as slots free up.
     policy_temperature may be 0 (main.py:73-76 switches to it after `temperature_threshold` iterations)."""
@@ -187,7 +193,7 @@ def execute_episodes(n_episodes, board_size, neural_network, degree_exploration,
     if game_ids is None:
         game_ids = allocate_game_ids(n_episodes)
     sp = SelfPlay(board_size, neural_network, degree_exploration, max_games=min(n_episodes, max_concurrent),
-                  num_simulations=num_simulations, device=device, seed=seed, rules=rules)
+                  num_simulations=num_simulations, device=device, seed=seed, rules=rules, scoring=scoring)
     try:
         rec = sp.play(n_episodes, policy_temperature, e_greedy, game_ids=game_ids)
     finally:
@@ -237,12 +243,14 @@ class Worker:
         return f'{self.__class__.__name__}-{str(uuid.uuid4()).split("-", 1)[0]}'
 
 
-def make_b200_worker(worker_base=Worker, device: int = 0, seed: int | None = None, rules: str = "reference"):
+def make_b200_worker(worker_base=Worker, device: int = 0, seed: int | None = None, rules: str = "reference",
+                     scoring: str = "reference"):
     """Builds a ``B200Worker`` class deriving from ``worker_base`` — pass the reference's ``workers.Worker`` so that
     ``WorkerManager.add_worker``'s isinstance check (workers.py:186-190) accepts it.  seed=None (default): the
     process-wide OS-drawn seed; game ids always come from the process-wide allocator, so every run() of every worker
-    plays episodes nobody has played before (see allocate_game_ids).  ``rules`` is the rule set of every work type."""
-    _e.board_arg(8, rules)  # unknown rule sets fail here, not in the worker thread
+    plays episodes nobody has played before (see allocate_game_ids).  ``rules`` and ``scoring`` are the rule set and the
+    scoring of every work type."""
+    _e.board_arg(8, rules, scoring)  # unknown rule sets / scorings fail here, not in the worker thread
 
     class B200Worker(worker_base):
         def __init__(self):
@@ -250,6 +258,7 @@ def make_b200_worker(worker_base=Worker, device: int = 0, seed: int | None = Non
             self.device = device
             self.seed = seed
             self.rules = rules
+            self.scoring = scoring
 
         def _run(self, work_type, iterations, args, kwargs):
             # workers.py:57-65 runs the target once per iteration; here all iterations are one GPU batch and
@@ -259,32 +268,35 @@ def make_b200_worker(worker_base=Worker, device: int = 0, seed: int | None = Non
             if work_type == WorkType.EXECUTE_EPISODE:
                 logging.info(f'Task {work_type}: {iterations} episodes as one GPU job on cuda:{self.device}')
                 results = execute_episodes(iterations, *args, device=self.device, seed=self.seed, rules=self.rules,
-                                           **kwargs)
+                                           scoring=self.scoring, **kwargs)
             elif work_type == WorkType.DUEL_BETWEEN_NEURAL_NETWORKS:
                 from . import arena
                 logging.info(f'Task {work_type}: {iterations} duels as one GPU batch on cuda:{self.device}')
                 results = arena.duels_between_neural_networks(iterations, *args, device=self.device, rules=self.rules,
-                                                              **kwargs)
+                                                              scoring=self.scoring, **kwargs)
             elif work_type == WorkType.EVALUATE_NEURAL_NETWORK:
                 from . import arena
                 logging.info(f'Task {work_type}: {iterations} evaluations as one GPU batch on cuda:{self.device}')
                 results = arena.evaluate_neural_network(*args, device=self.device, repeats=iterations,
-                                                        rules=self.rules, **kwargs)
+                                                        rules=self.rules, scoring=self.scoring, **kwargs)
                 results = results if isinstance(results, list) else [results]
             else:
                 raise TypeError('expecting WorkType object')
             self._results.extend(results)
 
         def execute_episode(self, *args, **kwargs):
-            return execute_episode(*args, device=self.device, seed=self.seed, rules=self.rules, **kwargs)
+            return execute_episode(*args, device=self.device, seed=self.seed, rules=self.rules, scoring=self.scoring,
+                                   **kwargs)
 
         def duel_between_neural_networks(self, *args, **kwargs):
             from . import arena
-            return arena.duels_between_neural_networks(1, *args, device=self.device, rules=self.rules, **kwargs)[0]
+            return arena.duels_between_neural_networks(1, *args, device=self.device, rules=self.rules,
+                                                       scoring=self.scoring, **kwargs)[0]
 
         def evaluate_neural_network(self, *args, **kwargs):
             from . import arena
-            return arena.evaluate_neural_network(*args, device=self.device, rules=self.rules, **kwargs)
+            return arena.evaluate_neural_network(*args, device=self.device, rules=self.rules, scoring=self.scoring,
+                                                 **kwargs)
 
     return B200Worker
 

@@ -75,10 +75,10 @@ def perft_leg(E, rules: str, launches: int, device: int) -> dict:
     return {"ms": ms, "plies": plies, "plies_per_s": plies / (ms * 1e-3)}
 
 
-def tree_leg(E, rules: str, device: int) -> dict:
+def tree_leg(E, rules: str, device: int, scoring: str = "reference") -> dict:
     G, sims = 4096, 100
     e = E.Engine(8, max_games=G, nodes_per_game=sims * 61 + 64, prior_mode=E.PRIOR_HASH, seed=5, device=device,
-                 rules=rules)
+                 rules=rules, scoring=scoring)
     try:
         e.selfplay_begin(G, sims, 1.0, 0.9, game_ids=np.arange(G, dtype=np.uint64))    # warm-up job
         e.selfplay_run(-1)
@@ -90,7 +90,9 @@ def tree_leg(E, rules: str, device: int) -> dict:
         e.sync()
         s = time.perf_counter() - t0
         c = e.counters()
-        return {"s": s, "sims": c["sims"], "moves": c["moves"], "sims_per_s": c["sims"] / s}
+        draws = int((e.selfplay_records()["winner"] == 2).sum())
+        return {"s": s, "sims": c["sims"], "moves": c["moves"], "terminal_visits": c["terminal_visits"], "draws": draws,
+                "sims_per_s": c["sims"] / s}
     finally:
         e.close()
 
@@ -110,12 +112,12 @@ def steady_starts(E, n_games: int, rules: str, device: int, spread: int = 57):
     return b, w, p
 
 
-def selfplay_leg(E, blob, rules: str, steps: int, warmup: int, device: int) -> dict:
+def selfplay_leg(E, blob, rules: str, steps: int, warmup: int, device: int, scoring: str = "reference") -> dict:
     G, sims, C_ = 4096, 100, 512
     total = 3 * G
     b, w, p = steady_starts(E, total, rules, device)
     e = E.Engine(8, max_games=G, nodes_per_game=sims * 61 + 64, prior_mode=E.PRIOR_NET, seed=7, device=device,
-                 eval_cache_log2=22, rules=rules)
+                 eval_cache_log2=22, rules=rules, scoring=scoring)
     try:
         e.load_weights(blob, C_)
         e.selfplay_begin(total, sims, 1.0, 0.9, -1, b, w, p, np.arange(total, dtype=np.uint64))

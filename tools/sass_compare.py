@@ -1,9 +1,11 @@
 """Compares the SASS of kernels between two builds of liboz_b200.so, instruction by instruction.
 
-Kernels are matched by demangled name with the return type and the template arguments `<0>` (the reference-rule
-instantiation, ozbb::RULES_REFERENCE) removed, so that a kernel that became `template <int RULES>` is compared with its
-pre-template self.  Instruction addresses and encodings are ignored; branch and call targets are offsets inside the
-kernel's own section, so identical code gives identical text.  Needs cuobjdump and c++filt, no GPU.
+Kernels are matched by demangled name with the return type removed, a trailing template argument `, 0` (the
+reference-scoring instantiation, SCORING_REFERENCE) dropped and then the template arguments `<0>` (the reference-rule
+instantiation, ozbb::RULES_REFERENCE) removed: a kernel that became `template <int RULES>` is compared with its
+pre-template self, and `tree_step_kernel<R, 0>` with `tree_step_kernel<R>`.  Every instantiation of a listed kernel that
+the OLD build has is compared.  Instruction addresses and encodings are ignored; branch and call targets are offsets
+inside the kernel's own section, so identical code gives identical text.  Needs cuobjdump and c++filt, no GPU.
 
 usage: python tools/sass_compare.py OLD.so NEW.so [kernel ...]
        (default kernels: tree_step_kernel rules_apply_kernel perft_playout_kernel)
@@ -37,6 +39,7 @@ def functions(so: str) -> dict[str, list[str]]:
 
 def normalize(demangled: str) -> str:
     s = re.sub(r"^void ", "", demangled)
+    s = re.sub(r"<(\d+), 0>\(", r"<\1>(", s)
     return s.replace("<0>(", "(")
 
 
@@ -45,16 +48,21 @@ def main(argv: list[str]) -> int:
     kernels = argv[3:] or DEFAULT
     ok = True
     for k in kernels:
-        o = [n for n in old if n.startswith(k + "(")]
-        if len(o) != 1 or o[0] not in new:
-            print(f"{k}: not found once in both builds (old {o})")
+        names = sorted(n for n in old if n.startswith(k + "(") or n.startswith(k + "<"))
+        if not names:
+            print(f"{k}: not found in the old build")
             ok = False
-            continue
-        a, b = old[o[0]], new[o[0]]
-        same = a == b
-        ok &= same
-        first = next((i for i, (x, y) in enumerate(zip(a, b)) if x != y), min(len(a), len(b)))
-        print(f"{k}: {len(a)} vs {len(b)} instructions, " + ("identical" if same else f"first difference at {first}"))
+        for name in names:
+            label = name.split("(")[0]
+            if name not in new:
+                print(f"{label}: not found in the new build")
+                ok = False
+                continue
+            a, b = old[name], new[name]
+            same = a == b
+            ok &= same
+            first = next((i for i, (x, y) in enumerate(zip(a, b)) if x != y), min(len(a), len(b)))
+            print(f"{label}: {len(a)} vs {len(b)} instructions, " + ("identical" if same else f"first difference at {first}"))
     return 0 if ok else 1
 
 
