@@ -141,6 +141,26 @@ int oz_perft_playouts_dev(int32_t board_size, uint64_t seed, uint64_t first_game
                           int32_t max_moves, uint64_t* black, uint64_t* white, uint32_t* info, uint8_t* moves,
                           void* stream);
 
+/* ---- exact endgame solver (stateless, batched) -------------------------------------------- */
+#define OZ_SOLVE_MAX_EMPTIES 20
+#define OZ_SOLVE_NONE (-128) /* move_margin: not a legal move; margin: position not searched (_dev only) */
+/* Exact final disc margin own-opp (empties not counted) under perfect play, side to move = own.  The game is the
+ * engine's: a side without a legal move passes, a position where neither side can move is finished and worth its disc
+ * difference.  The margin does not depend on the scoring; the outcome under either scoring follows from its sign and
+ * the mover's colour.
+ * board_size as everywhere (| OZ_RULES_STANDARD selects the flip rule; OZ_SCORING_STANDARD accepted and ignored).
+ * margin [n]; move_margin [n][64] by square bit, may be NULL (then one work item per position; else one per legal root
+ * move, each searched with the full window, and margin = the row's maximum); a finished position, or one whose mover
+ * must pass, has an all-OZ_SOLVE_NONE row.  nodes [n] (positions visited per position, may be NULL).
+ * max_empties in [0, OZ_SOLVE_MAX_EMPTIES].  _host checks every position before launching (discs must not overlap, must
+ * lie on the N x N board, at most max_empties empties) and fails with OZ_ERR_INVALID naming the first bad one; _dev does
+ * not validate content and marks a position with more than max_empties empties OZ_SOLVE_NONE without searching it
+ * (it allocates its scratch stream-ordered on `stream`). */
+int oz_endgame_solve_host(int32_t device, int32_t board_size, const uint64_t* own, const uint64_t* opp, int64_t n,
+                          int32_t max_empties, int8_t* margin, int8_t* move_margin, uint64_t* nodes);
+int oz_endgame_solve_dev(int32_t board_size, const uint64_t* own, const uint64_t* opp, int64_t n,
+                         int32_t max_empties, int8_t* margin, int8_t* move_margin, uint64_t* nodes, void* stream);
+
 /* ---- engine ----------------------------------------------------------------------------- */
 int oz_engine_create(const oz_engine_config* cfg, oz_engine** out);
 int oz_engine_destroy(oz_engine* e);

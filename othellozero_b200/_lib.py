@@ -17,6 +17,8 @@ RULES = ("reference", "standard")
 SCORING_STANDARD = 0x400  # OZ_SCORING_STANDARD, OR-ed into a board_size argument
 SCORINGS = ("reference", "standard")
 WINNER_DRAW = 2  # OZ_WINNER_DRAW: self-play winner code of a drawn game under standard scoring
+SOLVE_MAX_EMPTIES = 20  # OZ_SOLVE_MAX_EMPTIES: the endgame solver's limit
+SOLVE_NONE = -128  # OZ_SOLVE_NONE: not a legal move (move_margin) / not searched (margin)
 
 
 def board_arg(board_size: int, rules: str = "reference", scoring: str = "reference") -> int:
@@ -40,6 +42,7 @@ u64p = C.POINTER(C.c_uint64)
 i32p = C.POINTER(C.c_int32)
 u32p = C.POINTER(C.c_uint32)
 u8p = C.POINTER(C.c_uint8)
+i8p = C.POINTER(C.c_int8)
 f32p = C.POINTER(C.c_float)
 f64p = C.POINTER(C.c_double)
 vp = C.c_void_p
@@ -58,6 +61,8 @@ SIGNATURES = {
     "oz_perft_playouts_host": (C.c_int, [C.c_int32, C.c_int32, C.c_uint64, C.c_uint64, C.c_int64, C.c_int32, u64p,
                                          u64p, u32p, u8p]),
     "oz_perft_playouts_dev": (C.c_int, [C.c_int32, C.c_uint64, C.c_uint64, C.c_int64, C.c_int32, vp, vp, vp, vp, vp]),
+    "oz_endgame_solve_host": (C.c_int, [C.c_int32, C.c_int32, u64p, u64p, C.c_int64, C.c_int32, i8p, i8p, u64p]),
+    "oz_endgame_solve_dev": (C.c_int, [C.c_int32, vp, vp, C.c_int64, C.c_int32, vp, vp, vp, vp]),
     "oz_engine_create": (C.c_int, [C.POINTER(EngineConfig), C.POINTER(vp)]),
     "oz_engine_destroy": (C.c_int, [vp]),
     "oz_engine_sync": (C.c_int, [vp]),

@@ -8,7 +8,7 @@ import subprocess
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "liboz_b200.so")
-SOURCES = ["oz_rules.cu", "oz_tree.cu", "oz_net.cu", "oz_capi.cu", "oz_dist.cu"]
+SOURCES = ["oz_rules.cu", "oz_tree.cu", "oz_net.cu", "oz_capi.cu", "oz_dist.cu", "oz_solve.cu"]
 
 
 def nvcc_path() -> str:

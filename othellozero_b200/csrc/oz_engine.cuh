@@ -29,6 +29,50 @@ void oz_set_error(const char* fmt, ...);
         }                            \
     } while (0)
 
+// ---- host-buffer entry points: per-thread device scratch + pinned staging + stream (oz_rules.cu, oz_solve.cu) ----------
+struct OzHostScratch {
+    int device = -1;
+    unsigned char* dev = nullptr;
+    unsigned char* pin = nullptr;
+    size_t cap = 0;
+    cudaStream_t st = nullptr;
+    void release() {
+        if (dev) cudaFree(dev);
+        if (pin) cudaFreeHost(pin);
+        if (st) cudaStreamDestroy(st);
+        dev = pin = nullptr; st = nullptr; cap = 0; device = -1;
+    }
+    ~OzHostScratch() { release(); }  // at thread exit; errors after runtime teardown are ignored
+    int reserve(int dev_id, size_t bytes) {
+        cudaError_t e = cudaSetDevice(dev_id);
+        if (e != cudaSuccess) { oz_set_error("cudaSetDevice(%d) failed: %s", dev_id, cudaGetErrorString(e)); return OZ_ERR_CUDA; }
+        if (device != dev_id) release();
+        if (!st) {
+            e = cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking);
+            if (e != cudaSuccess) { oz_set_error("cudaStreamCreate failed: %s", cudaGetErrorString(e)); return OZ_ERR_CUDA; }
+            device = dev_id;
+        }
+        if (bytes <= cap) return OZ_OK;
+        size_t want = cap ? cap : 4096;
+        while (want < bytes) want *= 2;
+        if (dev) cudaFree(dev);
+        if (pin) cudaFreeHost(pin);
+        dev = pin = nullptr; cap = 0;
+        e = cudaMalloc((void**)&dev, want);
+        if (e == cudaSuccess) e = cudaMallocHost((void**)&pin, want);
+        if (e != cudaSuccess) {
+            oz_set_error("scratch allocation of %zu bytes failed: %s", want, cudaGetErrorString(e));
+            if (dev) cudaFree(dev);
+            dev = nullptr;
+            return OZ_ERR_NOMEM;
+        }
+        cap = want;
+        return OZ_OK;
+    }
+};
+inline size_t oz_up256(size_t x) { return (x + 255) & ~(size_t)255; }
+OzHostScratch& oz_host_scratch();
+
 // Scorings of the tree kernel (instantiated per scoring, chosen at launch): REFERENCE counts a draw as a BLACK win,
 // STANDARD scores it as a draw (value 0, winner code OZ_WINNER_DRAW).
 enum : int { SCORING_REFERENCE = 0, SCORING_STANDARD = 1 };

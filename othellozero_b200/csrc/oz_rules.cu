@@ -152,58 +152,19 @@ extern "C" int oz_perft_playouts_dev(int32_t board_size, uint64_t seed, uint64_t
 // The reference calls the rules one position at a time from Python (Othello/__init__.py), so these calls are latency
 // bound: each calling thread keeps ONE device scratch + ONE pinned staging buffer + ONE stream (grown on demand, reused
 // across calls) instead of cudaMalloc/cudaFree per call; inputs go up in one async copy, outputs come back in one.
-namespace {
-struct HostScratch {
-    int device = -1;
-    unsigned char* dev = nullptr;
-    unsigned char* pin = nullptr;
-    size_t cap = 0;
-    cudaStream_t st = nullptr;
-    void release() {
-        if (dev) cudaFree(dev);
-        if (pin) cudaFreeHost(pin);
-        if (st) cudaStreamDestroy(st);
-        dev = pin = nullptr; st = nullptr; cap = 0; device = -1;
-    }
-    ~HostScratch() { release(); }  // at thread exit; errors after runtime teardown are ignored
-    int reserve(int dev_id, size_t bytes) {
-        cudaError_t e = cudaSetDevice(dev_id);
-        if (e != cudaSuccess) { oz_set_error("cudaSetDevice(%d) failed: %s", dev_id, cudaGetErrorString(e)); return OZ_ERR_CUDA; }
-        if (device != dev_id) release();
-        if (!st) {
-            e = cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking);
-            if (e != cudaSuccess) { oz_set_error("cudaStreamCreate failed: %s", cudaGetErrorString(e)); return OZ_ERR_CUDA; }
-            device = dev_id;
-        }
-        if (bytes <= cap) return OZ_OK;
-        size_t want = cap ? cap : 4096;
-        while (want < bytes) want *= 2;
-        if (dev) cudaFree(dev);
-        if (pin) cudaFreeHost(pin);
-        dev = pin = nullptr; cap = 0;
-        e = cudaMalloc((void**)&dev, want);
-        if (e == cudaSuccess) e = cudaMallocHost((void**)&pin, want);
-        if (e != cudaSuccess) {
-            oz_set_error("scratch allocation of %zu bytes failed: %s", want, cudaGetErrorString(e));
-            if (dev) cudaFree(dev);
-            dev = nullptr;
-            return OZ_ERR_NOMEM;
-        }
-        cap = want;
-        return OZ_OK;
-    }
-};
-thread_local HostScratch g_scratch;
-inline size_t up256(size_t x) { return (x + 255) & ~(size_t)255; }
-}  // namespace
+// One per calling thread, shared by every host-buffer entry point of the library (oz_engine.cuh).
+OzHostScratch& oz_host_scratch() {
+    static thread_local OzHostScratch s;
+    return s;
+}
 
 extern "C" int oz_rules_legal_moves_host(int32_t device, int32_t board_size, const uint64_t* own,
                                          const uint64_t* opp, uint64_t* moves, int64_t n) {
     if (oz_decode_board(board_size, nullptr, nullptr)) return OZ_ERR_INVALID;
     OZ_REQUIRE(n >= 0 && (n == 0 || (own && opp && moves)), "null buffer");
     if (n == 0) return OZ_OK;
-    HostScratch& S = g_scratch;
-    const size_t b8 = up256((size_t)n * 8);
+    OzHostScratch& S = oz_host_scratch();
+    const size_t b8 = oz_up256((size_t)n * 8);
     int rc = S.reserve(device, 3 * b8);
     if (rc) return rc;
     memcpy(S.pin, own, (size_t)n * 8);
@@ -224,8 +185,8 @@ extern "C" int oz_rules_apply_host(int32_t device, int32_t board_size, const uin
     if (oz_decode_board(board_size, nullptr, nullptr)) return OZ_ERR_INVALID;
     OZ_REQUIRE(n >= 0 && (n == 0 || (own && opp && sq && own_out && opp_out && flags)), "null buffer");
     if (n == 0) return OZ_OK;
-    HostScratch& S = g_scratch;
-    const size_t b8 = up256((size_t)n * 8), b4 = up256((size_t)n * 4);
+    OzHostScratch& S = oz_host_scratch();
+    const size_t b8 = oz_up256((size_t)n * 8), b4 = oz_up256((size_t)n * 4);
     // layout: [own | opp | sq] inputs, [own' | opp' | next_legal | flags] outputs
     const size_t o_in = 0, o_out = 2 * b8 + b4, total = o_out + 3 * b8 + b4;
     int rc = S.reserve(device, total);
@@ -252,8 +213,8 @@ extern "C" int oz_rules_score_host(int32_t device, const uint64_t* black, const 
                                    int32_t* white_points, int64_t n) {
     OZ_REQUIRE(n >= 0 && (n == 0 || (black && white && black_points && white_points)), "null buffer");
     if (n == 0) return OZ_OK;
-    HostScratch& S = g_scratch;
-    const size_t b8 = up256((size_t)n * 8), b4 = up256((size_t)n * 4);
+    OzHostScratch& S = oz_host_scratch();
+    const size_t b8 = oz_up256((size_t)n * 8), b4 = oz_up256((size_t)n * 4);
     int rc = S.reserve(device, 2 * b8 + 2 * b4);
     if (rc) return rc;
     memcpy(S.pin, black, (size_t)n * 8);
@@ -275,9 +236,9 @@ extern "C" int oz_perft_playouts_host(int32_t device, int32_t board_size, uint64
     if (oz_decode_board(board_size, nullptr, nullptr)) return OZ_ERR_INVALID;
     OZ_REQUIRE(n_games >= 0 && (n_games == 0 || (black && white && info)), "null buffer");
     if (n_games == 0) return OZ_OK;
-    HostScratch& S = g_scratch;
-    const size_t b8 = up256((size_t)n_games * 8), b4 = up256((size_t)n_games * 4);
-    const size_t bm = moves ? up256((size_t)n_games * 64) : 0;
+    OzHostScratch& S = oz_host_scratch();
+    const size_t b8 = oz_up256((size_t)n_games * 8), b4 = oz_up256((size_t)n_games * 4);
+    const size_t bm = moves ? oz_up256((size_t)n_games * 64) : 0;
     int rc = S.reserve(device, 2 * b8 + b4 + bm);
     if (rc) return rc;
     unsigned char* d = S.dev;

@@ -30,14 +30,18 @@ def broadcast_weights(blob, src: int = 0, device=None):
     return t
 
 
-def pack_records(rec: dict) -> np.ndarray:
+def pack_records(rec: dict, winners=None) -> np.ndarray:
     """Self-play records -> compact uint64 rows [black, white, action | player<<8 | winner<<16 | game<<32] per move
-    (18 B of information per position, SURVEY §8e)."""
+    (18 B of information per position, SURVEY §8e).  winners: optional per-position winner codes [G, 64]
+    (selfplay.solve_record_winners) for the winner field in place of each game's winner."""
     nm = np.asarray(rec["n_moves"]).astype(np.int64)
     g = nm.shape[0]
     valid = np.arange(64)[None, :] < nm[:, None]
     gi = np.broadcast_to(np.arange(g, dtype=np.uint64)[:, None], (g, 64))
-    win = np.broadcast_to((np.asarray(rec["winner"]).astype(np.int64) & 0xFF).astype(np.uint64)[:, None], (g, 64))
+    if winners is None:
+        win = np.broadcast_to((np.asarray(rec["winner"]).astype(np.int64) & 0xFF).astype(np.uint64)[:, None], (g, 64))
+    else:
+        win = (np.asarray(winners).astype(np.int64) & 0xFF).astype(np.uint64).reshape(g, 64)
     meta = rec["action"].astype(np.uint64) | (rec["player"].astype(np.uint64) << np.uint64(8)) | \
         (win << np.uint64(16)) | (gi << np.uint64(32))
     return np.stack([rec["black"][valid].astype(np.uint64), rec["white"][valid].astype(np.uint64), meta[valid]], axis=1)

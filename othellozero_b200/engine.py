@@ -7,7 +7,8 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import (PRIOR_HASH, PRIOR_HOST, PRIOR_NET, board_arg, check, f32p, f64p, i32p, ptr, u8p, u32p, u64p)
+from ._lib import (PRIOR_HASH, PRIOR_HOST, PRIOR_NET, SCORINGS, SOLVE_MAX_EMPTIES, SOLVE_NONE, WINNER_DRAW, board_arg,
+                   check, f32p, f64p, i8p, i32p, ptr, u8p, u32p, u64p)
 
 M64 = (1 << 64) - 1
 
@@ -76,6 +77,36 @@ def decode_perft_info(info) -> dict:
     info = np.asarray(info, dtype=np.uint32)
     return dict(plies=(info & 0xFF).astype(np.int32), player=((info >> 8) & 1).astype(np.int32),
                 finished=((info >> 9) & 1).astype(bool), passes=(info >> 16).astype(np.int32))
+
+
+def solve_endgame(own, opp, board_size: int = 8, max_empties: int = SOLVE_MAX_EMPTIES, per_move: bool = False,
+                  device: int = 0, rules: str = "reference") -> dict:
+    """Exact endgame solver (oz_endgame_solve_host): the final disc margin own - opp under perfect play by both sides,
+    side to move = own, empties left at the end not counted.  Returns dict(margin int8 [n], move_margin int8 [n, 64] by
+    square bit or None, nodes uint64 [n]).  per_move=True also solves every legal root move with the full window
+    (SOLVE_NONE on squares that are not legal moves; the whole row for a finished position or one whose mover must pass).
+    Every position must have at most max_empties (<= SOLVE_MAX_EMPTIES) empties, else AssertionError.  The margin does
+    not depend on the scoring: see perfect_play_winner."""
+    bs = board_arg(board_size, rules)
+    own, opp = _u64(np.atleast_1d(own)), _u64(np.atleast_1d(opp))
+    assert own.shape == opp.shape and own.ndim == 1
+    margin = np.zeros(own.size, dtype=np.int8)
+    move_margin = np.zeros((own.size, 64), dtype=np.int8) if per_move else None
+    nodes = np.zeros(own.size, dtype=np.uint64)
+    check(_lib.load().oz_endgame_solve_host(device, bs, ptr(own, u64p), ptr(opp, u64p), own.size, int(max_empties),
+                                            ptr(margin, i8p), ptr(move_margin, i8p), ptr(nodes, u64p)))
+    return dict(margin=margin, move_margin=move_margin, nodes=nodes)
+
+
+def perfect_play_winner(margin, player, scoring: str = "reference") -> np.ndarray:
+    """Winner codes of solved positions (the records' codes: 0 BLACK, 1 WHITE, WINNER_DRAW) from the mover's exact
+    margin and colour (player 0 = BLACK): a positive margin is a win for the mover, a negative one for the opponent, and
+    margin 0 is a BLACK win under reference scoring (Othello/__init__.py:254-256) and a draw under standard scoring."""
+    if scoring not in SCORINGS:
+        raise ValueError(f"scoring must be one of {SCORINGS}, got {scoring!r}")
+    margin, player = np.asarray(margin).astype(np.int64), np.asarray(player).astype(np.int64)
+    even = WINNER_DRAW if scoring == "standard" else 0
+    return np.where(margin > 0, player, np.where(margin < 0, 1 - player, even)).astype(np.int32)
 
 
 def probe_l2_read(megabytes: int = 32, passes: int = 50, device: int = 0) -> float:

@@ -46,6 +46,7 @@ class IterationConfig:
     seed: int = 0
     rules: str = "reference"         # "standard": self-play and arena under standard Othello flipping
     scoring: str = "reference"       # "standard": a drawn game is a draw (z = 0; no arena win for either network)
+    solve_empties: int = 0           # > 0: positions with <= this many empties get perfect-play targets (exact solver)
 
 
 def unpack_rows(rows: np.ndarray):
@@ -125,9 +126,22 @@ class Trainer:
             info["selfplay_sims_this_rank"] = sp.engine.counters()["sims"]
             sp.close()
         timed("selfplay_s", t0)
+        # ---- exact endgame targets: every rank relabels the positions of its own games ---------------------------------
+        winners = None
+        if cfg.solve_empties > 0:
+            t0 = time.perf_counter()
+            solved = relabelled = 0
+            if rec is not None:
+                winners = selfplay.solve_record_winners(rec, n, cfg.solve_empties, cfg.rules, cfg.scoring,
+                                                        device=self.local)
+                mask = selfplay.solvable_positions(rec, n, cfg.solve_empties)
+                solved = int(mask.sum())
+                relabelled = int((mask & (winners != np.asarray(rec["winner"])[:, None])).sum())
+            info["solve_this_rank"] = (solved, relabelled)
+            timed("solve_s", t0)
         # ---- C2: gather the packed example records; every rank keeps the same replay buffer ----------------------------
         t0 = time.perf_counter()
-        packed = ozd.pack_records(rec) if rec is not None else np.zeros((0, 3), dtype=np.uint64)
+        packed = ozd.pack_records(rec, winners) if rec is not None else np.zeros((0, 3), dtype=np.uint64)
         rows = ozd.gather_examples(packed) if self.world > 1 else packed
         self.buffer.extend(rows)
         timed("gather_s", t0)
@@ -173,13 +187,21 @@ class Trainer:
             info["selfplay_sims"] = int(s.item())
         else:
             info["selfplay_sims"] = info.get("selfplay_sims_this_rank", 0)
+        solve = {}
+        if cfg.solve_empties > 0:
+            counts = info["solve_this_rank"]
+            if self.world > 1:
+                t = torch.tensor(list(counts), dtype=torch.int64, device=dev)
+                dist.all_reduce(t)
+                counts = (int(t[0].item()), int(t[1].item()))
+            solve = dict(solved_positions=counts[0], solve_relabelled=counts[1])
         return dict(iteration=self.iteration, phases=phases, episodes=cfg.episodes, positions_gathered=int(rows.shape[0]),
                     buffer_examples=len(self.buffer), train_examples=int(arrays[0].shape[0]),
                     train_steps=cfg.epochs * ((arrays[0].shape[0] + cfg.batch_size - 1) // cfg.batch_size),
                     train_history=hist, arena_new_wins=wins, arena_draws=draws, arena_games=cfg.arena_games,
                     promoted=bool(promoted),
                     selfplay_sims=info["selfplay_sims"],
-                    selfplay_sims_per_s=info["selfplay_sims"] / max(phases["selfplay_s"], 1e-9))
+                    selfplay_sims_per_s=info["selfplay_sims"] / max(phases["selfplay_s"], 1e-9), **solve)
 
 
 def main(argv=None):
@@ -191,6 +213,9 @@ def main(argv=None):
                         **({"choices": choices[f]} if f in choices else {}))
     ap.add_argument("--iterations", type=int, default=1)
     args = ap.parse_args(argv)
+    from ._lib import SOLVE_MAX_EMPTIES
+    if not 0 <= args.solve_empties <= SOLVE_MAX_EMPTIES:
+        ap.error(f"--solve-empties must be in [0, {SOLVE_MAX_EMPTIES}] (got {args.solve_empties})")
     import torch
     import torch.distributed as dist
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -140,10 +140,11 @@ def expand_symmetries(black, white, action, board_size: int):
     return b8, p8
 
 
-def records_to_examples_batch(rec: dict, board_size: int, games=None):
+def records_to_examples_batch(rec: dict, board_size: int, games=None, winners=None):
     """All games' records -> per-game example lists (training.py:58-72 + the 8 symmetries of :13-23), built with array
     operations over every (game, ply) at once: ~40x faster than calling records_to_examples per game (45 s -> ~1 s per
-    4096 8x8 games).  The tuples hold views into three big arrays; order and values equal records_to_examples'."""
+    4096 8x8 games).  The tuples hold views into three big arrays; order and values equal records_to_examples'.
+    winners: optional per-position winner codes [G, 64] (solve_record_winners) in place of each game's winner."""
     n = board_size
     games = range(len(rec["n_moves"])) if games is None else list(games)
     nm = np.asarray([int(rec["n_moves"][g]) for g in games], dtype=np.int64)
@@ -152,7 +153,7 @@ def records_to_examples_batch(rec: dict, board_size: int, games=None):
     P = int(gsel.size)
     b8, p8 = expand_symmetries(np.asarray(rec["black"])[gsel, psel], np.asarray(rec["white"])[gsel, psel],
                                np.asarray(rec["action"])[gsel, psel], n)
-    w = np.asarray(rec["winner"])[gsel]
+    w = np.asarray(rec["winner"])[gsel] if winners is None else np.asarray(winners)[gsel, psel]
     z = np.where(w == WINNER_DRAW, 0, np.where(w == np.asarray(rec["player"])[gsel, psel], 1, -1))
     # one (board view, policy view, z) tuple per example, made by C-level iteration over the leading axis
     flat = list(zip(b8.reshape(P * 8, n, n, 2), p8.reshape(P * 8, n, n), np.repeat(np.asarray(z, dtype=np.int64), 8).tolist()))
@@ -161,6 +162,32 @@ def records_to_examples_batch(rec: dict, board_size: int, games=None):
         out.append(flat[row:row + 8 * int(k)])
         row += 8 * int(k)
     return out
+
+
+def solvable_positions(rec: dict, board_size: int, empties: int) -> np.ndarray:
+    """[G, 64] bool: the recorded positions (before their move) with at most `empties` empty squares."""
+    both = np.asarray(rec["black"], dtype=np.uint64) | np.asarray(rec["white"], dtype=np.uint64)
+    discs = np.unpackbits(both.view(np.uint8).reshape(both.shape + (8,)), axis=-1).sum(axis=-1)  # off-board bits are 0
+    valid = np.arange(64)[None, :] < np.asarray(rec["n_moves"]).astype(np.int64)[:, None]
+    return valid & (board_size * board_size - discs <= empties)
+
+
+def solve_record_winners(rec: dict, board_size: int, empties: int, rules: str = "reference", scoring: str = "reference",
+                         device: int = 0) -> np.ndarray:
+    """Per-position winner codes [G, 64] for training targets: every recorded position (before its move) with at most
+    `empties` empty squares gets the winner under perfect play from there (engine.solve_endgame ->
+    engine.perfect_play_winner); every other entry keeps its game's winner.  The record arrays are not changed."""
+    n = board_size
+    winners = np.repeat(np.asarray(rec["winner"]).astype(np.int32)[:, None], 64, axis=1)
+    black, white = np.asarray(rec["black"], dtype=np.uint64), np.asarray(rec["white"], dtype=np.uint64)
+    player = np.asarray(rec["player"]).astype(np.int64)
+    sel = solvable_positions(rec, n, empties)
+    if sel.any():
+        own = np.where(player[sel] == 0, black[sel], white[sel])
+        opp = np.where(player[sel] == 0, white[sel], black[sel])
+        out = _e.solve_endgame(own, opp, board_size=n, max_empties=empties, device=device, rules=rules)
+        winners[sel] = _e.perfect_play_winner(out["margin"], player[sel], scoring)
+    return winners
 
 
 # ---- RNG streams of episodes -------------------------------------------------------------------------------------
@@ -184,10 +211,15 @@ def allocate_game_ids(n: int) -> np.ndarray:
 
 def execute_episodes(n_episodes, board_size, neural_network, degree_exploration, num_simulations, policy_temperature,
                      e_greedy, device: int = 0, seed: int | None = None, reference_aliasing: bool = False, game_ids=None,
-                     max_concurrent: int = 4096, rules: str = "reference", scoring: str = "reference"):
+                     max_concurrent: int = 4096, rules: str = "reference", scoring: str = "reference",
+                     solve_empties: int = 0):
     """n_episodes x training.execute_episode as one GPU job; returns a list of example lists.  At most `max_concurrent`
     episodes are in flight (node pools are per slot); the others are queued on the device and start as slots free up.
-    policy_temperature may be 0 (main.py:73-76 switches to it after `temperature_threshold` iterations)."""
+    policy_temperature may be 0 (main.py:73-76 switches to it after `temperature_threshold` iterations).
+    solve_empties > 0: the target z of every position with at most that many empties comes from the winner under perfect
+    play (solve_record_winners), not from the game's outcome; not available with reference_aliasing."""
+    if solve_empties and reference_aliasing:
+        raise ValueError("solve_empties > 0 needs per-position targets, which reference_aliasing=True does not have")
     if seed is None:
         seed = _PROCESS_SEED
     if game_ids is None:
@@ -202,7 +234,8 @@ def execute_episodes(n_episodes, board_size, neural_network, degree_exploration,
         logging.info(f'Episode finished: game {g}, winner channel {int(rec["winner"][g])}.')
     if reference_aliasing:
         return [records_to_examples(rec, g, board_size, True) for g in range(n_episodes)]
-    return records_to_examples_batch(rec, board_size)
+    winners = solve_record_winners(rec, board_size, solve_empties, rules, scoring, device) if solve_empties else None
+    return records_to_examples_batch(rec, board_size, winners=winners)
 
 
 def execute_episode(board_size, neural_network, degree_exploration, num_simulations, policy_temperature, e_greedy,
