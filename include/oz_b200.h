@@ -240,6 +240,19 @@ int oz_net_load_weights(oz_engine* e, const float* blob, int64_t n_floats, int32
 /* Same, from a DEVICE float32 blob (e.g. a tensor just received by ncclBroadcast). */
 int oz_net_load_weights_dev(oz_engine* e, const float* blob_dev, int64_t n_floats, int32_t channels);
 int64_t oz_net_blob_floats(int32_t board_size, int32_t channels);
+/* FP8 evaluation (DESIGN.md 13): OR OZ_NET_FP8 into the `channels` argument of oz_net_load_weights[_dev] and
+ * oz_dist_broadcast_weights to run conv3, conv4 and fc1 on e4m3 operands (per-output-channel weight scales, one static
+ * scale per input activation calibrated at load, fp32 accumulation).  Everything else stays bf16 and the blob format is
+ * unchanged (oz_net_blob_floats takes the plain channel count).  FP8 needs channels to be a multiple of 256 and the
+ * default kernels: with OZ_NET_CONV2=gemm, OZ_NET_CONV3=wino or OZ_NET_NO_2SM=1 in the environment an FP8 load fails
+ * with OZ_ERR_STATE.  The precision is fixed by an engine's first load, like the channel count: a later load with the
+ * other precision fails with OZ_ERR_STATE. */
+#define OZ_NET_FP8 0x10000
+/* Scales of the loaded FP8 network into a HOST buffer of 3 + 2 * channels + 1024 floats: sa_2, sa_3, sa_4 (the static
+ * scales of act2, act3, act4 = the inputs of conv3, conv4, fc1), then the per-output-channel weight scales of conv3
+ * [channels], conv4 [channels] and fc1 [1024].  A real value x is stored as e4m3_rn(x / scale).  OZ_ERR_STATE unless the
+ * engine's weights were loaded with OZ_NET_FP8. */
+int oz_net_fp8_scales(oz_engine* e, float* out);
 /* Batched predict on canonical boards. pi: [n][N*N] softmax probabilities (r*N+c), logits same shape (may be
  * NULL), v: [n] tanh.  HOST buffers (rows of N*N floats) / DEVICE buffers (rows padded to a stride of 64 floats). */
 int oz_net_forward_host(oz_engine* e, const uint64_t* own, const uint64_t* opp, int32_t n, float* pi,
@@ -247,7 +260,9 @@ int oz_net_forward_host(oz_engine* e, const uint64_t* own, const uint64_t* opp, 
 int oz_net_forward_dev(oz_engine* e, const uint64_t* own, const uint64_t* opp, int32_t n, float* pi,
                        float* logits, float* v);
 /* Debug/inspection: raw bf16 activations of the last forward. layer 0..5 = conv1, conv2, conv3, conv4, fc1, fc2
- * outputs ([n][rows][channels] row-major); copies `bytes` bytes to the HOST buffer.  conv1+conv2 normally run as one
+ * outputs ([n][rows][channels] row-major); copies `bytes` bytes to the HOST buffer.  An FP8 network (OZ_NET_FP8) stores
+ * layers 1..3 (act2, act3, act4) as raw e4m3 bytes, one per element, in units of their scales (oz_net_fp8_scales); layers
+ * 4 and 5 stay bf16.  conv1+conv2 normally run as one
  * gather over a pre-computed partial-product table (DESIGN.md 3a), which never materialises conv1's output: layer 0 then
  * fails with OZ_ERR_STATE (engines created with OZ_NET_CONV2=gemm in the environment keep it); likewise layer 1 with the
  * opt-in OZ_NET_CONV3=wino (conv3 as a Winograd F(2,3) kernel fed by the gather's input transform, DESIGN.md 3b). */

@@ -19,6 +19,8 @@ SCORINGS = ("reference", "standard")
 WINNER_DRAW = 2  # OZ_WINNER_DRAW: self-play winner code of a drawn game under standard scoring
 SOLVE_MAX_EMPTIES = 20  # OZ_SOLVE_MAX_EMPTIES: the endgame solver's limit
 SOLVE_NONE = -128  # OZ_SOLVE_NONE: not a legal move (move_margin) / not searched (margin)
+NET_FP8 = 0x10000  # OZ_NET_FP8, OR-ed into a channels argument
+PRECISIONS = ("bf16", "fp8")
 
 
 def board_arg(board_size: int, rules: str = "reference", scoring: str = "reference") -> int:
@@ -30,6 +32,14 @@ def board_arg(board_size: int, rules: str = "reference", scoring: str = "referen
     if scoring not in SCORINGS:
         raise ValueError(f"scoring must be one of {SCORINGS}, got {scoring!r}")
     return board_size | (RULES_STANDARD if rules == "standard" else 0) | (SCORING_STANDARD if scoring == "standard" else 0)
+
+
+def channels_arg(channels: int, precision: str = "bf16") -> int:
+    """The C-ABI channels argument of the weight loaders for a network precision: "bf16" (the default) or "fp8" (conv3,
+    conv4 and fc1 on e4m3 operands, DESIGN.md 13).  Anything else raises ValueError."""
+    if precision not in PRECISIONS:
+        raise ValueError(f"precision must be one of {PRECISIONS}, got {precision!r}")
+    return int(channels) | (NET_FP8 if precision == "fp8" else 0)
 
 
 class EngineConfig(C.Structure):
@@ -88,6 +98,7 @@ SIGNATURES = {
     "oz_net_forward_host": (C.c_int, [vp, u64p, u64p, C.c_int32, f32p, f32p, f32p]),
     "oz_net_forward_dev": (C.c_int, [vp, vp, vp, C.c_int32, vp, vp, vp]),
     "oz_net_get_activation": (C.c_int, [vp, C.c_int32, vp, C.c_int64]),
+    "oz_net_fp8_scales": (C.c_int, [vp, f32p]),
     "oz_engine_launches": (C.c_int, [vp, u64p]),
     "oz_net_layer_times": (C.c_int, [vp, f32p]),
     "oz_net_set_timing": (C.c_int, [vp, C.c_int32]),

@@ -138,7 +138,7 @@ def pit(board_size, net_black, net_white, num_simulations, degree_exploration=1,
         e = _e.Engine(n, max_games=n_games, nodes_per_game=nodes, prior_mode=mode, c_puct=float(degree_exploration),
                       device=device, rules=rules, scoring=scoring)
         if mode == _e.PRIOR_NET:
-            e.load_weights(net.blob, net.channels)
+            e.load_weights(net.blob, net.channels, net.precision)
         engines.append(e)
     if start_black is None:
         from .othello import _bits

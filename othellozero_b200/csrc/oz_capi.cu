@@ -572,3 +572,9 @@ extern "C" int oz_net_get_activation(oz_engine* e, int32_t layer, void* host_bf1
     OZ_CUDA(cudaSetDevice(e->cfg.device));
     return oz_net_activation(e, layer, host_bf16, bytes);
 }
+
+extern "C" int oz_net_fp8_scales(oz_engine* e, float* out) {
+    OZ_REQUIRE(e && out, "null argument");
+    OZ_CUDA(cudaSetDevice(e->cfg.device));
+    return oz_net_scales(e, out);
+}

@@ -111,8 +111,9 @@ extern "C" int oz_dist_broadcast_weights(oz_engine* e, const float* blob, int64_
     if (!e->comm) { oz_set_error("oz_dist_init first"); return OZ_ERR_STATE; }
     OZ_REQUIRE(root >= 0 && root < e->dist_world, "root %d out of range", root);
     OZ_REQUIRE(e->dist_rank != root || blob, "the root rank must pass the weight blob");
-    OZ_REQUIRE(n_floats == oz_net_blob_floats(e->cfg.board_size, channels), "weight blob has %lld floats, expected %lld",
-               (long long)n_floats, (long long)oz_net_blob_floats(e->cfg.board_size, channels));
+    const int32_t plain = channels & ~OZ_NET_FP8;  // the blob does not depend on the precision
+    OZ_REQUIRE(n_floats == oz_net_blob_floats(e->cfg.board_size, plain), "weight blob has %lld floats, expected %lld",
+               (long long)n_floats, (long long)oz_net_blob_floats(e->cfg.board_size, plain));
     OZ_CUDA(cudaSetDevice(e->cfg.device));
     float* dev = nullptr;
     OZ_CUDA(cudaMalloc((void**)&dev, (size_t)n_floats * 4));
@@ -121,7 +122,7 @@ extern "C" int oz_dist_broadcast_weights(oz_engine* e, const float* blob, int64_
         OZ_CUDA(cudaMemcpyAsync(dev, blob, (size_t)n_floats * 4, cudaMemcpyHostToDevice, e->stream));
     OZ_NCCL(nccl_api()->Broadcast(dev, dev, (size_t)n_floats, ncclFloat32, root, (ncclComm_t)e->comm, e->stream));
     OZ_CUDA(cudaStreamSynchronize(e->stream));
-    return oz_net_load_weights_dev(e, dev, n_floats, channels);  // folds BN, casts to bf16, rebuilds the tables, clears the cache
+    return oz_net_load_weights_dev(e, dev, n_floats, channels);  // folds BN, casts to bf16 (or quantises, OZ_NET_FP8), rebuilds the tables, clears the cache
 }
 
 extern "C" int oz_dist_gather_examples(oz_engine* e, const uint64_t* rows, int64_t n_rows, uint64_t* out_rows, int64_t capacity_rows,

@@ -221,6 +221,7 @@ int oz_net_forward(oz_engine* e, const u64* own_dev, const u64* opp_dev, const i
                    float* pi_dev, float* logits_dev, float* v_dev, bool publish = false);
 int64_t oz_net_blob_floats_impl(int board_size, int channels);
 int oz_net_activation(oz_engine* e, int layer, void* host, int64_t bytes);
+int oz_net_scales(oz_engine* e, float* out);
 void oz_net_set_timing_impl(oz_engine* e, bool on);
 int oz_net_times(oz_engine* e, float* ms8);
 

@@ -19,7 +19,10 @@
 // (fp32, then cast to bf16) and a per-channel fp32 bias at load time.
 #include <cuda.h>
 #include <cuda_bf16.h>
+#include <cuda_fp8.h>
 #include <stdlib.h>
+
+#include <vector>
 
 #include "oz_engine.cuh"
 
@@ -67,6 +70,7 @@ struct GemmParams {
     // heads epilogue = also the evaluation cache's publish step (oz_tree.cu): row r of the batch belongs to cache entry
     // cache_idx[r] (>= 0) whose owner parked it as "pending"; null = no cache
     const int* cache_idx; float* cache_pi; float* cache_v; unsigned long long* cache_tags;
+    const float* alpha;  // FP8 epilogues (oz_gemm2_kernel<OP_FP8_*>): out = relu(fma(acc, alpha[co], bias[co]))
 };
 
 // ---- PTX wrappers -------------------------------------------------------------------------------------
@@ -198,6 +202,17 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 // Instruction descriptor: D=f32, A=B=bf16, both K-major, M x N.
 __host__ __device__ constexpr uint32_t make_idesc(int m, int n) {
     return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
+}
+// kind::f8f6f4 instruction descriptor: D=f32, A=B=E4M3 (format code 0), both K-major, M x N.
+__host__ __device__ constexpr uint32_t make_idesc_e4m3(int m, int n) {
+    return (1u << 4) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
+}
+// Four e4m3 bytes (satfinite, round-to-nearest, ReLU fused: F2FP.SATFINITE.RELU.E4M3) from a..d, a in the lowest byte.
+__device__ __forceinline__ uint32_t pack_relu_e4m3x4(float a, float b, float c, float d) {
+    uint16_t lo, hi;
+    asm("cvt.rn.satfinite.relu.e4m3x2.f32 %0, %1, %2;" : "=h"(lo) : "f"(b), "f"(a));
+    asm("cvt.rn.satfinite.relu.e4m3x2.f32 %0, %1, %2;" : "=h"(hi) : "f"(d), "f"(c));
+    return (uint32_t)lo | ((uint32_t)hi << 16);
 }
 
 // Table entries are consumed by fp32 accumulation only, so the pair (even, odd) is packed so that the odd element needs no
@@ -512,6 +527,15 @@ __device__ __forceinline__ void umma_bf16_2sm_lo(uint32_t d_tmem, uint32_t a_lo,
         "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %3, p;\n\t}"
         ::"r"(d_tmem), "r"(a_lo), "r"(b_lo), "r"(idesc), "r"(accumulate), "r"(SW128_DESC_HI) : "memory");
 }
+__device__ __forceinline__ void umma_e4m3_2sm_lo(uint32_t d_tmem, uint32_t a_lo, uint32_t b_lo, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "mov.b64 da, {%1, %5};\n\t"
+        "mov.b64 db, {%2, %5};\n\t"
+        "tcgen05.mma.cta_group::2.kind::f8f6f4 [%0], da, db, %3, p;\n\t}"
+        ::"r"(d_tmem), "r"(a_lo), "r"(b_lo), "r"(idesc), "r"(accumulate), "r"(SW128_DESC_HI) : "memory");
+}
 __device__ __forceinline__ void umma_commit_2sm(uint32_t bar, uint16_t cta_mask) {
     asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
                  ::"r"(bar), "h"(cta_mask) : "memory");
@@ -519,21 +543,29 @@ __device__ __forceinline__ void umma_commit_2sm(uint32_t bar, uint16_t cta_mask)
 
 constexpr int STAGES2 = 6;
 constexpr int B2_STAGE_BYTES = 128 * BLOCK_K * 2;  // this CTA's 128-row half of the 256-row B tile
+// Operand kinds of oz_gemm2_kernel.  A k-block is one 128-byte swizzle row either way (64 bf16 or 128 e4m3 channels), so
+// the ring, the TMA boxes' byte geometry and the 32-byte descriptor step per MMA (K = 16 bf16 / K = 32 e4m3) are shared.
+constexpr int OP_BF16 = 0;       // bf16 x bf16, epilogue relu(acc + bias) -> bf16
+constexpr int OP_FP8_E4M3 = 1;   // e4m3 x e4m3, epilogue relu(fma(acc, alpha, bias)) -> e4m3 (conv3, conv4; DESIGN 13)
+constexpr int OP_FP8_BF16 = 2;   // e4m3 x e4m3, epilogue relu(fma(acc, alpha, bias)) -> bf16 (fc1)
+template <int OP>
 struct Gemm2Smem {
     static constexpr int OFF_A = 0;
     static constexpr int OFF_B = STAGES2 * A_STAGE_BYTES;
     static constexpr int OFF_BAR = OFF_B + STAGES2 * B2_STAGE_BYTES;  // full[S], empty[S], tfull[2], tempty[2]
     static constexpr int OFF_TMEM = OFF_BAR + (2 * STAGES2 + 4) * 8;
-    static constexpr int OFF_BIAS = OFF_TMEM + 16;
-    static constexpr int BYTES = OFF_BIAS + 2 * 256 * 4;
+    static constexpr int OFF_BIAS = OFF_TMEM + 16;                    // [2][256] bias (+ [2][256] alpha for FP8)
+    static constexpr int BYTES = OFF_BIAS + (OP == OP_BF16 ? 1 : 2) * 2 * 256 * 4;
     static constexpr int DYN_BYTES = BYTES + 1024;
 };
 
+template <int OP>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(GEMM_THREADS, 1)
 oz_gemm2_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapA2,
                 const __grid_constant__ CUtensorMap mapB, const GemmParams p) {
-    using S = Gemm2Smem;
+    using S = Gemm2Smem<OP>;
     constexpr int BLOCK_N = 256;
+    constexpr int KB = OP == OP_BF16 ? BLOCK_K : 2 * BLOCK_K;  // channels (tensor-map elements) per k-block
     constexpr uint32_t TMEM_COLS = 2 * BLOCK_N;
     extern __shared__ uint8_t smem_raw[];
     const uint32_t raw = smem_u32(smem_raw);
@@ -601,7 +633,7 @@ oz_gemm2_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
                 int kcol = 0;
                 for (int ky = -p.pad; ky < ntaps_y - p.pad; ++ky) {
                     for (int kx = -p.pad; kx < p.ntaps_x - p.pad; ++kx) {
-                        for (int c0 = 0; c0 < p.chunks_per_tap * BLOCK_K; c0 += BLOCK_K) {
+                        for (int c0 = 0; c0 < p.chunks_per_tap * KB; c0 += KB) {
                             mbar_wait(empty_bar(stage), phase ^ 1u);
                             if (elect_one()) {
                                 const uint32_t fb = fb0 + 8u * (uint32_t)stage;
@@ -612,7 +644,7 @@ oz_gemm2_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
                                 tma_load_2d_2sm(sB + stage * B2_STAGE_BYTES, &mapB, fb, kcol, n0);
                             }
                             __syncwarp();
-                            kcol += BLOCK_K;
+                            kcol += KB;
                             if (++stage == STAGES2) { stage = 0; phase ^= 1u; }
                         }
                     }
@@ -622,7 +654,7 @@ oz_gemm2_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
         __syncwarp();
     } else if (warp == 1) {
         if (rank == 0) {  // ===== MMA issuer: one elected lane of the leader CTA's warp drives both tensor cores =====
-            constexpr uint32_t idesc = make_idesc(256, BLOCK_N);
+            constexpr uint32_t idesc = OP == OP_BF16 ? make_idesc(256, BLOCK_N) : make_idesc_e4m3(256, BLOCK_N);
             const uint32_t a_lo0 = sw128_desc_lo(sA), b_lo0 = sw128_desc_lo(sB);
             int stage = 0; uint32_t phase = 0;
             int acc = 0; uint32_t acc_phase = 0;
@@ -637,8 +669,12 @@ oz_gemm2_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
                     const uint32_t b_lo = b_lo0 + (uint32_t)stage * (B2_STAGE_BYTES >> 4);
                     if (elect_one()) {
 #pragma unroll
-                        for (int k = 0; k < BLOCK_K / UMMA_K; ++k)
-                            umma_bf16_2sm_lo(d_tmem, a_lo + 2u * k, b_lo + 2u * k, idesc, (kb | k) ? 1u : 0u);
+                        for (int k = 0; k < BLOCK_K / UMMA_K; ++k) {  // 4 x 32 bytes: K = 16 bf16 or 32 e4m3 per MMA
+                            if constexpr (OP == OP_BF16)
+                                umma_bf16_2sm_lo(d_tmem, a_lo + 2u * k, b_lo + 2u * k, idesc, (kb | k) ? 1u : 0u);
+                            else
+                                umma_e4m3_2sm_lo(d_tmem, a_lo + 2u * k, b_lo + 2u * k, idesc, (kb | k) ? 1u : 0u);
+                        }
                         umma_commit_2sm(empty_bar(stage), 3);  // frees the stage in BOTH CTAs
                     }
                     __syncwarp();
@@ -658,7 +694,10 @@ oz_gemm2_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
             const int m_pair = pt / p.n_tiles, n_idx = pt - m_pair * p.n_tiles;
             const int m_tile = 2 * m_pair + (int)rank;
             float* bias = s_bias + acc * BLOCK_N;
+            float* alpha = s_bias + (2 + acc) * BLOCK_N;  // FP8 only
             for (int i = et; i < BLOCK_N; i += 128) bias[i] = p.bias[n_idx * BLOCK_N + i];
+            if constexpr (OP != OP_BF16)
+                for (int i = et; i < BLOCK_N; i += 128) alpha[i] = p.alpha[n_idx * BLOCK_N + i];
             epi_bar_sync();
             mbar_wait(tfull_bar(acc), acc_phase);
             tc_fence_after();
@@ -673,17 +712,43 @@ oz_gemm2_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
                 tmem_ld32(t_row + (uint32_t)(c * 32), v);
                 tmem_ld_wait();
                 if (ok) {
-                    uint32_t packed[16];
+                    if constexpr (OP == OP_BF16) {
+                        uint32_t packed[16];
 #pragma unroll
-                    for (int j = 0; j < 16; ++j) {
-                        const float2 bj = *reinterpret_cast<const float2*>(bias + c * 32 + 2 * j);
-                        const float2 y = __fadd2_rn(make_float2(__uint_as_float(v[2 * j]), __uint_as_float(v[2 * j + 1])), bj);
-                        packed[j] = pack_relu_bf16x2(y.x, y.y);
+                        for (int j = 0; j < 16; ++j) {
+                            const float2 bj = *reinterpret_cast<const float2*>(bias + c * 32 + 2 * j);
+                            const float2 y = __fadd2_rn(make_float2(__uint_as_float(v[2 * j]), __uint_as_float(v[2 * j + 1])), bj);
+                            packed[j] = pack_relu_bf16x2(y.x, y.y);
+                        }
+                        uint4* dst = reinterpret_cast<uint4*>(orow + c * 32);
+#pragma unroll
+                        for (int q = 0; q < 4; ++q)
+                            dst[q] = make_uint4(packed[4 * q], packed[4 * q + 1], packed[4 * q + 2], packed[4 * q + 3]);
+                    } else {
+                        float y[32];
+#pragma unroll
+                        for (int j = 0; j < 16; ++j) {
+                            const float2 aj = *reinterpret_cast<const float2*>(alpha + c * 32 + 2 * j);
+                            const float2 bj = *reinterpret_cast<const float2*>(bias + c * 32 + 2 * j);
+                            const float2 t = __ffma2_rn(make_float2(__uint_as_float(v[2 * j]), __uint_as_float(v[2 * j + 1])), aj, bj);
+                            y[2 * j] = t.x; y[2 * j + 1] = t.y;
+                        }
+                        if constexpr (OP == OP_FP8_E4M3) {  // row stride p.ldc BYTES
+                            uint32_t packed[8];
+#pragma unroll
+                            for (int j = 0; j < 8; ++j) packed[j] = pack_relu_e4m3x4(y[4 * j], y[4 * j + 1], y[4 * j + 2], y[4 * j + 3]);
+                            uint4* dst = reinterpret_cast<uint4*>(reinterpret_cast<uint8_t*>(p.out) + grow * p.ldc +
+                                                                  (long long)n_idx * BLOCK_N + c * 32);
+                            dst[0] = make_uint4(packed[0], packed[1], packed[2], packed[3]);
+                            dst[1] = make_uint4(packed[4], packed[5], packed[6], packed[7]);
+                        } else {
+                            uint4* dst = reinterpret_cast<uint4*>(orow + c * 32);
+#pragma unroll
+                            for (int q = 0; q < 4; ++q)
+                                dst[q] = make_uint4(pack_relu_bf16x2(y[8 * q], y[8 * q + 1]), pack_relu_bf16x2(y[8 * q + 2], y[8 * q + 3]),
+                                                    pack_relu_bf16x2(y[8 * q + 4], y[8 * q + 5]), pack_relu_bf16x2(y[8 * q + 6], y[8 * q + 7]));
+                        }
                     }
-                    uint4* dst = reinterpret_cast<uint4*>(orow + c * 32);
-#pragma unroll
-                    for (int q = 0; q < 4; ++q)
-                        dst[q] = make_uint4(packed[4 * q], packed[4 * q + 1], packed[4 * q + 2], packed[4 * q + 3]);
                 }
             }
             tc_fence_before();
@@ -1350,9 +1415,11 @@ __device__ __forceinline__ float add_f32_bf16lo(float acc, uint32_t w) {
     asm("{\n\t.reg .b16 lo, hi;\n\tmov.b32 {lo, hi}, %1;\n\tadd.rn.f32.bf16 %0, lo, %0;\n\t}" : "+f"(acc) : "r"(w));
     return acc;
 }
-template <int NJ, bool EXACT>
+constexpr int OUT_BF16 = 0;  // conv2_table_gather_kernel output kinds: act2 as bf16
+constexpr int OUT_E4M3 = 1;  // act2 as e4m3 in units of its FP8 scale (DESIGN 13): 8 bytes per 16-byte table chunk
+template <int NJ, bool EXACT, int OUT>
 __device__ __forceinline__ void t2_square(const uint4* __restrict__ tab, const int* s_pat, int np2, int y, int x, int cpr_rt,
-                                          int lane, const float2 (&bs)[NJ][4], uint4 (&res)[NJ]) {
+                                          int lane, const float2 (&bs)[NJ][4], uint4 (&res)[NJ], float out_scale) {
     const int cpr = EXACT ? 32 * NJ : cpr_rt;
     uint4 v[9][NJ];
 #pragma unroll
@@ -1384,8 +1451,12 @@ __device__ __forceinline__ void t2_square(const uint4* __restrict__ tab, const i
             od[0] = __fadd2_rn(od[0], make_float2(__uint_as_float(w4[0]), __uint_as_float(w4[1])));
             od[1] = __fadd2_rn(od[1], make_float2(__uint_as_float(w4[2]), __uint_as_float(w4[3])));
         }
-        res[j] = make_uint4(pack_relu_bf16x2(ev[0], od[0].x), pack_relu_bf16x2(ev[1], od[0].y),
-                            pack_relu_bf16x2(ev[2], od[1].x), pack_relu_bf16x2(ev[3], od[1].y));
+        if constexpr (OUT == OUT_BF16)
+            res[j] = make_uint4(pack_relu_bf16x2(ev[0], od[0].x), pack_relu_bf16x2(ev[1], od[0].y),
+                                pack_relu_bf16x2(ev[2], od[1].x), pack_relu_bf16x2(ev[3], od[1].y));
+        else  // channels 0..7 of the chunk are ev0, od0.x, ev1, od0.y, ev2, od1.x, ev3, od1.y
+            res[j] = make_uint4(pack_relu_e4m3x4(ev[0] * out_scale, od[0].x * out_scale, ev[1] * out_scale, od[0].y * out_scale),
+                                pack_relu_e4m3x4(ev[2] * out_scale, od[1].x * out_scale, ev[3] * out_scale, od[1].y * out_scale), 0u, 0u);
     }
 }
 
@@ -1409,7 +1480,9 @@ __device__ __forceinline__ uint4 bf8_sub(const uint4& a, const uint4& b) {
 //               top to bottom, keeps the previous two (bf16-rounded) squares in registers and stores the input transform
 //               V [4][Bmax][T][n][C]:  V0 = d0-d2, V1 = d1+d2, V2 = d2-d1 when row 2ty+2 arrives, V3 = d1-d3 at row 2ty+3
 //               (bf16 subtraction of bf16 values: one rounding of the exact difference).
-template <int NJ, bool WINO, bool EXACT>  // 16-byte chunks per lane: C <= 256 * NJ (C = 128: NJ = 1, upper half-warp idle)
+// OUT = OUT_E4M3 (FP8 networks, WINO = false): act2 [B][n][n][C] as e4m3 bytes, e4m3_rn(relu(acc) * bias[C]); `bias` then
+//               holds C biases followed by 1 / sa_2, the reciprocal of act2's FP8 scale.
+template <int NJ, bool WINO, bool EXACT, int OUT>  // 16-byte chunks per lane: C <= 256 * NJ (C = 128: NJ = 1, upper half-warp idle)
 __global__ void __launch_bounds__(256, 2)
 conv2_table_gather_kernel(const u64* __restrict__ own, const u64* __restrict__ opp, const int* __restrict__ count,
                           int max_count, int n, int C, const bf16* __restrict__ table2, const float* __restrict__ bias,
@@ -1430,6 +1503,7 @@ conv2_table_gather_kernel(const u64* __restrict__ own, const u64* __restrict__ o
             bs[j][i] = (EXACT || ch < cpr) ? make_float2(bias[ch * 8 + 2 * i], bias[ch * 8 + 2 * i + 1]) : make_float2(0.f, 0.f);
     }
     const uint4* tab = reinterpret_cast<const uint4*>(table2);
+    const float out_scale = OUT == OUT_E4M3 ? bias[C] : 1.0f;
     for (int b = blockIdx.x; b < L; b += gridDim.x) {
         const u64 o = own[b], q = opp[b];
         if (threadIdx.x < np2 * np2) {
@@ -1458,12 +1532,21 @@ conv2_table_gather_kernel(const u64* __restrict__ own, const u64* __restrict__ o
             for (int pos = warp; pos < nsq; pos += 8) {
                 const int y = pos / n, x = pos - y * n;
                 uint4 res[NJ];
-                t2_square<NJ, EXACT>(tab, s_pat, np2, y, x, cpr, lane, bs, res);
-                uint4* orow = reinterpret_cast<uint4*>(out + ((size_t)b * nsq + pos) * C);
+                t2_square<NJ, EXACT, OUT>(tab, s_pat, np2, y, x, cpr, lane, bs, res, out_scale);
+                if constexpr (OUT == OUT_BF16) {
+                    uint4* orow = reinterpret_cast<uint4*>(out + ((size_t)b * nsq + pos) * C);
 #pragma unroll
-                for (int j = 0; j < NJ; ++j) {
-                    const int ch = lane + 32 * j;
-                    if (EXACT || ch < cpr) orow[ch] = res[j];
+                    for (int j = 0; j < NJ; ++j) {
+                        const int ch = lane + 32 * j;
+                        if (EXACT || ch < cpr) orow[ch] = res[j];
+                    }
+                } else {
+                    uint2* orow = reinterpret_cast<uint2*>(reinterpret_cast<uint8_t*>(out) + ((size_t)b * nsq + pos) * C);
+#pragma unroll
+                    for (int j = 0; j < NJ; ++j) {
+                        const int ch = lane + 32 * j;
+                        if (EXACT || ch < cpr) orow[ch] = make_uint2(res[j].x, res[j].y);
+                    }
                 }
             }
         } else {
@@ -1475,7 +1558,7 @@ conv2_table_gather_kernel(const u64* __restrict__ own, const u64* __restrict__ o
 #pragma unroll 1
                 for (int y = 0; y < n; ++y) {
                     uint4 cur[NJ];
-                    t2_square<NJ, EXACT>(tab, s_pat, np2, y, x, cpr, lane, bs, cur);
+                    t2_square<NJ, EXACT, OUT>(tab, s_pat, np2, y, x, cpr, lane, bs, cur, out_scale);
                     if (y >= 2) {
                         if (!(y & 1)) {
                             const int ty = (y - 2) >> 1;
@@ -1539,6 +1622,52 @@ __global__ void fold_weights_kernel(const float* __restrict__ W, const float* __
     }
 }
 
+// ---- FP8 evaluation (DESIGN 13): load-time quantisation and calibration -------------------------------------------------
+// Wq[o][k] = e4m3_rn_satfinite(W'[k][o] / sw[o]) with W' the BN-folded fp32 weight (the same product fold_weights_kernel
+// casts to bf16) and sw[o] = amax_k |W'[k][o]| / 448 (1 for an all-zero channel).  A block owns 32 output channels.
+__global__ void quantize_weights_e4m3_kernel(const float* __restrict__ W, const float* __restrict__ gamma,
+                                             const float* __restrict__ var, float eps, int K, int Nout,
+                                             uint8_t* __restrict__ Wq, float* __restrict__ sw) {
+    __shared__ float red[8][33];
+    const int o = blockIdx.x * 32 + threadIdx.x;
+    const bool on = o < Nout;
+    const float s = on ? gamma[o] / sqrtf(var[o] + eps) : 0.f;
+    float m = 0.f;
+    if (on)
+        for (int k = threadIdx.y; k < K; k += blockDim.y) m = fmaxf(m, fabsf(W[(size_t)k * Nout + o] * s));
+    red[threadIdx.y][threadIdx.x] = m;
+    __syncthreads();
+    for (int i = 0; i < 8; ++i) m = fmaxf(m, red[i][threadIdx.x]);
+    const float scale = m > 0.f ? m / 448.0f : 1.0f;
+    if (!on) return;
+    if (threadIdx.y == 0) sw[o] = scale;
+    for (int k = threadIdx.y; k < K; k += blockDim.y)
+        Wq[(size_t)o * K + k] = (uint8_t)__nv_cvt_float_to_fp8(W[(size_t)k * Nout + o] * s / scale, __NV_SATFINITE, __NV_E4M3);
+}
+
+// Largest value of the first count*per_board elements of a (non-negative, post-ReLU) bf16 activation, folded into *out
+// as fp32 bits (non-negative floats order like their bit patterns).
+__global__ void amax_bf16_kernel(const int* __restrict__ count, int max_count, const bf16* __restrict__ x, long long per_board,
+                                 unsigned* __restrict__ out) {
+    int L = *count;
+    if (L > max_count) L = max_count;
+    const long long n = (long long)L * per_board;
+    float m = 0.f;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+        m = fmaxf(m, __bfloat162float(x[i]));
+    const unsigned u = __reduce_max_sync(0xffffffffu, __float_as_uint(m));
+    if ((threadIdx.x & 31) == 0 && u) atomicMax(out, u);
+}
+
+// Epilogue coefficients of an FP8 layer: alpha[o] = sa_in * sw[o] / sa_out, beta[o] = bias[o] / sa_out.
+__global__ void fp8_coef_kernel(const float* __restrict__ sw, const float* __restrict__ bias, float sa_in, float sa_out, int n,
+                                float* __restrict__ alpha, float* __restrict__ beta) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    alpha[i] = sa_in * sw[i] / sa_out;
+    beta[i] = bias[i] / sa_out;
+}
+
 typedef CUresult (*PFN_tmapEncodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                         const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                         CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -1563,9 +1692,15 @@ struct OzLayer {
     GemmParams p;
     int block_n;
     int epi;
+    int op = OP_BF16;  // operand kind of the SM-pair kernel (FP8 layers: OP_FP8_*)
     int max_tiles;
     double flops_per_board;
 };
+
+// Calibration set of the FP8 activation scales (DESIGN 13): every position (side to move's frame) of CAL_GAMES uniformly
+// random games under the reference rules, from the RNG streams stream_key(CAL_SEED, game).
+constexpr int CAL_GAMES = 256;
+constexpr u64 CAL_SEED = 0xCA11B7A7Eull;
 
 struct OzNet {
     int n = 0, C = 0, Bmax = 0;
@@ -1593,6 +1728,19 @@ struct OzNet {
     bf16 *w[6] = {nullptr}; float* bias[6] = {nullptr};  // conv2, conv3, conv4, fc1, fc2, heads
     bf16 *act1 = nullptr, *act2 = nullptr, *act3 = nullptr, *act4 = nullptr, *f1 = nullptr, *f2 = nullptr;
     OzLayer layer[6];
+    // FP8 evaluation (OZ_NET_FP8, fixed at the first load): conv3, conv4, fc1 as layer8[0..2].  The bf16 layers stay
+    // set up: the calibration forward runs the bf16 gather, conv3 and conv4.
+    bool fp8 = false;
+    uint8_t* w8[3] = {nullptr};                       // [Nout][K] e4m3
+    float *sw8[3] = {nullptr}, *alpha8[3] = {nullptr}, *beta8[3] = {nullptr};
+    float* gcoef = nullptr;                           // the FP8 gather's bias[C] + 1 / sa_2
+    uint8_t *act2_8 = nullptr, *act3_8 = nullptr, *act4_8 = nullptr;
+    OzLayer layer8[3];
+    float sa[3] = {1.f, 1.f, 1.f};                   // act2, act3, act4
+    u64 *cal_own = nullptr, *cal_opp = nullptr;
+    int* cal_counts = nullptr;                        // boards of each Bmax-sized chunk
+    int cal_positions = 0;
+    unsigned* d_amax = nullptr;
     // per-layer timing: a ring of event sets, harvested lazily so the stream is never blocked
     static constexpr int RING = 8;
     cudaEvent_t ev[RING][8] = {{nullptr}};
@@ -1600,7 +1748,7 @@ struct OzNet {
     int ev_next = 0;
     double ms_sum[8] = {0};
     long ms_cnt = 0;
-    void* allocs[32];
+    void* allocs[64];
     int n_allocs = 0;
 };
 
@@ -1692,35 +1840,46 @@ void oz_net_destroy(oz_engine* e) {
     e->net = nullptr;
 }
 
-static int make_map_A(CUtensorMap* m, bf16* base, int Cdim, int W, int H, int B, int bw, int bh, int nb) {
+// es = element bytes: 2 (bf16) or 1 (e4m3, as UINT8).  The inner box is one 128-byte swizzle row either way.
+static int make_map_A(CUtensorMap* m, void* base, int Cdim, int W, int H, int B, int bw, int bh, int nb, int es = 2) {
     PFN_tmapEncodeTiled enc = get_encode_fn();
     if (!enc) { oz_set_error("cuTensorMapEncodeTiled entry point not available"); return OZ_ERR_CUDA; }
     cuuint64_t dims[4] = {(cuuint64_t)Cdim, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B};
-    cuuint64_t strides[3] = {(cuuint64_t)Cdim * 2, (cuuint64_t)Cdim * 2 * W, (cuuint64_t)Cdim * 2 * W * H};
-    cuuint32_t box[4] = {(cuuint32_t)BLOCK_K, (cuuint32_t)bw, (cuuint32_t)bh, (cuuint32_t)nb};
+    cuuint64_t strides[3] = {(cuuint64_t)Cdim * es, (cuuint64_t)Cdim * es * W, (cuuint64_t)Cdim * es * W * H};
+    cuuint32_t box[4] = {(cuuint32_t)(128 / es), (cuuint32_t)bw, (cuuint32_t)bh, (cuuint32_t)nb};
     cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+    CUresult r = enc(m, es == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_UINT8, 4, base, dims, strides, box,
+                     estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                      CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { oz_set_error("cuTensorMapEncodeTiled(A) failed: %d", (int)r); return OZ_ERR_CUDA; }
     return OZ_OK;
 }
 
-static int make_map_B(CUtensorMap* m, bf16* base, int K, int Nout, int block_n) {
+static int make_map_B(CUtensorMap* m, void* base, int K, int Nout, int block_n, int es = 2) {
     PFN_tmapEncodeTiled enc = get_encode_fn();
     if (!enc) { oz_set_error("cuTensorMapEncodeTiled entry point not available"); return OZ_ERR_CUDA; }
     cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)Nout};
-    cuuint64_t strides[1] = {(cuuint64_t)K * 2};
-    cuuint32_t box[2] = {(cuuint32_t)BLOCK_K, (cuuint32_t)block_n};
+    cuuint64_t strides[1] = {(cuuint64_t)K * es};
+    cuuint32_t box[2] = {(cuuint32_t)(128 / es), (cuuint32_t)block_n};
     cuuint32_t estr[2] = {1, 1};
-    CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+    CUresult r = enc(m, es == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, base, dims, strides, box,
+                     estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                      CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { oz_set_error("cuTensorMapEncodeTiled(B) failed: %d", (int)r); return OZ_ERR_CUDA; }
     return OZ_OK;
 }
 
-// layer li: input [B][ih][iw][cin] -> output [B][oh*ow][nout]; ntaps 3 (conv) or 1 (fc)
-static int setup_layer(OzNet* net, OzLayer& Lr, bf16* weights, const float* bias, int bmax, bf16* in, int cin, int iw, int ih,
-                       int ow, int oh, int ntaps, int pad, int nout_pad, int block_n, int epi, bf16* out, int ldc) {
+static bool allow_2sm() {
+    static const bool allow = !(getenv("OZ_NET_NO_2SM") && getenv("OZ_NET_NO_2SM")[0] == '1');
+    return allow;
+}
+
+// layer li: input [B][ih][iw][cin] -> output [B][oh*ow][nout]; ntaps 3 (conv) or 1 (fc).  op != OP_BF16: e4m3 weights and
+// input (FP8 layers, SM-pair kernel only), epilogue coefficients alpha / bias.
+static int setup_layer(OzNet* net, OzLayer& Lr, void* weights, const float* bias, int bmax, void* in, int cin, int iw, int ih,
+                       int ow, int oh, int ntaps, int pad, int nout_pad, int block_n, int epi, void* out, int ldc,
+                       int op = OP_BF16, const float* alpha = nullptr) {
+    const int es = op == OP_BF16 ? 2 : 1;  // operand element bytes
     GemmParams& p = Lr.p;
     memset(&p, 0, sizeof(p));
     if (epi == EPI_RELU_BF16) block_n = (nout_pad % 256 == 0) ? 256 : 128;
@@ -1745,42 +1904,158 @@ static int setup_layer(OzNet* net, OzLayer& Lr, bf16* weights, const float* bias
     }
     p.ntaps_x = ntaps;
     p.pad = pad;
-    p.chunks_per_tap = cin / BLOCK_K;
+    p.chunks_per_tap = cin / (128 / es);  // k-blocks of 128 bytes
     p.num_kb = ntaps * ntaps * p.chunks_per_tap;
     p.n_tiles = nout_pad / block_n;
     p.ldc = ldc;
     p.max_count = bmax;
-    p.a_bytes = (unsigned)(p.rows_valid * BLOCK_K * 2);
+    p.a_bytes = (unsigned)(p.rows_valid * BLOCK_K * 2);  // 128 bytes per row in either operand kind
     p.bias = bias;
-    p.out = out;
+    p.alpha = alpha;
+    p.out = (bf16*)out;
     p.nsq = net->n * net->n;
     Lr.block_n = block_n;
     Lr.epi = epi;
+    Lr.op = op;
     Lr.max_tiles = ((bmax * p.tile_num + p.tile_den - 1) / p.tile_den) * p.n_tiles;
-    int rc = make_map_A(&Lr.mapA, in, cin, iw, ih, bmax, ow, oh, nb);
+    int rc = make_map_A(&Lr.mapA, in, cin, iw, ih, bmax, ow, oh, nb, es);
     if (rc) return rc;
-    rc = make_map_A(&Lr.mapA2, in, cin, iw, ih, bmax, ow, p.split ? oh / 2 : oh, p.split ? 1 : nb);
+    rc = make_map_A(&Lr.mapA2, in, cin, iw, ih, bmax, ow, p.split ? oh / 2 : oh, p.split ? 1 : nb, es);
     if (rc) return rc;
-    static const bool allow_2sm = !(getenv("OZ_NET_NO_2SM") && getenv("OZ_NET_NO_2SM")[0] == '1');
     // measured (B200, 4096 boards, division-free producers): the SM-pair kernel wins everywhere it applies - conv3 (split
     // tiles) 0.471 vs 0.518 ms, conv4 0.212 vs 0.231, fc1 0.062 vs 0.067: at the power cap the halved B-operand traffic
     // is clock headroom.  (With the old producer loop, which was the supply limit, the two kernels tied.)
-    Lr.use_2sm = allow_2sm && epi == EPI_RELU_BF16 && block_n == 256;
+    Lr.use_2sm = allow_2sm() && epi == EPI_RELU_BF16 && block_n == 256;
+    if (op != OP_BF16 && !Lr.use_2sm) {
+        oz_set_error("FP8 layers run on the SM-pair GEMM only (OZ_NET_NO_2SM=1, or an output width that is not a multiple of 256)");
+        return OZ_ERR_STATE;
+    }
     if (Lr.use_2sm) {
-        rc = make_map_B(&Lr.mapB2, weights, ntaps * ntaps * cin, nout_pad, 128);
+        rc = make_map_B(&Lr.mapB2, weights, ntaps * ntaps * cin, nout_pad, 128, es);
         if (rc) return rc;
     }
-    return make_map_B(&Lr.mapB, weights, ntaps * ntaps * cin, nout_pad, block_n);
+    return make_map_B(&Lr.mapB, weights, ntaps * ntaps * cin, nout_pad, block_n, es);
+}
+
+// One launch of the SM-pair GEMM for layer Lr (cfg carries the stream and the PDL attribute).
+static cudaError_t launch_gemm2(OzNet* net, cudaLaunchConfig_t cfg, const OzLayer& Lr, const GemmParams& p, int max_count) {
+    int m_tiles = (max_count * p.tile_num + p.tile_den - 1) / p.tile_den;
+    int pairs = ((m_tiles + 1) / 2) * p.n_tiles;
+    int g2 = 2 * pairs < (net->sm_count & ~1) ? 2 * pairs : (net->sm_count & ~1);
+    if (g2 < 2) g2 = 2;
+    cfg.gridDim = dim3(g2);
+    switch (Lr.op) {
+        case OP_FP8_E4M3:
+            cfg.dynamicSmemBytes = Gemm2Smem<OP_FP8_E4M3>::DYN_BYTES;
+            return cudaLaunchKernelEx(&cfg, oz_gemm2_kernel<OP_FP8_E4M3>, Lr.mapA, Lr.mapA2, Lr.mapB2, p);
+        case OP_FP8_BF16:
+            cfg.dynamicSmemBytes = Gemm2Smem<OP_FP8_BF16>::DYN_BYTES;
+            return cudaLaunchKernelEx(&cfg, oz_gemm2_kernel<OP_FP8_BF16>, Lr.mapA, Lr.mapA2, Lr.mapB2, p);
+        default:
+            cfg.dynamicSmemBytes = Gemm2Smem<OP_BF16>::DYN_BYTES;
+            return cudaLaunchKernelEx(&cfg, oz_gemm2_kernel<OP_BF16>, Lr.mapA, Lr.mapA2, Lr.mapB2, p);
+    }
+}
+
+// conv1∘conv2 as the table gather: act2 in bf16 (out_kind OUT_BF16; or the Winograd input transform) or e4m3 (OUT_E4M3).
+static void launch_gather(OzNet* net, cudaStream_t st, const u64* own_dev, const u64* opp_dev, const int* count_dev,
+                          int max_count, int out_kind, unsigned long long* ts) {
+    const int n = net->n, C = net->C;
+    int blocks = max_count < net->sm_count * 2 ? max_count : net->sm_count * 2;  // 2 resident CTAs/SM, grid-stride
+    const bf16* t2 = net->table2; const float* b2 = net->bias[0];
+#define OZ_T2K(NJ, W, X, O, B, OUT) conv2_table_gather_kernel<NJ, W, X, O><<<blocks, 256, 0, st>>>(own_dev, opp_dev, count_dev, max_count, n, C, t2, B, OUT, net->Bmax, ts)
+#define OZ_T2(NJ)                                                                                                       \
+    if (out_kind == OUT_E4M3) OZ_T2K(NJ, false, true, OUT_E4M3, net->gcoef, (bf16*)net->act2_8);   /* C == 256 * NJ */  \
+    else if (net->conv3_wino) { if (C == 256 * NJ) OZ_T2K(NJ, true, true, OUT_BF16, b2, net->v3); else OZ_T2K(NJ, true, false, OUT_BF16, b2, net->v3); } \
+    else { if (C == 256 * NJ) OZ_T2K(NJ, false, true, OUT_BF16, b2, net->act2); else OZ_T2K(NJ, false, false, OUT_BF16, b2, net->act2); }
+    switch (C / 256) {
+        case 0: case 1: OZ_T2(1); break;
+        case 2: OZ_T2(2); break;
+        case 3: OZ_T2(3); break;
+        default: OZ_T2(4); break;
+    }
+#undef OZ_T2
+#undef OZ_T2K
+}
+
+// Every position of the calibration games (see CAL_GAMES), in the frame of the side to move.
+static void calibration_positions(int n, std::vector<u64>& own, std::vector<u64>& opp) {
+    const u64 full = ozbb::full_mask(n);
+    for (int g = 0; g < CAL_GAMES; ++g) {
+        const u64 key = ozbb::stream_key(CAL_SEED, (u64)g);
+        u64 o, q;
+        ozbb::initial_position(n, &o, &q);  // BLACK moves first
+        u64 legal = ozbb::legal_moves(o, q, full);
+        for (int ply = 0; legal; ++ply) {
+            own.push_back(o);
+            opp.push_back(q);
+            const int sq = ozbb::kth_set_bit(legal, (int)ozbb::pick_index(ozbb::sm64(key + (u64)ply), (unsigned)ozbb::popc(legal)));
+            ozbb::play_move<ozbb::RULES_REFERENCE>(1ull << sq, &o, &q, full, &legal);
+        }
+    }
+}
+
+// FP8 activation scales: the calibration set through the bf16 gather, conv3 and conv4 in chunks of Bmax boards, the
+// largest act2 / act3 / act4 value over all of it.  A max is order-free and the tower is row-independent, so the result
+// depends on the weights, the board size and the channel count only.
+static int fp8_calibrate(oz_engine* e, OzNet* net) {
+    cudaStream_t st = e->stream;
+    const int n = net->n, C = net->C, B = net->Bmax;
+    OZ_CUDA(cudaMemsetAsync(net->d_amax, 0, 3 * sizeof(unsigned), st));
+    const long long per_board[3] = {(long long)n * n * C, (long long)(n - 2) * (n - 2) * C, (long long)(n - 4) * (n - 4) * C};
+    const bf16* acts[3] = {net->act2, net->act3, net->act4};
+    cudaLaunchConfig_t cfg{};
+    cfg.blockDim = dim3(GEMM_THREADS);
+    cfg.stream = st;
+    for (int c = 0; c * B < net->cal_positions; ++c) {
+        const int cnt = net->cal_positions - c * B < B ? net->cal_positions - c * B : B;
+        const int* count = net->cal_counts + c;
+        launch_gather(net, st, net->cal_own + (size_t)c * B, net->cal_opp + (size_t)c * B, count, cnt, OUT_BF16, nullptr);
+        OZ_CUDA(cudaGetLastError());
+        for (int li = 1; li <= 2; ++li) {
+            GemmParams p = net->layer[li].p;
+            p.count = count;
+            p.max_count = cnt;
+            OZ_CUDA(launch_gemm2(net, cfg, net->layer[li], p, cnt));
+        }
+        for (int l = 0; l < 3; ++l) {
+            long long total = cnt * per_board[l];
+            int blocks = (int)((total + 255) / 256) < net->sm_count * 4 ? (int)((total + 255) / 256) : net->sm_count * 4;
+            amax_bf16_kernel<<<blocks, 256, 0, st>>>(count, cnt, acts[l], per_board[l], net->d_amax + l);
+        }
+        OZ_CUDA(cudaGetLastError());
+        e->launches += 6;
+    }
+    unsigned amax[3];
+    OZ_CUDA(cudaMemcpyAsync(amax, net->d_amax, sizeof(amax), cudaMemcpyDeviceToHost, st));
+    OZ_CUDA(cudaStreamSynchronize(st));
+    for (int l = 0; l < 3; ++l) {
+        float a;
+        memcpy(&a, &amax[l], 4);
+        net->sa[l] = a > 0.f ? a / 448.0f : 1.0f;  // an all-zero activation: any scale represents it
+    }
+    return OZ_OK;
 }
 
 int oz_net_load(oz_engine* e, const float* blob, int64_t n_floats, int channels, bool on_device) {
     OzNet* net = e->net;
     if (!net) { oz_set_error("engine was not created with OZ_PRIOR_NET"); return OZ_ERR_STATE; }
-    const int n = net->n, C = channels, nsq = n * n, B = net->Bmax;
+    const bool fp8 = (channels & OZ_NET_FP8) != 0;
+    const int n = net->n, C = channels & ~OZ_NET_FP8, nsq = n * n, B = net->Bmax;
     OZ_REQUIRE(C >= 128 && C % 128 == 0 && C <= 1024, "channels must be a multiple of 128 in [128,1024] (got %d)", C);
     const int64_t need = oz_net_blob_floats_impl(n, C);
     OZ_REQUIRE(n_floats == need, "weight blob has %lld floats, expected %lld", (long long)n_floats, (long long)need);
     if (net->loaded && net->C != C) { oz_set_error("channel count cannot change after the first load"); return OZ_ERR_STATE; }
+    if (net->loaded && net->fp8 != fp8) {
+        oz_set_error("precision cannot change after the first load (this engine's network is %s)", net->fp8 ? "fp8" : "bf16");
+        return OZ_ERR_STATE;
+    }
+    if (fp8) {
+        OZ_REQUIRE(C % 256 == 0, "FP8 evaluation needs channels to be a multiple of 256 (got %d)", C);
+        if (!net->conv2_table) { oz_set_error("FP8 evaluation needs the conv1∘conv2 table gather, but OZ_NET_CONV2=gemm is set"); return OZ_ERR_STATE; }
+        if (net->conv3_wino) { oz_set_error("FP8 evaluation needs the direct conv3 kernel, but OZ_NET_CONV3=wino is set"); return OZ_ERR_STATE; }
+        if (!allow_2sm()) { oz_set_error("FP8 evaluation runs on the SM-pair GEMM, but OZ_NET_NO_2SM=1 is set"); return OZ_ERR_STATE; }
+    }
     cudaStream_t st = e->stream;
     const int o2 = n - 2, o4 = n - 4;
     const int K1 = o4 * o4 * C;
@@ -1864,10 +2139,49 @@ int oz_net_load(oz_engine* e, const float* blob, int64_t n_floats, int channels,
                                      GemmSmem<128>::DYN_BYTES));
         OZ_CUDA(cudaFuncSetAttribute(oz_gemm_kernel<128, EPI_RELU_BF16>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                      GemmSmem<128>::DYN_BYTES));
-        OZ_CUDA(cudaFuncSetAttribute(oz_gemm2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, Gemm2Smem::DYN_BYTES));
+        OZ_CUDA(cudaFuncSetAttribute(oz_gemm2_kernel<OP_BF16>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                     Gemm2Smem<OP_BF16>::DYN_BYTES));
         OZ_CUDA(cudaFuncSetAttribute(oz_tail_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TailSmem::DYN_BYTES));
         OZ_CUDA(cudaMemsetAsync(net->w[5], 0, 128ull * 512 * 2, st));
         OZ_CUDA(cudaMemsetAsync(net->bias[5], 0, 128 * 4, st));
+        if (fp8) {
+            net->fp8 = true;
+            const int kin[3] = {9 * C, 9 * C, K1}, nout[3] = {C, C, 1024};
+            for (int i = 0; i < 3; ++i) {
+                if ((rc = net_alloc(net, (void**)&net->w8[i], (size_t)kin[i] * nout[i]))) return rc;
+                if ((rc = net_alloc(net, (void**)&net->sw8[i], (size_t)nout[i] * 4))) return rc;
+                if ((rc = net_alloc(net, (void**)&net->alpha8[i], (size_t)nout[i] * 4))) return rc;
+                if ((rc = net_alloc(net, (void**)&net->beta8[i], (size_t)nout[i] * 4))) return rc;
+            }
+            if ((rc = net_alloc(net, (void**)&net->gcoef, (size_t)(C + 1) * 4))) return rc;
+            if ((rc = net_alloc(net, (void**)&net->act2_8, (size_t)B * nsq * C))) return rc;
+            if ((rc = net_alloc(net, (void**)&net->act3_8, (size_t)B * o2 * o2 * C))) return rc;
+            if ((rc = net_alloc(net, (void**)&net->act4_8, (size_t)B * o4 * o4 * C))) return rc;
+            if ((rc = net_alloc(net, (void**)&net->d_amax, 16))) return rc;
+            if ((rc = setup_layer(net, net->layer8[0], net->w8[0], net->beta8[0], B, net->act2_8, C, n, n, o2, o2, 3, 0, C, 256,
+                                  EPI_RELU_BF16, net->act3_8, C, OP_FP8_E4M3, net->alpha8[0]))) return rc;
+            if ((rc = setup_layer(net, net->layer8[1], net->w8[1], net->beta8[1], B, net->act3_8, C, o2, o2, o4, o4, 3, 0, C, 256,
+                                  EPI_RELU_BF16, net->act4_8, C, OP_FP8_E4M3, net->alpha8[1]))) return rc;
+            if ((rc = setup_layer(net, net->layer8[2], net->w8[2], net->beta8[2], B, net->act4_8, K1, 1, 1, 1, 1, 1, 0, 1024, 256,
+                                  EPI_RELU_BF16, net->f1, 1024, OP_FP8_BF16, net->alpha8[2]))) return rc;
+            OZ_CUDA(cudaFuncSetAttribute(oz_gemm2_kernel<OP_FP8_E4M3>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         Gemm2Smem<OP_FP8_E4M3>::DYN_BYTES));
+            OZ_CUDA(cudaFuncSetAttribute(oz_gemm2_kernel<OP_FP8_BF16>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         Gemm2Smem<OP_FP8_BF16>::DYN_BYTES));
+            std::vector<u64> own, opp;
+            calibration_positions(n, own, opp);
+            net->cal_positions = (int)own.size();
+            const int chunks = (net->cal_positions + B - 1) / B;
+            std::vector<int> counts(chunks);
+            for (int c = 0; c < chunks; ++c) counts[c] = net->cal_positions - c * B < B ? net->cal_positions - c * B : B;
+            if ((rc = net_alloc(net, (void**)&net->cal_own, own.size() * 8))) return rc;
+            if ((rc = net_alloc(net, (void**)&net->cal_opp, opp.size() * 8))) return rc;
+            if ((rc = net_alloc(net, (void**)&net->cal_counts, (size_t)chunks * 4))) return rc;
+            OZ_CUDA(cudaMemcpyAsync(net->cal_own, own.data(), own.size() * 8, cudaMemcpyHostToDevice, st));
+            OZ_CUDA(cudaMemcpyAsync(net->cal_opp, opp.data(), opp.size() * 8, cudaMemcpyHostToDevice, st));
+            OZ_CUDA(cudaMemcpyAsync(net->cal_counts, counts.data(), (size_t)chunks * 4, cudaMemcpyHostToDevice, st));
+            OZ_CUDA(cudaStreamSynchronize(st));
+        }
     }
     // stage the blob on the device
     const float* d = blob;
@@ -1886,6 +2200,7 @@ int oz_net_load(oz_engine* e, const float* blob, int64_t n_floats, int channels,
     const float* q = d;
     auto take = [&](int64_t cnt) { const float* r = q; q += cnt; return r; };
     dim3 tb(32, 8);
+    const float *q_w[3], *q_g[3], *q_v[3];  // fp32 conv3, conv4, fc1 kernels and BN scale inputs (FP8 quantisation)
     {   // conv1 + bn1 -> table
         const float* w1 = take(18LL * C); const float* b1 = take(C);
         const float* g = take(C); const float* be = take(C); const float* mu = take(C); const float* va = take(C);
@@ -1900,6 +2215,7 @@ int oz_net_load(oz_engine* e, const float* blob, int64_t n_floats, int channels,
         fold_weights_kernel<<<dim3((K + 31) / 32, (C + 31) / 32), tb, 0, st>>>(w, b, g, be, mu, va, eps, K, C, net->w[li], net->bias[li]);
         OZ_CUDA(cudaGetLastError());
         e->launches++;
+        if (li > 0) { q_w[li - 1] = w; q_g[li - 1] = g; q_v[li - 1] = va; }
         if (li == 1 && net->conv3_wino) {
             wino_weights_kernel<<<net->sm_count * 8, 256, 0, st>>>(w, g, va, eps, C, net->u3);
             OZ_CUDA(cudaGetLastError());
@@ -1931,6 +2247,7 @@ int oz_net_load(oz_engine* e, const float* blob, int64_t n_floats, int channels,
         fold_weights_kernel<<<dim3((K1 + 31) / 32, 32), tb, 0, st>>>(w, b, g, be, mu, va, eps, K1, 1024, net->w[3], net->bias[3]);
         OZ_CUDA(cudaGetLastError());
         e->launches++;
+        q_w[2] = w; q_g[2] = g; q_v[2] = va;
     }
     {   // fc2 + bn6
         const float* w = take(1024LL * 512); const float* b = take(512);
@@ -1950,8 +2267,43 @@ int oz_net_load(oz_engine* e, const float* blob, int64_t n_floats, int channels,
         OZ_CUDA(cudaGetLastError());
         e->launches += 2;
     }
+    if (net->fp8) {  // DESIGN 13: quantise conv3 / conv4 / fc1, calibrate the activation scales, build the epilogue coefficients
+        const int kin[3] = {9 * C, 9 * C, K1}, nout[3] = {C, C, 1024};
+        for (int i = 0; i < 3; ++i) {
+            quantize_weights_e4m3_kernel<<<(nout[i] + 31) / 32, tb, 0, st>>>(q_w[i], q_g[i], q_v[i], eps, kin[i], nout[i], net->w8[i],
+                                                                             net->sw8[i]);
+            OZ_CUDA(cudaGetLastError());
+            e->launches++;
+        }
+        if ((rc = fp8_calibrate(e, net))) return rc;  // synchronises: the staged blob is no longer read after this
+        const float sa_out[3] = {net->sa[1], net->sa[2], 1.0f};  // fc1 writes bf16 in real units
+        for (int i = 0; i < 3; ++i) {
+            fp8_coef_kernel<<<(nout[i] + 255) / 256, 256, 0, st>>>(net->sw8[i], net->bias[i + 1], net->sa[i], sa_out[i], nout[i],
+                                                                   net->alpha8[i], net->beta8[i]);
+            OZ_CUDA(cudaGetLastError());
+            e->launches++;
+        }
+        const float inv_sa2 = 1.0f / net->sa[0];
+        OZ_CUDA(cudaMemcpyAsync(net->gcoef, net->bias[0], (size_t)C * 4, cudaMemcpyDeviceToDevice, st));
+        OZ_CUDA(cudaMemcpyAsync(net->gcoef + C, &inv_sa2, 4, cudaMemcpyHostToDevice, st));
+    }
     OZ_CUDA(cudaStreamSynchronize(st));
     net->loaded = true;
+    return OZ_OK;
+}
+
+int oz_net_scales(oz_engine* e, float* out) {
+    OzNet* net = e->net;
+    if (!net || !net->loaded || !net->fp8) {
+        oz_set_error("no FP8 network is loaded (oz_net_load_weights with OZ_NET_FP8)");
+        return OZ_ERR_STATE;
+    }
+    const int C = net->C;
+    for (int l = 0; l < 3; ++l) out[l] = net->sa[l];
+    OZ_CUDA(cudaMemcpyAsync(out + 3, net->sw8[0], (size_t)C * 4, cudaMemcpyDeviceToHost, e->stream));
+    OZ_CUDA(cudaMemcpyAsync(out + 3 + C, net->sw8[1], (size_t)C * 4, cudaMemcpyDeviceToHost, e->stream));
+    OZ_CUDA(cudaMemcpyAsync(out + 3 + 2 * C, net->sw8[2], 1024 * 4, cudaMemcpyDeviceToHost, e->stream));
+    OZ_CUDA(cudaStreamSynchronize(e->stream));
     return OZ_OK;
 }
 
@@ -1979,27 +2331,13 @@ int oz_net_forward(oz_engine* e, const u64* own_dev, const u64* opp_dev, const i
     }
     if (tm) cudaEventRecord(ev[1], st);
     if (net->conv2_table) {  // conv1 + conv2 in one gather-sum over the partial-product table
-        int blocks = max_count < net->sm_count * 2 ? max_count : net->sm_count * 2;  // 2 resident CTAs/SM, grid-stride
-        const bf16* t2 = net->table2; const float* b2 = net->bias[0];
-        unsigned long long* ts = trace_slot(net, "gather");
-#define OZ_T2K(NJ, W, X, OUT) conv2_table_gather_kernel<NJ, W, X><<<blocks, 256, 0, st>>>(own_dev, opp_dev, count_dev, max_count, n, C, t2, b2, OUT, net->Bmax, ts)
-#define OZ_T2(NJ)                                                                  \
-    if (net->conv3_wino) { if (C == 256 * NJ) OZ_T2K(NJ, true, true, net->v3); else OZ_T2K(NJ, true, false, net->v3); } \
-    else { if (C == 256 * NJ) OZ_T2K(NJ, false, true, net->act2); else OZ_T2K(NJ, false, false, net->act2); }
-        switch (C / 256) {
-            case 0: case 1: OZ_T2(1); break;
-            case 2: OZ_T2(2); break;
-            case 3: OZ_T2(3); break;
-            default: OZ_T2(4); break;
-        }
-#undef OZ_T2
-#undef OZ_T2K
+        launch_gather(net, st, own_dev, opp_dev, count_dev, max_count, net->fp8 ? OUT_E4M3 : OUT_BF16, trace_slot(net, "gather"));
         OZ_CUDA(cudaGetLastError());
         e->launches++;
         if (tm) cudaEventRecord(ev[2], st);
     }
     for (int li = net->conv2_table ? 1 : 0; li < 6; ++li) {
-        OzLayer& Lr = net->layer[li];
+        OzLayer& Lr = (net->fp8 && li >= 1 && li <= 3) ? net->layer8[li - 1] : net->layer[li];
         GemmParams p = Lr.p;
         p.count = count_dev;
         p.max_count = max_count;
@@ -2060,13 +2398,7 @@ int oz_net_forward(oz_engine* e, const u64* own_dev, const u64* opp_dev, const i
             cfg.dynamicSmemBytes = WinoSmem::DYN_BYTES;
             lerr = cudaLaunchKernelEx(&cfg, oz_wino_kernel, net->mapV, net->mapU, wp);
         } else if (Lr.use_2sm) {
-            int m_tiles = (max_count * p.tile_num + p.tile_den - 1) / p.tile_den;
-            int pairs = ((m_tiles + 1) / 2) * p.n_tiles;
-            int g2 = 2 * pairs < (net->sm_count & ~1) ? 2 * pairs : (net->sm_count & ~1);
-            if (g2 < 2) g2 = 2;
-            cfg.gridDim = dim3(g2);
-            cfg.dynamicSmemBytes = Gemm2Smem::DYN_BYTES;
-            lerr = cudaLaunchKernelEx(&cfg, oz_gemm2_kernel, Lr.mapA, Lr.mapA2, Lr.mapB2, p);
+            lerr = launch_gemm2(net, cfg, Lr, p, max_count);
         } else if (Lr.epi == EPI_RELU_BF16 && Lr.block_n == 256) {
             cfg.gridDim = dim3(grid);
             cfg.dynamicSmemBytes = GemmSmem<256>::DYN_BYTES;
@@ -2111,10 +2443,15 @@ int oz_net_activation(oz_engine* e, int layer, void* host, int64_t bytes) {
     OzNet* net = e->net;
     if (!net || !net->loaded) { oz_set_error("network not loaded"); return OZ_ERR_STATE; }
     const int n = net->n, C = net->C, B = net->Bmax;
-    bf16* ptrs[6] = {net->act1, net->act2, net->act3, net->act4, net->f1, net->f2};
+    void* ptrs[6] = {net->act1, net->act2, net->act3, net->act4, net->f1, net->f2};
     int64_t sizes[6] = {(int64_t)B * n * n * C, (int64_t)B * n * n * C, (int64_t)B * (n - 2) * (n - 2) * C,
                         (int64_t)B * (n - 4) * (n - 4) * C, (int64_t)B * 1024, (int64_t)B * 512};
     OZ_REQUIRE(layer >= 0 && layer < 6, "layer %d out of range", layer);
+    int64_t es = 2;  // element bytes
+    if (net->fp8 && layer >= 1 && layer <= 3) {  // e4m3 bytes
+        ptrs[layer] = layer == 1 ? net->act2_8 : layer == 2 ? net->act3_8 : net->act4_8;
+        es = 1;
+    }
     if (layer == 0 && net->conv2_table) {
         oz_set_error("conv1's output is not materialised while conv2 runs as the table gather (OZ_NET_CONV2=gemm keeps it)");
         return OZ_ERR_STATE;
@@ -2123,7 +2460,7 @@ int oz_net_activation(oz_engine* e, int layer, void* host, int64_t bytes) {
         oz_set_error("conv2's output is not materialised while conv3 runs as the Winograd kernel (the default OZ_NET_CONV3=direct keeps it)");
         return OZ_ERR_STATE;
     }
-    OZ_REQUIRE(bytes >= 0 && bytes <= sizes[layer] * 2, "bytes out of range");
+    OZ_REQUIRE(bytes >= 0 && bytes <= sizes[layer] * es, "bytes out of range");
     OZ_CUDA(cudaMemcpyAsync(host, ptrs[layer], (size_t)bytes, cudaMemcpyDeviceToHost, e->stream));
     OZ_CUDA(cudaStreamSynchronize(e->stream));
     return OZ_OK;

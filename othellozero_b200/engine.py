@@ -8,9 +8,22 @@ import numpy as np
 
 from . import _lib
 from ._lib import (PRIOR_HASH, PRIOR_HOST, PRIOR_NET, SCORINGS, SOLVE_MAX_EMPTIES, SOLVE_NONE, WINNER_DRAW, board_arg,
-                   check, f32p, f64p, i8p, i32p, ptr, u8p, u32p, u64p)
+                   channels_arg, check, f32p, f64p, i8p, i32p, ptr, u8p, u32p, u64p)
 
 M64 = (1 << 64) - 1
+
+
+def _e4m3_values() -> np.ndarray:
+    """float32 value of each e4m3 (OCP E4M3FN) byte: 1 sign, 4 exponent (bias 7), 3 mantissa bits; 0x7f / 0xff = NaN."""
+    b = np.arange(256)
+    e, m = (b >> 3) & 15, b & 7
+    mag = np.where(e == 0, m / 8.0 * 2.0 ** -6, (1 + m / 8.0) * 2.0 ** (e - 7))
+    v = np.where(b & 128, -mag, mag)
+    v[(b & 127) == 127] = np.nan
+    return v.astype(np.float32)
+
+
+E4M3_VALUES = _e4m3_values()
 
 
 def _u64(a):
@@ -130,6 +143,7 @@ class Engine:
         self._L = _lib.load()
         self.board_size = board_size
         self.rules = rules
+        self.precision, self.channels = "bf16", 0  # of the loaded network (load_weights)
         self.scoring = scoring
         self.nsq = board_size * board_size
         self.max_games = max_games
@@ -260,12 +274,25 @@ class Engine:
         return b, w, p
 
     # -- network -----------------------------------------------------------------------------------
-    def load_weights(self, blob: np.ndarray, channels: int):
+    def load_weights(self, blob: np.ndarray, channels: int, precision: str = "bf16"):
+        """`precision`: "bf16" or "fp8" (conv3, conv4, fc1 on e4m3 operands, DESIGN.md 13); fixed by the first load."""
+        arg = channels_arg(channels, precision)
         blob = np.ascontiguousarray(blob, dtype=np.float32)
-        check(self._L.oz_net_load_weights(self._h, ptr(blob, f32p), blob.size, channels))
+        check(self._L.oz_net_load_weights(self._h, ptr(blob, f32p), blob.size, arg))
+        self.precision, self.channels = precision, int(channels)
 
-    def load_weights_dev(self, dev_ptr: int, n_floats: int, channels: int):
-        check(self._L.oz_net_load_weights_dev(self._h, C.c_void_p(dev_ptr), n_floats, channels))
+    def load_weights_dev(self, dev_ptr: int, n_floats: int, channels: int, precision: str = "bf16"):
+        check(self._L.oz_net_load_weights_dev(self._h, C.c_void_p(dev_ptr), n_floats, channels_arg(channels, precision)))
+        self.precision, self.channels = precision, int(channels)
+
+    def fp8_scales(self) -> dict:
+        """Scales of the loaded FP8 network: "act" = [sa_2, sa_3, sa_4] (inputs of conv3, conv4, fc1) and the
+        per-output-channel weight scales "conv3", "conv4", "fc1".  A value x is stored as e4m3_rn(x / scale)."""
+        C_ = self.channels
+        out = np.zeros(3 + 2 * C_ + 1024, dtype=np.float32)
+        check(self._L.oz_net_fp8_scales(self._h, ptr(out, f32p)))
+        return {"act": out[:3].copy(), "conv3": out[3:3 + C_].copy(), "conv4": out[3 + C_:3 + 2 * C_].copy(),
+                "fc1": out[3 + 2 * C_:].copy()}
 
     def net_forward(self, own, opp, want_logits: bool = True):
         own, opp = _u64(np.atleast_1d(own)), _u64(np.atleast_1d(opp))
@@ -278,7 +305,12 @@ class Engine:
         return pi, lg, v
 
     def activation(self, layer: int, n_boards: int, rows: int, channels: int) -> np.ndarray:
-        """bf16 activations of the last forward as float32 [n_boards, rows, channels] (debug/tests)."""
+        """bf16 activations of the last forward as float32 [n_boards, rows, channels] (debug/tests).  An FP8 network
+        stores layers 1..3 as e4m3: those come back decoded, in units of their scale (fp8_scales()["act"][layer - 1])."""
+        if self.precision == "fp8" and 1 <= layer <= 3:
+            raw8 = np.zeros(n_boards * rows * channels, dtype=np.uint8)
+            check(self._L.oz_net_get_activation(self._h, layer, raw8.ctypes.data_as(C.c_void_p), raw8.nbytes))
+            return E4M3_VALUES[raw8].reshape(n_boards, rows, channels)
         raw = np.zeros(n_boards * rows * channels, dtype=np.uint16)
         check(self._L.oz_net_get_activation(self._h, layer, raw.ctypes.data_as(C.c_void_p), raw.nbytes))
         return (raw.astype(np.uint32) << 16).view(np.float32).reshape(n_boards, rows, channels)
@@ -289,10 +321,10 @@ class Engine:
     def stream(self) -> int:
         return int(self._L.oz_engine_stream(self._h) or 0)
 
-    def load_weights_from_tensor(self, t, channels: int):
+    def load_weights_from_tensor(self, t, channels: int, precision: str = "bf16"):
         """float32 CUDA tensor (e.g. just received by an NCCL broadcast) -> fold + cast on device."""
         assert t.is_cuda and t.dtype.is_floating_point and t.element_size() == 4 and t.is_contiguous()
-        self.load_weights_dev(t.data_ptr(), t.numel(), channels)
+        self.load_weights_dev(t.data_ptr(), t.numel(), channels, precision)
 
     # -- dist (NCCL through the C-ABI, oz_dist.cu) ---------------------------------------------------------------
     @staticmethod
@@ -307,11 +339,13 @@ class Engine:
         assert buf.size == 128
         check(self._L.oz_dist_init(self._h, rank, world, ptr(buf, u8p)))
 
-    def dist_broadcast_weights(self, blob, channels: int, root: int = 0):
+    def dist_broadcast_weights(self, blob, channels: int, root: int = 0, precision: str = "bf16"):
         """C1: `root` passes the float32 blob, the others None; every rank ends with the weights loaded."""
+        arg = channels_arg(channels, precision)
         blob = None if blob is None else np.ascontiguousarray(blob, dtype=np.float32)
         n = int(self._L.oz_net_blob_floats(self.board_size, channels))
-        check(self._L.oz_dist_broadcast_weights(self._h, ptr(blob, f32p), n, channels, root))
+        check(self._L.oz_dist_broadcast_weights(self._h, ptr(blob, f32p), n, arg, root))
+        self.precision, self.channels = precision, int(channels)
 
     def dist_gather_examples(self, rows: np.ndarray) -> np.ndarray:
         """C2: packed example rows [n, 3] uint64 of this rank -> the concatenation over all ranks, in rank order."""

@@ -47,6 +47,7 @@ class IterationConfig:
     rules: str = "reference"         # "standard": self-play and arena under standard Othello flipping
     scoring: str = "reference"       # "standard": a drawn game is a draw (z = 0; no arena win for either network)
     solve_empties: int = 0           # > 0: positions with <= this many empties get perfect-play targets (exact solver)
+    precision: str = "bf16"          # "fp8": self-play and arena nets evaluate conv3/conv4/fc1 in FP8 (training stays fp32)
 
 
 def unpack_rows(rows: np.ndarray):
@@ -76,6 +77,10 @@ class Trainer:
         import torch
         import torch.distributed as dist
         from . import buffer, net as oznet
+        from ._lib import channels_arg
+        channels_arg(cfg.channels, cfg.precision)  # ValueError for an unknown precision, before any GPU work
+        if cfg.precision == "fp8" and cfg.channels % 256:
+            raise ValueError(f"FP8 evaluation needs channels to be a multiple of 256 (got {cfg.channels})")
         self.cfg = cfg
         self.world = dist.get_world_size() if dist.is_initialized() else 1
         self.rank = dist.get_rank() if dist.is_initialized() else 0
@@ -116,7 +121,7 @@ class Trainer:
         self._sync(); t0 = time.perf_counter()
         ids = np.arange(self.next_game_id + self.rank, self.next_game_id + cfg.episodes, self.world, dtype=np.uint64)
         self.next_game_id += cfg.episodes
-        net_now = oznet.B200NNet((n, n), C, device=self.local, max_batch=8, blob=self.blob)
+        net_now = oznet.B200NNet((n, n), C, device=self.local, max_batch=8, blob=self.blob, precision=cfg.precision)
         rec = None
         if ids.size:
             sp = selfplay.SelfPlay(n, net_now, cfg.degree_exploration, max_games=min(int(ids.size), cfg.max_concurrent),
@@ -157,8 +162,8 @@ class Trainer:
         half = cfg.arena_games // 2
         mine_a = len(range(self.rank, half, self.world))
         mine_b = len(range(self.rank, cfg.arena_games - half, self.world))
-        new_net = oznet.B200NNet((n, n), C, device=self.local, max_batch=8, blob=new_blob)
-        old_net = oznet.B200NNet((n, n), C, device=self.local, max_batch=8, blob=self.old_blob)
+        new_net = oznet.B200NNet((n, n), C, device=self.local, max_batch=8, blob=new_blob, precision=cfg.precision)
+        old_net = oznet.B200NNet((n, n), C, device=self.local, max_batch=8, blob=self.old_blob, precision=cfg.precision)
         wins = draws = 0
         rng = np.random.default_rng(cfg.seed * 1000 + self.iteration * 64 + self.rank)
         for games, black_net, white_net, new_side in ((mine_a, new_net, old_net, 0), (mine_b, old_net, new_net, 1)):
@@ -205,8 +210,8 @@ class Trainer:
 
 
 def main(argv=None):
-    from ._lib import RULES, SCORINGS
-    choices = {"rules": RULES, "scoring": SCORINGS}
+    from ._lib import PRECISIONS, RULES, SCORINGS
+    choices = {"rules": RULES, "scoring": SCORINGS, "precision": PRECISIONS}
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     for f, v in asdict(IterationConfig()).items():
         ap.add_argument("--" + f.replace("_", "-"), type=type(v), default=v,

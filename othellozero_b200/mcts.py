@@ -55,7 +55,7 @@ class OthelloMCTS:
                               c_puct=float(degree_exploration), device=device, rules=rules, scoring=scoring)
         self._game = game_class(rules, scoring)
         if mode == _e.PRIOR_NET:
-            self._eng.load_weights(neural_network.blob, neural_network.channels)
+            self._eng.load_weights(neural_network.blob, neural_network.channels, neural_network.precision)
         self._eng.reset(1)
         self._root = None
 

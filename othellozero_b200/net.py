@@ -12,7 +12,7 @@ import enum
 import numpy as np
 
 from . import engine as _engine
-from ._lib import PRIOR_NET
+from ._lib import PRIOR_NET, channels_arg
 
 
 class NeuralNets(enum.Enum):
@@ -185,10 +185,12 @@ class B200NNet:
 
     ``predict(board (N,N,2)) -> (pi (N,N) float32 probabilities, v float32)`` — Net/NNet.py:70-87.
     ``train`` is not part of the self-play hot path (SURVEY §8f rank 3) and raises.
+    ``precision``: "bf16" (default) or "fp8" (conv3, conv4 and fc1 on e4m3 tcgen05 MMAs, DESIGN.md 13).  Self-play and
+    the arena evaluate a net at its own precision; training stays fp32.
     """
 
     def __init__(self, board_size=(8, 8), num_channels_1: int = 512, network=NeuralNets.ONN, device: int = 0,
-                 max_batch: int = 4096, seed: int = 0, blob: np.ndarray | None = None):
+                 max_batch: int = 4096, seed: int = 0, blob: np.ndarray | None = None, precision: str = "bf16"):
         if network is not NeuralNets.ONN:
             raise TypeError("only NeuralNets.ONN is implemented on the B200 path (BNN is out of scope)")
         self.board_size_x, self.board_size_y = board_size
@@ -198,14 +200,20 @@ class B200NNet:
         self.channels = num_channels_1
         self.device = device
         self.max_batch = max_batch
+        channels_arg(num_channels_1, precision)  # ValueError before any device work
+        self.precision = precision
         self.blob = blob if blob is not None else init_weights(self.board_size_x, num_channels_1, seed)
         self._eng = _engine.Engine(self.board_size_x, max_games=max_batch, nodes_per_game=2, prior_mode=PRIOR_NET,
                                    device=device)
-        self._eng.load_weights(self.blob, self.channels)
+        self._eng.load_weights(self.blob, self.channels, precision)
 
     def set_weights(self, blob: np.ndarray):
         self.blob = np.ascontiguousarray(blob, dtype=np.float32)
-        self._eng.load_weights(self.blob, self.channels)
+        self._eng.load_weights(self.blob, self.channels, self.precision)
+
+    def fp8_scales(self) -> dict:
+        """Engine.fp8_scales of this (precision="fp8") net."""
+        return self._eng.fp8_scales()
 
     def predict_batch(self, own, opp, want_logits: bool = False):
         """Canonical bitboards -> (pi [B,N*N], v [B]) (+ logits)."""
@@ -244,4 +252,4 @@ class B200NNet:
 
     def copy(self):
         return B200NNet((self.board_size_x, self.board_size_y), self.channels, self.network_type, self.device,
-                        self.max_batch, blob=self.blob.copy())
+                        self.max_batch, blob=self.blob.copy(), precision=self.precision)

@@ -68,10 +68,10 @@ class SelfPlay:
                                 eval_cache_log2=eval_cache_log2 if mode == _e.PRIOR_NET else 0, rules=rules,
                                 scoring=scoring)
         if mode == _e.PRIOR_NET:
-            self.engine.load_weights(neural_network.blob, neural_network.channels)
+            self.engine.load_weights(neural_network.blob, neural_network.channels, neural_network.precision)
 
     def set_weights(self, blob, channels):
-        self.engine.load_weights(blob, channels)
+        self.engine.load_weights(blob, channels, self.engine.precision)
 
     def play(self, n_games: int, policy_temperature: float = 1.0, e_greedy: float = 1.0, game_ids=None,
              black=None, white=None, player=None, max_moves: int = -1) -> dict:

@@ -1,14 +1,17 @@
 """Compares the SASS of kernels between two builds of liboz_b200.so, instruction by instruction.
 
-Kernels are matched by demangled name with the return type removed, a trailing template argument `, 0` (the
-reference-scoring instantiation, SCORING_REFERENCE) dropped and then the template arguments `<0>` (the reference-rule
-instantiation, ozbb::RULES_REFERENCE) removed: a kernel that became `template <int RULES>` is compared with its
-pre-template self, and `tree_step_kernel<R, 0>` with `tree_step_kernel<R>`.  Every instantiation of a listed kernel that
+Kernels are matched by demangled name with the return type removed, a trailing template argument `, 0` dropped and
+then the template arguments `<0>` removed.  A trailing 0 is the reference-scoring instantiation (SCORING_REFERENCE) or the
+bf16 one (OUT_BF16 of conv2_table_gather_kernel); a lone `<0>` is the reference-rule instantiation (ozbb::RULES_REFERENCE)
+or the bf16 SM-pair GEMM (OP_BF16).  So a kernel that became `template <int RULES>` or `template <int OP>` is compared with
+its pre-template self, `tree_step_kernel<R, 0>` with `tree_step_kernel<R>` and `conv2_table_gather_kernel<NJ, W, X, 0>`
+with `conv2_table_gather_kernel<NJ, W, X>`.  Every instantiation of a listed kernel that
 the OLD build has is compared.  Instruction addresses and encodings are ignored; branch and call targets are offsets
 inside the kernel's own section, so identical code gives identical text.  Needs cuobjdump and c++filt, no GPU.
 
 usage: python tools/sass_compare.py OLD.so NEW.so [kernel ...]
-       (default kernels: tree_step_kernel rules_apply_kernel perft_playout_kernel)
+       (default kernels: tree_step_kernel rules_apply_kernel perft_playout_kernel; the network's kernels, e.g.
+        oz_gemm2_kernel oz_gemm_kernel conv2_table_gather_kernel, are matched without their anonymous namespace)
 exit status 0 iff every listed kernel is identical.
 """
 from __future__ import annotations
@@ -38,8 +41,8 @@ def functions(so: str) -> dict[str, list[str]]:
 
 
 def normalize(demangled: str) -> str:
-    s = re.sub(r"^void ", "", demangled)
-    s = re.sub(r"<(\d+), 0>\(", r"<\1>(", s)
+    s = re.sub(r"^void ", "", demangled).replace("(anonymous namespace)::", "")  # oz_net.cu's kernels
+    s = re.sub(r", 0>\(", ">(", s)
     return s.replace("<0>(", "(")
 
 
