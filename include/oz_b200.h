@@ -197,6 +197,25 @@ int oz_search_get_status(oz_engine* e, int32_t* status);
  * [6] transposition hits, [7] moves played. */
 int oz_engine_counters(oz_engine* e, uint64_t* out8);
 
+/* ---- search values (search and self-play) ------------------------------------------------- */
+/* How a simulation backs a child's value up to the edge that led to it.  OZ_VALUES_REFERENCE (the default) negates it at
+ * every ply, as the reference does: a move that finishes the game, or after which the opponent must pass, is credited
+ * to the wrong side.  OZ_VALUES_STANDARD negates it only when the move swapped the side to move: a finished child is
+ * worth +reward of the scoring to the edge that finished it, a child reached through a pass +v, every other child -v.
+ * solve_leaves = K > 0 (OZ_VALUES_STANDARD and OZ_SCORING_STANDARD only): a new, non-finished child position below the
+ * root with at most K empties is not expanded and not evaluated; its value is the sign (+1, 0, -1) of its perfect-play
+ * margin for its side to move, backed up as an integer like a terminal and cached on the edge.  The root is never
+ * solved.  Argument errors (unknown values, K outside [0, OZ_SOLVE_LEAVES_MAX], K > 0 without standard values and
+ * standard scoring) fail with OZ_ERR_INVALID before any CUDA call.  Latched by the next oz_search_reset /
+ * oz_selfplay_begin. */
+#define OZ_VALUES_REFERENCE 0
+#define OZ_VALUES_STANDARD 1
+#define OZ_SOLVE_LEAVES_MAX 12
+int oz_search_set_values(oz_engine* e, int32_t values, int32_t solve_leaves);
+/* [0] leaves solved, [1] positions the leaf solver visited (each solved leaf, its children and their subtrees); cleared
+ * with the other counters by oz_search_reset / oz_selfplay_begin. */
+int oz_search_solve_counters(oz_engine* e, uint64_t* out2);
+
 /* ---- self-play: training.execute_episode (training.py:26-72) ------------------------------ */
 /* Starts n_games episodes (start positions as oz_search_reset; a start whose side to move has no legal move is
  * rejected with OZ_ERR_INVALID).  temperature > 0: the greedy action is the first arg-max of the visit counts

@@ -19,6 +19,8 @@ SCORINGS = ("reference", "standard")
 WINNER_DRAW = 2  # OZ_WINNER_DRAW: self-play winner code of a drawn game under standard scoring
 SOLVE_MAX_EMPTIES = 20  # OZ_SOLVE_MAX_EMPTIES: the endgame solver's limit
 SOLVE_NONE = -128  # OZ_SOLVE_NONE: not a legal move (move_margin) / not searched (margin)
+VALUES = ("reference", "standard")  # OZ_VALUES_REFERENCE / OZ_VALUES_STANDARD: how the search backs values up
+SOLVE_LEAVES_MAX = 12  # OZ_SOLVE_LEAVES_MAX: the largest solve_leaves (empties of a leaf the search solves)
 NET_FP8 = 0x10000  # OZ_NET_FP8, OR-ed into a channels argument
 PRECISIONS = ("bf16", "fp8")
 
@@ -32,6 +34,22 @@ def board_arg(board_size: int, rules: str = "reference", scoring: str = "referen
     if scoring not in SCORINGS:
         raise ValueError(f"scoring must be one of {SCORINGS}, got {scoring!r}")
     return board_size | (RULES_STANDARD if rules == "standard" else 0) | (SCORING_STANDARD if scoring == "standard" else 0)
+
+
+def values_arg(values: str = "reference", solve_leaves: int = 0, scoring: str = "reference") -> int:
+    """The C-ABI values argument of oz_search_set_values: "reference" (negate a child's value at every ply, the
+    reference's backup, the default) or "standard" (negate it only when the move swapped the side to move).
+    solve_leaves = K in [0, SOLVE_LEAVES_MAX] solves new leaves with at most K empties exactly; K > 0 needs
+    values="standard" and scoring="standard".  Anything else raises ValueError."""
+    if values not in VALUES:
+        raise ValueError(f"values must be one of {VALUES}, got {values!r}")
+    if isinstance(solve_leaves, bool) or not isinstance(solve_leaves, int) or not 0 <= solve_leaves <= SOLVE_LEAVES_MAX:
+        raise ValueError(f"solve_leaves must be an int in [0, {SOLVE_LEAVES_MAX}], got {solve_leaves!r}")
+    if solve_leaves and (values != "standard" or scoring != "standard"):
+        raise ValueError("solve_leaves > 0 needs values='standard' and scoring='standard' (under reference scoring a "
+                         f"drawn final position is not a function of the margin); got values={values!r}, "
+                         f"scoring={scoring!r}")
+    return VALUES.index(values)
 
 
 def channels_arg(channels: int, precision: str = "bf16") -> int:
@@ -87,6 +105,8 @@ SIGNATURES = {
     "oz_search_get_root_stats": (C.c_int, [vp, C.c_int32, f64p, f64p, i32p]),
     "oz_search_get_status": (C.c_int, [vp, i32p]),
     "oz_engine_counters": (C.c_int, [vp, u64p]),
+    "oz_search_set_values": (C.c_int, [vp, C.c_int32, C.c_int32]),
+    "oz_search_solve_counters": (C.c_int, [vp, u64p]),
     "oz_selfplay_begin": (C.c_int, [vp, C.c_int32, u64p, u64p, i32p, u64p, C.c_int32, C.c_double, C.c_double,
                                     C.c_int32]),
     "oz_selfplay_run": (C.c_int, [vp, C.c_int32, i32p]),

@@ -14,7 +14,8 @@ The reference's own drivers ``training.duel_between_neural_networks`` / ``evalua
 ``rules="standard"`` plays every game of a batched driver under standard Othello flipping; the per-game agents take the
 rule set from their game (``othello.StandardOthelloGame``).  ``scoring="standard"`` scores a game with equal disc counts
 as a draw (winner code 2, no win for either side) in the search and in the result; the per-game agents take it from
-their game too (``othello.game_class``).
+their game too (``othello.game_class``).  The batched drivers take ``values`` and ``solve_leaves``, the search's value
+convention and leaf solving (``engine.Engine``); the per-game agents search with the reference values.
 """
 from __future__ import annotations
 
@@ -115,7 +116,8 @@ def _draw_indices(rng, counts: np.ndarray) -> np.ndarray:
 
 
 def pit(board_size, net_black, net_white, num_simulations, degree_exploration=1, n_games=64, device=0, rng=None,
-        start_black=None, start_white=None, start_player=None, rules="reference", scoring="reference"):
+        start_black=None, start_white=None, start_player=None, rules="reference", scoring="reference",
+        values="reference", solve_leaves=0):
     """n_games simultaneous duels, net_black playing BLACK.  Returns dict(winner [n_games] 0/1, black, white, plies,
     points, draws [n_games] bool: equal final counts).  Under reference scoring a draw is a BLACK win (winner 0); under
     ``scoring="standard"`` its winner is 2, and both searches value drawn terminals as 0.
@@ -124,19 +126,25 @@ def pit(board_size, net_black, net_white, num_simulations, degree_exploration=1,
     ``RANDOM_AGENT`` side (RandomOthelloAgent.play, agents.py:20-24; main.py:165-197 evaluates the network against it),
     one rules launch to apply the moves.  Ties in the visit counts and the random agent's moves are drawn from ``rng``
     (Python's ``random`` like the reference, or a numpy Generator for fully vectorised draws) over the candidates in
-    row-major order.  Both sides search, and every move is applied, under ``rules``."""
+    row-major order.  Both sides search, and every move is applied, under ``rules``.  ``values`` and ``solve_leaves``
+    are the searches' value convention and leaf solving; either may be a pair (BLACK side, WHITE side), so that two
+    search settings of the same network can meet."""
     _e.board_arg(board_size, rules, scoring)
+    values = tuple(values) if isinstance(values, (tuple, list)) else (values, values)
+    solve_leaves = tuple(solve_leaves) if isinstance(solve_leaves, (tuple, list)) else (solve_leaves, solve_leaves)
+    for v, k in zip(values, solve_leaves):
+        _e.values_arg(v, k, scoring)
     rng = rng or random
     n = board_size
     nodes = num_simulations * (n * n) + 64
     engines = []
-    for net in (net_black, net_white):
+    for side, net in enumerate((net_black, net_white)):
         if isinstance(net, str) and net == RANDOM_AGENT:
             engines.append(None)
             continue
         mode = _mode_for(net)
         e = _e.Engine(n, max_games=n_games, nodes_per_game=nodes, prior_mode=mode, c_puct=float(degree_exploration),
-                      device=device, rules=rules, scoring=scoring)
+                      device=device, rules=rules, scoring=scoring, values=values[side], solve_leaves=solve_leaves[side])
         if mode == _e.PRIOR_NET:
             e.load_weights(net.blob, net.channels, net.precision)
         engines.append(e)
@@ -199,18 +207,19 @@ def pit(board_size, net_black, net_white, num_simulations, degree_exploration=1,
 
 # ---- batched arena drivers (the worker work types of workers.py:18-21,72-79) -----------------------------------------
 def duels_between_neural_networks(n_duels, board_size, neural_network_1, neural_network_2, degree_exploration,
-                                  num_simulations, device=0, rng=None, rules="reference", scoring="reference"):
+                                  num_simulations, device=0, rng=None, rules="reference", scoring="reference",
+                                  values="reference", solve_leaves=0):
     """``n_duels`` x training.duel_between_neural_networks (training.py:75-89) as one batch: network 1 plays BLACK
     (agent_1 of duel_between_agents, agents.py:71-74); each entry is 0 if network 1 won, 1 if network 2 won, and 2 for a
     draw under standard scoring."""
     out = pit(board_size, neural_network_1, neural_network_2, num_simulations, degree_exploration, n_games=n_duels,
-              device=device, rng=rng, rules=rules, scoring=scoring)
+              device=device, rng=rng, rules=rules, scoring=scoring, values=values, solve_leaves=solve_leaves)
     return [int(w) for w in out["winner"]]
 
 
 def evaluate_neural_network(board_size, total_iterations, neural_network, num_simulations, degree_exploration,
                             agent_class=RandomOthelloAgent, agent_arguments=(), device=0, rng=None, repeats=1,
-                            rules="reference", scoring="reference"):
+                            rules="reference", scoring="reference", values="reference", solve_leaves=0):
     """training.evaluate_neural_network (training.py:92-115) with the working semantics of main.py:165-197: the network
     meets ``agent_class`` (RandomOthelloAgent) in ``total_iterations`` games, colours shuffled per game; returns the
     network's wins (a draw under standard scoring is not a win).  ``repeats`` > 1 plays that many evaluations in the
@@ -218,6 +227,7 @@ def evaluate_neural_network(board_size, total_iterations, neural_network, num_si
     if agent_class is not RandomOthelloAgent:
         raise TypeError("the batched evaluation plays against RandomOthelloAgent (main.py:165-197)")
     _e.board_arg(board_size, rules, scoring)
+    _e.values_arg(values, solve_leaves, scoring)
     rng = rng or random
     games = total_iterations * repeats
     net_is_black = np.array([rng.random() < 0.5 for _ in range(games)], dtype=bool)   # random.shuffle of two agents
@@ -228,7 +238,7 @@ def evaluate_neural_network(board_size, total_iterations, neural_network, num_si
             continue
         a, b = (neural_network, RANDOM_AGENT) if black_side else (RANDOM_AGENT, neural_network)
         out = pit(board_size, a, b, num_simulations, degree_exploration, n_games=int(sel.size), device=device, rng=rng,
-                  rules=rules, scoring=scoring)
+                  rules=rules, scoring=scoring, values=values, solve_leaves=solve_leaves)
         net_won[sel] = out["winner"] == (0 if black_side else 1)
     wins = net_won.reshape(repeats, total_iterations).sum(axis=1)
     return int(wins[0]) if repeats == 1 else [int(w) for w in wins]

@@ -141,6 +141,28 @@ extern "C" int oz_engine_counters(oz_engine* e, uint64_t* out8) {
     return OZ_OK;
 }
 
+extern "C" int oz_search_set_values(oz_engine* e, int32_t values, int32_t solve_leaves) {
+    OZ_REQUIRE(e, "null engine");
+    OZ_REQUIRE(values == OZ_VALUES_REFERENCE || values == OZ_VALUES_STANDARD,
+               "values must be OZ_VALUES_REFERENCE or OZ_VALUES_STANDARD (got %d)", values);
+    OZ_REQUIRE(solve_leaves >= 0 && solve_leaves <= OZ_SOLVE_LEAVES_MAX, "solve_leaves must be in [0, %d] (got %d)",
+               OZ_SOLVE_LEAVES_MAX, solve_leaves);
+    // under reference scoring a drawn final position is worth +1 to whoever moved last: not a function of the margin
+    OZ_REQUIRE(solve_leaves == 0 || (values == OZ_VALUES_STANDARD && e->scoring == SCORING_STANDARD),
+               "solve_leaves > 0 needs standard values and standard scoring (OZ_SCORING_STANDARD)");
+    e->values_req = values;
+    e->solve_leaves_req = solve_leaves;
+    return OZ_OK;
+}
+
+extern "C" int oz_search_solve_counters(oz_engine* e, uint64_t* out2) {
+    OZ_REQUIRE(e && out2, "null argument");
+    OZ_CUDA(cudaSetDevice(e->cfg.device));
+    OZ_CUDA(cudaMemcpyAsync(out2, e->tp.solve_counters, 2 * sizeof(u64), cudaMemcpyDeviceToHost, e->stream));
+    OZ_CUDA(cudaStreamSynchronize(e->stream));
+    return OZ_OK;
+}
+
 extern "C" int oz_engine_launches(oz_engine* e, uint64_t* launches) {
     OZ_REQUIRE(e && launches, "null argument");
     *launches = e->launches;

@@ -76,6 +76,8 @@ OzHostScratch& oz_host_scratch();
 // Scorings of the tree kernel (instantiated per scoring, chosen at launch): REFERENCE counts a draw as a BLACK win,
 // STANDARD scores it as a draw (value 0, winner code OZ_WINNER_DRAW).
 enum : int { SCORING_REFERENCE = 0, SCORING_STANDARD = 1 };
+// Value conventions of the tree kernel (instantiated per convention, chosen at launch; oz_search_set_values).
+enum : int { VALUES_REFERENCE = OZ_VALUES_REFERENCE, VALUES_STANDARD = OZ_VALUES_STANDARD };
 
 // The board_size argument of the C-ABI: N (4, 6 or 8), optionally | OZ_RULES_STANDARD | OZ_SCORING_STANDARD.  -> N, the
 // ozbb rule set and the scoring (any output may be null); any other bit is OZ_ERR_INVALID.  Only the C-ABI entry points
@@ -160,6 +162,10 @@ struct OzTreeParams {
     // counters (device)
     u64* counters;  // see oz_engine_counters
     int* n_active;
+    // standard values only (appended: the fields above keep their offsets in the kernel's parameter block)
+    int solve_leaves;            // K: new child positions below the root with <= K empties are solved, not expanded
+    u64 corners, near_corners;   // the leaf solver's move ordering (oz_ordering_masks)
+    u64* solve_counters;         // [0] leaves solved, [1] solver positions (oz_search_solve_counters)
 };
 
 struct OzNet;  // oz_net.cu
@@ -168,6 +174,8 @@ struct oz_engine {
     oz_engine_config cfg;      // cfg.board_size holds plain N; the flags of the caller's value are in `rules`, `scoring`
     int rules = ozbb::RULES_REFERENCE;
     int scoring = SCORING_REFERENCE;
+    int values = VALUES_REFERENCE;    // latched from the requested values by oz_tree_reset(clear)
+    int values_req = VALUES_REFERENCE, solve_leaves_req = 0;  // oz_search_set_values
     cudaStream_t stream = nullptr;
     OzTreeParams tp{};
     int n_games = 0;

@@ -24,7 +24,7 @@
 // the start of the next step.  This fills the leaf batch with few games but changes visit counts relative to the
 // sequential reference BY DESIGN; vl_width = 1 is the bit-exact mode and executes exactly the sequential code path.
 // The in-flight count of an edge lives in the top 8 bits of its N word, the node's total in the header's `vns`.
-#include "oz_engine.cuh"
+#include "oz_solve.cuh"
 
 using namespace ozbb;
 
@@ -133,15 +133,35 @@ __device__ __forceinline__ void path_set(SimPath& p, int lane, int depth, u32 no
 }
 
 // MCTS/__init__.py:68-70 for every edge of the path, lanes in parallel (a path never repeats a node).
-// (is_int, iv, fv) = the value handed to the DEEPEST edge; it alternates sign going up (:71).
+// (is_int, iv, fv) = the value handed to the DEEPEST edge.  Reference values: it alternates sign going up (:71).
+// Standard values: edge t gets the value of edge t+1, negated iff edge t swapped the side to move.  Whether it did is read
+// off the path's own nodes: node t+1 (the child of edge t) still has node t's mover to move iff its `own` discs contain
+// node t's (a mover's discs never change colour, and a node's side to move has at least one disc).  So the sign of edge t
+// is the parity of the swaps among edges t .. depth-2 - one ballot and a popcount, and nothing to keep during the descent
+// or to park with a virtual-loss wave's pending leaves.
 constexpr int N_MASK = 0x00FFFFFF;  // low 24 bits of an N word = visits, high 8 bits = virtual (in-flight) visits
 
+template <int VALUES>
 __device__ __forceinline__ void backup_path(unsigned char* arena, const SimPath& p, int lane, int depth, bool is_int, int iv,
                                             float fv, bool vl) {
+    u64 swaps = 0;  // standard values: bit t = edge t (t < depth - 1) swapped the side to move
+    if constexpr (VALUES == VALUES_STANDARD) {
+        const u64 o0 = lane < depth ? node_at(arena, ref_off((int)p.n0))->own : 0ull;
+        const u64 o1 = lane + 32 < depth ? node_at(arena, ref_off((int)p.n1))->own : 0ull;
+        const u64 o32 = __shfl_sync(FULLW, o1, 0);
+        u64 c0 = __shfl_down_sync(FULLW, o0, 1);  // own of node t+1
+        if (lane == 31) c0 = o32;
+        const u64 c1 = __shfl_down_sync(FULLW, o1, 1);
+        const unsigned s0 = __ballot_sync(FULLW, lane + 1 < depth && (c0 & o0) != o0);
+        const unsigned s1 = __ballot_sync(FULLW, lane + 33 < depth && (c1 & o1) != o1);
+        swaps = (u64)s0 | ((u64)s1 << 32);
+    }
     for (int t = lane; t < depth; t += 32) {
         const int nref = (int)((t < 32) ? p.n0 : p.n1);
         u32 e = (t < 32) ? p.e0 : p.e1;
-        bool neg = ((depth - 1 - t) & 1) != 0;
+        bool neg;
+        if constexpr (VALUES == VALUES_STANDARD) neg = (__popcll(swaps >> t) & 1) != 0;
+        else neg = ((depth - 1 - t) & 1) != 0;
         int vi = neg ? -iv : iv;
         float vf = neg ? -fv : fv;
         OzNodeHdr* h = node_at(arena, ref_off(nref));
@@ -413,6 +433,35 @@ __device__ __noinline__ double ucb_value_call(int nraw, double q, double pj, dou
     return ucb_value(nraw, q, pj, sq_ns, c);
 }
 
+// Leaf solver (standard values, solve_leaves > 0): the sign (+1, 0, -1) of the perfect-play margin of a non-finished
+// position (own to move, `legal` its moves) with at most OZ_SOLVE_LEAVES_MAX empties, so fewer than 32 legal moves.  Lane l
+// searches the l-th legal move's child as the solver's per-move mode does (oz_solve.cu), with the null window (-1, 1):
+// fail-soft, the result is then exact in sign, which is all the search needs.  A warp max gives the position's sign.
+// Returns (positions visited << 2) | (sign + 1): the leaf, its children and their subtrees.  A real call (see above), so
+// the solver's code stays out of the descent loop.
+template <int RULES>
+__device__ __noinline__ u64 solve_leaf_call(u64 own, u64 opp, u64 legal, u64 full, u64 corners, u64 near_corners) {
+    const int lane = threadIdx.x & 31;
+    int v = -1;  // lanes without a move: the minimum, so they do not change the max
+    u64 nodes = 0;
+    if (lane < popc(legal)) {
+        u64 m = legal;
+        for (int i = 0; i < lane; ++i) m &= m - 1ull;
+        m &= 0ull - m;
+        u64 o = own, p = opp, nl;
+        const unsigned fl = play_move<RULES>(m, &o, &p, full, &nl);
+        nodes = 1;  // the child
+        int s;
+        if (fl & MOVE_FINISHED) s = popc(o) - popc(p);
+        else if (fl & MOVE_SWAPPED) s = -solve_negamax<RULES, OZ_SOLVE_LEAVES_MAX>(o, p, nl, -1, 1, full, corners, near_corners, &nodes);
+        else s = solve_negamax<RULES, OZ_SOLVE_LEAVES_MAX>(o, p, nl, -1, 1, full, corners, near_corners, &nodes);
+        v = (s > 0) - (s < 0);
+    }
+    const int best = __reduce_max_sync(FULLW, v);
+    const u32 total = __reduce_add_sync(FULLW, (u32)nodes) + 1u;  // + the leaf
+    return ((u64)total << 2) | (u64)(best + 1);
+}
+
 // The engine step.  Every warp: (1) finishes the simulations that were waiting for their leaves, (2) keeps simulating
 // until it needs another network evaluation or runs out of work.
 //
@@ -425,7 +474,7 @@ __device__ __noinline__ double ucb_value_call(int nraw, double q, double pj, dou
 #ifndef OZ_TREE_MIN_CTAS
 #define OZ_TREE_MIN_CTAS 7
 #endif
-template <int RULES, int SCORING>
+template <int RULES, int SCORING, int VALUES>
 __global__ void __launch_bounds__(TREE_WARPS * 32, OZ_TREE_MIN_CTAS) tree_step_kernel(const OzTreeParams P) {
     __shared__ double s_a[TREE_WARPS][72];  // [0,64): masked priors of the node being expanded, [64,72): its partial sums
     const int lane = threadIdx.x & 31;
@@ -515,6 +564,12 @@ __global__ void __launch_bounds__(TREE_WARPS * 32, OZ_TREE_MIN_CTAS) tree_step_k
             c_nodes += made; c_trans += 1 - made;
             if (exp_counts_as_ran) ++ran;
             do_backup = true; b_int = false; b_fv = -exp_v; b_depth = pd.depth;  // MCTS:57 returns -v to the parent
+            if constexpr (VALUES == VALUES_STANDARD) {  // ... which keeps it when the move into the leaf passed
+                if (pd.parent >= 0) {
+                    const u64 po = node_at(arena, ref_off(pd.parent))->own;
+                    if ((pd.own & po) == po) b_fv = exp_v;
+                }
+            }
         } else {
             // yield (see oz_tree_alloc): a game that keeps finding evaluator-free simulations (terminal visits, cache hits)
             // stops once the launch has lasted `time_budget` clocks - by then the other games' warps have parked their
@@ -695,18 +750,35 @@ __global__ void __launch_bounds__(TREE_WARPS * 32, OZ_TREE_MIN_CTAS) tree_step_k
                 const unsigned fl = play_move_dev<RULES>(1ull << sq, own, opp, P.full, nl);
                 if (fl & MOVE_FINISHED) {
                     // is_terminal_state -> return -reward; reward = +1 iff ch0 count >= ch1 count (draw -> BLACK)
+                    // (standard values: +reward - the finishing move did not swap the side, so nothing negates it)
                     if constexpr (SCORING == SCORING_STANDARD) {
                         // ... except that equal counts are a draw: reward 0, backed up as the integer 0
                         const int a = popc(own), b = popc(opp);
                         term_val = (a > b) ? -1 : (a < b ? 1 : 0);
+                        if constexpr (VALUES == VALUES_STANDARD) term_val = -term_val;
                         if (lane == 0) Cp[bj] = (term_val > 0) ? OZ_CH_TERM_POS : (term_val < 0 ? OZ_CH_TERM_NEG : OZ_CH_TERM_DRAW);
                     } else {
                         int reward = (popc(own) >= popc(opp)) ? 1 : -1;
-                        term_val = -reward;
+                        term_val = (VALUES == VALUES_STANDARD) ? reward : -reward;
                         if (lane == 0) Cp[bj] = (term_val > 0) ? OZ_CH_TERM_POS : OZ_CH_TERM_NEG;
                     }
                     outcome = 1;
                     break;
+                }
+                if constexpr (VALUES == VALUES_STANDARD && SCORING == SCORING_STANDARD) {
+                    // leaf solving: a new child with <= K empties is worth the sign s of its perfect-play margin for its
+                    // side to move; the child returns -s, which the edge keeps negated (s) unless the move swapped (-s)
+                    if (P.solve_leaves > 0 && popc(P.full & ~(own | opp)) <= P.solve_leaves) {
+                        const u64 r = solve_leaf_call<RULES>(own, opp, nl, P.full, P.corners, P.near_corners);
+                        const int s = (int)(r & 3ull) - 1;
+                        term_val = (fl & MOVE_SWAPPED) ? -s : s;
+                        if (lane == 0) Cp[bj] = (term_val > 0) ? OZ_CH_TERM_POS : (term_val < 0 ? OZ_CH_TERM_NEG : OZ_CH_TERM_DRAW);
+                        // counted here rather than in per-launch registers: a solve costs far more than two atomics,
+                        // and extra loop-carried locals perturb the spill order of every other instantiation
+                        if (lane == 0) { atomicAdd(&P.solve_counters[0], 1ull); atomicAdd(&P.solve_counters[1], r >> 2); }
+                        outcome = 1;
+                        break;
+                    }
                 }
                 const int found = find_ref(table_find(table, P.table_log2, arena, own, opp));
                 if (found >= 0) {  // transposition: the state already has a node
@@ -790,7 +862,7 @@ __global__ void __launch_bounds__(TREE_WARPS * 32, OZ_TREE_MIN_CTAS) tree_step_k
         }
         if (do_backup) {
             // ===== backup site (the only one): MCTS/__init__.py:67-71 ============================================
-            backup_path(arena, path, lane, b_depth, b_int, b_iv, b_fv, vl);
+            backup_path<VALUES>(arena, path, lane, b_depth, b_int, b_iv, b_fv, vl);
             ++c_sims;
             --sims_left;
         }
@@ -930,8 +1002,11 @@ int oz_tree_alloc(oz_engine* e) {
     A(path_node, u32, GV * OZ_MAX_DEPTH) A(path_edge, u32, GV * OZ_MAX_DEPTH)
     A(arena, unsigned char, (size_t)G * stride) A(bump, u32, G) A(table, u64, (size_t)G << log2)
     A(leaf_own, u64, GV) A(leaf_opp, u64, GV) A(leaf_count, int, 8)
-    A(counters, u64, 8) A(n_active, int, 4)
+    A(counters, u64, 10) A(n_active, int, 4)
     P.next_game = P.n_active + 1;
+    P.solve_counters = P.counters + 8;
+    P.solve_leaves = 0;
+    oz_ordering_masks(P.n, &P.corners, &P.near_corners);
     P.total_games = 0;
     P.q_black = P.q_white = nullptr; P.q_player = nullptr; P.q_ids = nullptr;
     if ((rc = oz_tree_reserve_records(e, (size_t)G))) return rc;
@@ -955,7 +1030,7 @@ int oz_tree_alloc(oz_engine* e) {
     if ((rc = oz_dev_alloc<float>(e, &e->leaf_v, GV))) return rc;
     P.leaf_pi = e->leaf_pi;
     P.leaf_v = e->leaf_v;
-    OZ_CUDA(cudaMemsetAsync(P.counters, 0, 8 * sizeof(u64), e->stream));
+    OZ_CUDA(cudaMemsetAsync(P.counters, 0, 10 * sizeof(u64), e->stream));
     OZ_CUDA(cudaMemsetAsync(P.status, 0, G * sizeof(int), e->stream));
     OZ_CUDA(cudaMemsetAsync(P.pend_count, 0, G * sizeof(int), e->stream));
     OZ_CUDA(cudaMemsetAsync(P.leaf_count, 0, 8 * sizeof(int), e->stream));
@@ -1058,8 +1133,10 @@ int oz_tree_reset(oz_engine* e, int n_games, const u64* black, const u64* white,
     }
     if (clear) {
         OZ_CUDA(cudaMemsetAsync(P.table, 0, ((size_t)n_games << P.table_log2) * sizeof(u64), e->stream));
-        OZ_CUDA(cudaMemsetAsync(P.counters, 0, 8 * sizeof(u64), e->stream));
+        OZ_CUDA(cudaMemsetAsync(P.counters, 0, 10 * sizeof(u64), e->stream));
         OZ_CUDA(cudaMemsetAsync(P.leaf_count, 0, sizeof(int), e->stream));
+        e->values = e->values_req;  // oz_search_set_values is latched here (search reset / self-play begin)
+        P.solve_leaves = e->solve_leaves_req;
     }
     P.G = n_games;
     tree_init_slots_kernel<<<(G + 255) / 256, 256, 0, e->stream>>>(P, n_games, d_b, d_w, d_p, d_id, clear ? 1 : 0);
@@ -1077,11 +1154,17 @@ int oz_tree_reset(oz_engine* e, int n_games, const u64* black, const u64* white,
 int oz_tree_step(oz_engine* e) {
     OzTreeParams& P = e->tp;
     int blocks = (P.G + TREE_WARPS - 1) / TREE_WARPS;
-    auto kernel = e->rules == RULES_STANDARD
-                      ? (e->scoring == SCORING_STANDARD ? tree_step_kernel<RULES_STANDARD, SCORING_STANDARD>
-                                                        : tree_step_kernel<RULES_STANDARD, SCORING_REFERENCE>)
-                      : (e->scoring == SCORING_STANDARD ? tree_step_kernel<RULES_REFERENCE, SCORING_STANDARD>
-                                                        : tree_step_kernel<RULES_REFERENCE, SCORING_REFERENCE>);
+    // one instantiation per (rule set, scoring, value convention): [rules][scoring][values]
+    static void (*const kernels[2][2][2])(const OzTreeParams) = {
+        {{tree_step_kernel<RULES_REFERENCE, SCORING_REFERENCE, VALUES_REFERENCE>,
+          tree_step_kernel<RULES_REFERENCE, SCORING_REFERENCE, VALUES_STANDARD>},
+         {tree_step_kernel<RULES_REFERENCE, SCORING_STANDARD, VALUES_REFERENCE>,
+          tree_step_kernel<RULES_REFERENCE, SCORING_STANDARD, VALUES_STANDARD>}},
+        {{tree_step_kernel<RULES_STANDARD, SCORING_REFERENCE, VALUES_REFERENCE>,
+          tree_step_kernel<RULES_STANDARD, SCORING_REFERENCE, VALUES_STANDARD>},
+         {tree_step_kernel<RULES_STANDARD, SCORING_STANDARD, VALUES_REFERENCE>,
+          tree_step_kernel<RULES_STANDARD, SCORING_STANDARD, VALUES_STANDARD>}}};
+    auto kernel = kernels[e->rules == RULES_STANDARD][e->scoring == SCORING_STANDARD][e->values == VALUES_STANDARD];
     kernel<<<blocks, TREE_WARPS * 32, 0, e->stream>>>(P);
     OZ_CUDA(cudaGetLastError());
     e->launches++;

@@ -8,7 +8,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import (PRIOR_HASH, PRIOR_HOST, PRIOR_NET, SCORINGS, SOLVE_MAX_EMPTIES, SOLVE_NONE, WINNER_DRAW, board_arg,
-                   channels_arg, check, f32p, f64p, i8p, i32p, ptr, u8p, u32p, u64p)
+                   channels_arg, check, f32p, f64p, i8p, i32p, ptr, u8p, u32p, u64p, values_arg)
 
 M64 = (1 << 64) - 1
 
@@ -133,18 +133,24 @@ class Engine:
     """oz_engine handle: node pools + per-game state for `max_games` concurrent games on one GPU.  `rules` is the rule
     set of every simulation and self-play move: "reference" (default) or "standard" Othello flipping.  `scoring` is how a
     finished game with equal disc counts is scored: "reference" (default) counts it as a BLACK win, "standard" as a draw
-    (value 0 in the search, winner code 2 in self-play records)."""
+    (value 0 in the search, winner code 2 in self-play records).  `values` is how a simulation backs values up:
+    "reference" (default) negates a child's value at every ply, as the reference does; "standard" negates it only when
+    the move swapped the side to move (a game-ending move is worth its own result, a value crossing a pass keeps its
+    sign).  `solve_leaves` = K > 0 (values="standard" and scoring="standard" only) replaces the evaluation of every new
+    leaf below the root with at most K empties by the sign of its perfect-play margin (DESIGN.md 14)."""
 
     def __init__(self, board_size: int = 8, max_games: int = 1, nodes_per_game: int = 8192,
                  prior_mode: int = PRIOR_HASH, c_puct: float = 1.0, seed: int = 0, device: int = 0,
                  log_visits: bool = False, eval_cache_log2: int = 0, vl_width: int = 1, rules: str = "reference",
-                 scoring: str = "reference"):
+                 scoring: str = "reference", values: str = "reference", solve_leaves: int = 0):
         bs = board_arg(board_size, rules, scoring)
+        va = values_arg(values, solve_leaves, scoring)
         self._L = _lib.load()
         self.board_size = board_size
         self.rules = rules
         self.precision, self.channels = "bf16", 0  # of the loaded network (load_weights)
         self.scoring = scoring
+        self.values, self.solve_leaves = values, solve_leaves
         self.nsq = board_size * board_size
         self.max_games = max_games
         self.prior_mode = prior_mode
@@ -157,6 +163,7 @@ class Engine:
         h = C.c_void_p()
         check(self._L.oz_engine_create(C.byref(cfg), C.byref(h)))
         self._h = h
+        check(self._L.oz_search_set_values(h, va, solve_leaves))
         self.n_games = self.n_slots = 0
 
     def close(self):
@@ -223,6 +230,12 @@ class Engine:
         check(self._L.oz_engine_counters(self._h, ptr(c, u64p)))
         names = ["sims", "nodes", "terminal_visits", "cache_hits", "cache_aliases", "max_depth", "transpositions", "moves"]
         return {k: int(x) for k, x in zip(names, c)}
+
+    def solve_counters(self) -> dict:
+        """Leaf-solver counters since the last reset / selfplay_begin: leaves solved, positions the solver visited."""
+        c = np.zeros(2, dtype=np.uint64)
+        check(self._L.oz_search_solve_counters(self._h, ptr(c, u64p)))
+        return {"solved_leaves": int(c[0]), "solver_nodes": int(c[1])}
 
     def launches(self) -> int:
         n = C.c_uint64(0)

@@ -48,6 +48,8 @@ class IterationConfig:
     scoring: str = "reference"       # "standard": a drawn game is a draw (z = 0; no arena win for either network)
     solve_empties: int = 0           # > 0: positions with <= this many empties get perfect-play targets (exact solver)
     precision: str = "bf16"          # "fp8": self-play and arena nets evaluate conv3/conv4/fc1 in FP8 (training stays fp32)
+    values: str = "reference"        # "standard": self-play and arena searches negate a value only when the side swapped
+    solve_leaves: int = 0            # > 0: self-play and arena searches solve new leaves with <= this many empties exactly
 
 
 def unpack_rows(rows: np.ndarray):
@@ -126,7 +128,8 @@ class Trainer:
         if ids.size:
             sp = selfplay.SelfPlay(n, net_now, cfg.degree_exploration, max_games=min(int(ids.size), cfg.max_concurrent),
                                    num_simulations=cfg.num_simulations, device=self.local, seed=cfg.seed,
-                                   rules=cfg.rules, scoring=cfg.scoring)
+                                   rules=cfg.rules, scoring=cfg.scoring, values=cfg.values,
+                                   solve_leaves=cfg.solve_leaves)
             rec = sp.play(int(ids.size), cfg.temperature, cfg.e_greedy, game_ids=ids)
             info["selfplay_sims_this_rank"] = sp.engine.counters()["sims"]
             sp.close()
@@ -169,7 +172,8 @@ class Trainer:
         for games, black_net, white_net, new_side in ((mine_a, new_net, old_net, 0), (mine_b, old_net, new_net, 1)):
             if games:
                 out = arena.pit(n, black_net, white_net, cfg.arena_simulations, cfg.degree_exploration, n_games=games,
-                                device=self.local, rng=rng, rules=cfg.rules, scoring=cfg.scoring)
+                                device=self.local, rng=rng, rules=cfg.rules, scoring=cfg.scoring, values=cfg.values,
+                                solve_leaves=cfg.solve_leaves)
                 wins += int((out["winner"] == new_side).sum())
                 draws += int(out["draws"].sum()) if cfg.scoring == "standard" else 0
         if self.world > 1:
@@ -210,17 +214,29 @@ class Trainer:
 
 
 def main(argv=None):
-    from ._lib import PRECISIONS, RULES, SCORINGS
-    choices = {"rules": RULES, "scoring": SCORINGS, "precision": PRECISIONS}
+    from ._lib import PRECISIONS, RULES, SCORINGS, VALUES
+    choices = {"rules": RULES, "scoring": SCORINGS, "precision": PRECISIONS, "values": VALUES}
+    # the two solver flags do different things and compose: one relabels training targets, the other changes the search
+    helps = {"solve_empties": "training targets: positions with <= K empties get the perfect-play winner as z "
+                              "(self-play and its search unchanged)",
+             "solve_leaves": "search: new leaves with <= K empties are solved exactly instead of evaluated by the "
+                             "network (needs --values standard --scoring standard; targets unchanged)",
+             "values": "search value backup: 'standard' negates a child's value only when the move swapped the side "
+                       "to move"}
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     for f, v in asdict(IterationConfig()).items():
-        ap.add_argument("--" + f.replace("_", "-"), type=type(v), default=v,
+        ap.add_argument("--" + f.replace("_", "-"), type=type(v), default=v, help=helps.get(f),
                         **({"choices": choices[f]} if f in choices else {}))
     ap.add_argument("--iterations", type=int, default=1)
     args = ap.parse_args(argv)
     from ._lib import SOLVE_MAX_EMPTIES
     if not 0 <= args.solve_empties <= SOLVE_MAX_EMPTIES:
         ap.error(f"--solve-empties must be in [0, {SOLVE_MAX_EMPTIES}] (got {args.solve_empties})")
+    from ._lib import values_arg
+    try:
+        values_arg(args.values, args.solve_leaves, args.scoring)
+    except ValueError as err:
+        ap.error(str(err))
     import torch
     import torch.distributed as dist
     world = int(os.environ.get("WORLD_SIZE", "1"))

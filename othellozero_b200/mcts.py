@@ -14,7 +14,9 @@ the CUDA tree kernel.  Same constructor and method names as the reference:
     ``predict`` is called once per expanded node, exactly as the reference does (OZ_PRIOR_HOST).
 Aliases ``search`` / ``getActionProb`` are the alpha-zero-general names used in BASELINE.json.
 ``rules="standard"`` searches under standard Othello flipping instead of the reference's flip rule, and
-``scoring="standard"`` values a drawn terminal as 0 instead of as a BLACK win.
+``scoring="standard"`` values a drawn terminal as 0 instead of as a BLACK win.  ``values="standard"`` negates a child's
+value only when the move swapped the side to move, and ``solve_leaves=K`` (with standard values and scoring) solves new
+leaves with at most K empties exactly (``engine.Engine``).
 """
 from __future__ import annotations
 
@@ -37,7 +39,8 @@ class HashPriorNet:
 
 class OthelloMCTS:
     def __init__(self, board_size, neural_network, degree_exploration, nodes: int = 65536, device: int = 0,
-                 rules: str = "reference", scoring: str = "reference"):
+                 rules: str = "reference", scoring: str = "reference", values: str = "reference",
+                 solve_leaves: int = 0):
         self._board_size = board_size
         self._neural_network = neural_network
         self.degree_explorarion = degree_exploration  # (sic) MCTS/__init__.py:27
@@ -52,7 +55,8 @@ class OthelloMCTS:
             mode = _e.PRIOR_HOST
         self._mode = mode
         self._eng = _e.Engine(board_size, max_games=1, nodes_per_game=nodes, prior_mode=mode,
-                              c_puct=float(degree_exploration), device=device, rules=rules, scoring=scoring)
+                              c_puct=float(degree_exploration), device=device, rules=rules, scoring=scoring,
+                              values=values, solve_leaves=solve_leaves)
         self._game = game_class(rules, scoring)
         if mode == _e.PRIOR_NET:
             self._eng.load_weights(neural_network.blob, neural_network.channels, neural_network.precision)

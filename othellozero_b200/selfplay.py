@@ -10,7 +10,10 @@ boards are true per-move snapshots unless ``reference_aliasing=True`` (the refer
 SURVEY §0.8); with e_greedy < 1 the random moves come from the engine's counter RNG, not CPython's.
 Every entry point takes ``rules="reference"`` (the reference's flip rule) or ``rules="standard"`` (standard Othello),
 and ``scoring="reference"`` (a draw counts as a BLACK win) or ``scoring="standard"`` (a draw is a draw: winner code 2,
-z = 0 for every example of the game).
+z = 0 for every example of the game).  ``values="standard"`` backs search values up with the standard sign (a child's
+value is negated only when the move swapped the side to move), and ``solve_leaves=K`` (standard values and scoring only)
+solves the search's new leaves with at most K empties exactly; this changes the search, not the targets, and composes
+with ``solve_empties``, which relabels the targets.
 """
 from __future__ import annotations
 
@@ -50,7 +53,8 @@ class SelfPlay:
 
     def __init__(self, board_size: int, neural_network, degree_exploration: float = 1.0, max_games: int = 4096,
                  num_simulations: int = 100, device: int = 0, seed: int = 0, log_visits: bool = False,
-                 eval_cache_log2: int = 22, rules: str = "reference", scoring: str = "reference"):
+                 eval_cache_log2: int = 22, rules: str = "reference", scoring: str = "reference",
+                 values: str = "reference", solve_leaves: int = 0):
         self.board_size = board_size
         self.num_simulations = num_simulations
         if isinstance(neural_network, HashPriorNet):
@@ -66,7 +70,7 @@ class SelfPlay:
                                 # identical positions reached by different games are evaluated once (results unchanged:
                                 # tests/test_gpu_net.py::test_eval_cache_is_results_preserving); 272 B per entry
                                 eval_cache_log2=eval_cache_log2 if mode == _e.PRIOR_NET else 0, rules=rules,
-                                scoring=scoring)
+                                scoring=scoring, values=values, solve_leaves=solve_leaves)
         if mode == _e.PRIOR_NET:
             self.engine.load_weights(neural_network.blob, neural_network.channels, neural_network.precision)
 
@@ -212,12 +216,14 @@ def allocate_game_ids(n: int) -> np.ndarray:
 def execute_episodes(n_episodes, board_size, neural_network, degree_exploration, num_simulations, policy_temperature,
                      e_greedy, device: int = 0, seed: int | None = None, reference_aliasing: bool = False, game_ids=None,
                      max_concurrent: int = 4096, rules: str = "reference", scoring: str = "reference",
-                     solve_empties: int = 0):
+                     solve_empties: int = 0, values: str = "reference", solve_leaves: int = 0):
     """n_episodes x training.execute_episode as one GPU job; returns a list of example lists.  At most `max_concurrent`
     episodes are in flight (node pools are per slot); the others are queued on the device and start as slots free up.
     policy_temperature may be 0 (main.py:73-76 switches to it after `temperature_threshold` iterations).
     solve_empties > 0: the target z of every position with at most that many empties comes from the winner under perfect
-    play (solve_record_winners), not from the game's outcome; not available with reference_aliasing."""
+    play (solve_record_winners), not from the game's outcome; not available with reference_aliasing.
+    values / solve_leaves: the search's value convention and leaf solving (Engine)."""
+    _e.values_arg(values, solve_leaves, scoring)
     if solve_empties and reference_aliasing:
         raise ValueError("solve_empties > 0 needs per-position targets, which reference_aliasing=True does not have")
     if seed is None:
@@ -225,7 +231,8 @@ def execute_episodes(n_episodes, board_size, neural_network, degree_exploration,
     if game_ids is None:
         game_ids = allocate_game_ids(n_episodes)
     sp = SelfPlay(board_size, neural_network, degree_exploration, max_games=min(n_episodes, max_concurrent),
-                  num_simulations=num_simulations, device=device, seed=seed, rules=rules, scoring=scoring)
+                  num_simulations=num_simulations, device=device, seed=seed, rules=rules, scoring=scoring,
+                  values=values, solve_leaves=solve_leaves)
     try:
         rec = sp.play(n_episodes, policy_temperature, e_greedy, game_ids=game_ids)
     finally:
@@ -277,13 +284,14 @@ class Worker:
 
 
 def make_b200_worker(worker_base=Worker, device: int = 0, seed: int | None = None, rules: str = "reference",
-                     scoring: str = "reference"):
+                     scoring: str = "reference", values: str = "reference", solve_leaves: int = 0):
     """Builds a ``B200Worker`` class deriving from ``worker_base`` — pass the reference's ``workers.Worker`` so that
     ``WorkerManager.add_worker``'s isinstance check (workers.py:186-190) accepts it.  seed=None (default): the
     process-wide OS-drawn seed; game ids always come from the process-wide allocator, so every run() of every worker
-    plays episodes nobody has played before (see allocate_game_ids).  ``rules`` and ``scoring`` are the rule set and the
-    scoring of every work type."""
-    _e.board_arg(8, rules, scoring)  # unknown rule sets / scorings fail here, not in the worker thread
+    plays episodes nobody has played before (see allocate_game_ids).  ``rules``, ``scoring``, ``values`` and
+    ``solve_leaves`` are the rule set, the scoring and the search values of every work type."""
+    _e.board_arg(8, rules, scoring)  # unknown rule sets / scorings / values fail here, not in the worker thread
+    _e.values_arg(values, solve_leaves, scoring)
 
     class B200Worker(worker_base):
         def __init__(self):
@@ -292,6 +300,7 @@ def make_b200_worker(worker_base=Worker, device: int = 0, seed: int | None = Non
             self.seed = seed
             self.rules = rules
             self.scoring = scoring
+            self.search_kw = dict(values=values, solve_leaves=solve_leaves)
 
         def _run(self, work_type, iterations, args, kwargs):
             # workers.py:57-65 runs the target once per iteration; here all iterations are one GPU batch and
@@ -301,17 +310,17 @@ def make_b200_worker(worker_base=Worker, device: int = 0, seed: int | None = Non
             if work_type == WorkType.EXECUTE_EPISODE:
                 logging.info(f'Task {work_type}: {iterations} episodes as one GPU job on cuda:{self.device}')
                 results = execute_episodes(iterations, *args, device=self.device, seed=self.seed, rules=self.rules,
-                                           scoring=self.scoring, **kwargs)
+                                           scoring=self.scoring, **self.search_kw, **kwargs)
             elif work_type == WorkType.DUEL_BETWEEN_NEURAL_NETWORKS:
                 from . import arena
                 logging.info(f'Task {work_type}: {iterations} duels as one GPU batch on cuda:{self.device}')
                 results = arena.duels_between_neural_networks(iterations, *args, device=self.device, rules=self.rules,
-                                                              scoring=self.scoring, **kwargs)
+                                                              scoring=self.scoring, **self.search_kw, **kwargs)
             elif work_type == WorkType.EVALUATE_NEURAL_NETWORK:
                 from . import arena
                 logging.info(f'Task {work_type}: {iterations} evaluations as one GPU batch on cuda:{self.device}')
                 results = arena.evaluate_neural_network(*args, device=self.device, repeats=iterations,
-                                                        rules=self.rules, scoring=self.scoring, **kwargs)
+                                                        rules=self.rules, scoring=self.scoring, **self.search_kw, **kwargs)
                 results = results if isinstance(results, list) else [results]
             else:
                 raise TypeError('expecting WorkType object')
@@ -319,17 +328,17 @@ def make_b200_worker(worker_base=Worker, device: int = 0, seed: int | None = Non
 
         def execute_episode(self, *args, **kwargs):
             return execute_episode(*args, device=self.device, seed=self.seed, rules=self.rules, scoring=self.scoring,
-                                   **kwargs)
+                                   **self.search_kw, **kwargs)
 
         def duel_between_neural_networks(self, *args, **kwargs):
             from . import arena
             return arena.duels_between_neural_networks(1, *args, device=self.device, rules=self.rules,
-                                                       scoring=self.scoring, **kwargs)[0]
+                                                       scoring=self.scoring, **self.search_kw, **kwargs)[0]
 
         def evaluate_neural_network(self, *args, **kwargs):
             from . import arena
             return arena.evaluate_neural_network(*args, device=self.device, rules=self.rules, scoring=self.scoring,
-                                                 **kwargs)
+                                                 **self.search_kw, **kwargs)
 
     return B200Worker
 
