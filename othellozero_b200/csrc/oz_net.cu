@@ -1957,6 +1957,16 @@ static cudaError_t launch_gemm2(OzNet* net, cudaLaunchConfig_t cfg, const OzLaye
     }
 }
 
+// 16-byte chunks per lane of conv2_table_gather_kernel for C channels: a lane covers 256 channels per chunk, so C needs
+// ceil(C / 256) of them.
+constexpr int gather_nj(int C) { return (C + 255) / 256; }
+constexpr bool gather_nj_covers_all_channel_counts() {
+    for (int C = 128; C <= 1024; C += 128)
+        if (256 * gather_nj(C) < C || gather_nj(C) > 4) return false;
+    return true;
+}
+static_assert(gather_nj_covers_all_channel_counts(), "the gather must cover every channel count oz_net_load accepts");
+
 // conv1∘conv2 as the table gather: act2 in bf16 (out_kind OUT_BF16; or the Winograd input transform) or e4m3 (OUT_E4M3).
 static void launch_gather(OzNet* net, cudaStream_t st, const u64* own_dev, const u64* opp_dev, const int* count_dev,
                           int max_count, int out_kind, unsigned long long* ts) {
@@ -1968,8 +1978,8 @@ static void launch_gather(OzNet* net, cudaStream_t st, const u64* own_dev, const
     if (out_kind == OUT_E4M3) OZ_T2K(NJ, false, true, OUT_E4M3, net->gcoef, (bf16*)net->act2_8);   /* C == 256 * NJ */  \
     else if (net->conv3_wino) { if (C == 256 * NJ) OZ_T2K(NJ, true, true, OUT_BF16, b2, net->v3); else OZ_T2K(NJ, true, false, OUT_BF16, b2, net->v3); } \
     else { if (C == 256 * NJ) OZ_T2K(NJ, false, true, OUT_BF16, b2, net->act2); else OZ_T2K(NJ, false, false, OUT_BF16, b2, net->act2); }
-    switch (C / 256) {
-        case 0: case 1: OZ_T2(1); break;
+    switch (gather_nj(C)) {
+        case 1: OZ_T2(1); break;
         case 2: OZ_T2(2); break;
         case 3: OZ_T2(3); break;
         default: OZ_T2(4); break;

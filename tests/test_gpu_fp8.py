@@ -63,7 +63,7 @@ def _code_mismatch(a, b):
 
 
 @pytest.mark.parametrize("randomize_bn", [False, True])
-@pytest.mark.parametrize("n,C", [(6, 256), (6, 512), (8, 256), (8, 512)])
+@pytest.mark.parametrize("n,C", [(6, 256), (6, 512), (8, 256), (8, 512), (6, 768), (8, 1024)])
 def test_fp8_tower_matches_emulation(n, C, randomize_bn):
     from othellozero_b200 import net
     blob = net.init_weights(n, C, seed=3, randomize_bn=randomize_bn)
@@ -80,9 +80,9 @@ def test_fp8_tower_matches_emulation(n, C, randomize_bn):
     assert np.all(sc["act"] > 0)
     epi, elg, ev, ehid = fp8_emul.forward(blob, own, opp, n, C, scales=sc)
     # layer by layer: act2 from the boards; act3 / act4 from the device's act2 / act3; the outputs from the device's act4
-    checks = [("act2", hid[0], ehid[0])]
+    checks = [("act2", hid[0], ehid["act2"])]
     for i, (src, dst) in enumerate((("act2", "act3"), ("act3", "act4"))):
-        checks.append((dst, hid[i + 1], fp8_emul.forward(blob, own, opp, n, C, scales=sc, inject={src: hid[i]})[3][i + 1]))
+        checks.append((dst, hid[i + 1], fp8_emul.forward(blob, own, opp, n, C, scales=sc, inject={src: hid[i]})[3][dst]))
     for name, a, b in checks:
         frac, small = _code_mismatch(a, b)
         print(f"  {name}: {frac:.2e} of elements differ, max |diff| {np.abs(a - b).max():.3g} (e4m3 units)")

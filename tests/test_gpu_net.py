@@ -82,7 +82,7 @@ def test_net_small_channels_single_board(conv2_mode):
     _check(8, 128, 1, 8, seed=4, conv2_mode=conv2_mode)
 
 
-@pytest.mark.parametrize("C", [256, 768, 1024])
+@pytest.mark.parametrize("C", [256, 384, 640, 768, 896, 1024])
 def test_net_other_channel_counts(C, conv2_mode):
     _check(8, C, 37, 64, seed=12, conv2_mode=conv2_mode)
 
