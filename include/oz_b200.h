@@ -216,6 +216,37 @@ int oz_search_set_values(oz_engine* e, int32_t values, int32_t solve_leaves);
  * with the other counters by oz_search_reset / oz_selfplay_begin. */
 int oz_search_solve_counters(oz_engine* e, uint64_t* out2);
 
+/* ---- root exploration (search and self-play) ------------------------------------------------ */
+/* AlphaZero's two sources of exploration, both off by default.
+ * Root noise (alpha > 0): a node gets Dirichlet(alpha) noise once, when it first serves as the root of a descent (the
+ * root's second simulation when the first one created it, a self-play move onto a reused child, a root given by
+ * oz_search_set_roots): its priors over its k legal moves become P'_j = (1 - fraction) * P_j + fraction * eta_j, in
+ * double, each operation rounded separately, and a flag in the node header is set.  A flagged node is never noised
+ * again (repeated oz_search_begin calls, oz_search_set_roots back to an old root); a noised node that later becomes an
+ * interior node keeps its mixed priors.  k = 1 is only flagged.  The evaluation cache, the network outputs and the
+ * other nodes are unchanged.
+ * Noise stream, keyed by (seed, game id, root position) and independent of ply, slot, queue order, batch and cache:
+ *   base = sm64(sm64(seed ^ 0x5EEDC01D) + game_id) (the self-play base below), rk = sm64(sm64(base ^ own) + opp) with
+ *   (own, opp) the root's discs (side to move, other side; bit r*8+c); the j-th legal move (row-major) reads the words
+ *   w_t = sm64(sm64(rk + j) + t), t = 0, 1, ..., in the order it uses uniforms u = ((w >> 11) + 1) * 2^-53 in (0, 1].
+ *   g_j ~ Gamma(alpha): Marsaglia-Tsang on a = alpha + 1 if alpha < 1, else a = alpha: d = a - 1/3, c = 1 / sqrt(9d);
+ *   repeat { z = polar normal (x = 2u - 1, y = 2u' - 1, s = xx + yy, retried unless 0 < s < 1, z = x sqrt(-2 log(s) / s));
+ *   v = 1 + cz, retried if v <= 0; v = (vv)v; u; accept dv if u < 1 - (0.0331 z^2) z^2 or log u < 0.5 z^2 + d((1 - v) +
+ *   log v) } (each loop gives up after 256 tries: the normal as 0, the gamma as d); alpha < 1: g = dv * exp(log(u) / alpha)
+ *   with one more uniform.  eta_j = g_j / S, S = g_0 + g_1 + ... summed in ascending j (1/k if S = 0).
+ *   log and exp are the engine's own, built from +, -, *, /, sqrt and integer operations (DESIGN.md 15).
+ * Sampled moves (sample_moves = M, self-play only; no effect on the search API, which plays no moves): at move index
+ * p < M the action is the first legal move (row-major) whose running visit sum exceeds
+ * u = mulhi32(draw(p, 3) >> 32, sum of the root's visits); it replaces the first arg-max (temperature > 0) or the tie
+ * draw (temperature == 0).  The e_greedy coin still applies on top.  The record's visit counts are unchanged.
+ * NaN values, alpha outside [0, OZ_DIRICHLET_ALPHA_MAX], fraction outside [0, 1] or M outside [0, OZ_SAMPLE_MOVES_MAX]
+ * fail with OZ_ERR_INVALID before any CUDA call.  (The bound on alpha keeps the sum S of up to 64 gamma variates, each
+ * about alpha, far from overflow; a Dirichlet with alpha that large is the uniform distribution to double precision.)
+ * Latched by the next oz_search_reset / oz_selfplay_begin. */
+#define OZ_DIRICHLET_ALPHA_MAX 1e6
+#define OZ_SAMPLE_MOVES_MAX 64
+int oz_search_set_exploration(oz_engine* e, double alpha, double fraction, int32_t sample_moves);
+
 /* ---- self-play: training.execute_episode (training.py:26-72) ------------------------------ */
 /* Starts n_games episodes (start positions as oz_search_reset; a start whose side to move has no legal move is
  * rejected with OZ_ERR_INVALID).  temperature > 0: the greedy action is the first arg-max of the visit counts

@@ -21,6 +21,8 @@ SOLVE_MAX_EMPTIES = 20  # OZ_SOLVE_MAX_EMPTIES: the endgame solver's limit
 SOLVE_NONE = -128  # OZ_SOLVE_NONE: not a legal move (move_margin) / not searched (margin)
 VALUES = ("reference", "standard")  # OZ_VALUES_REFERENCE / OZ_VALUES_STANDARD: how the search backs values up
 SOLVE_LEAVES_MAX = 12  # OZ_SOLVE_LEAVES_MAX: the largest solve_leaves (empties of a leaf the search solves)
+DIRICHLET_ALPHA_MAX = 1e6  # OZ_DIRICHLET_ALPHA_MAX: the largest dirichlet_alpha
+SAMPLE_MOVES_MAX = 64  # OZ_SAMPLE_MOVES_MAX: the largest sample_moves (opening plies played in proportion to visits)
 NET_FP8 = 0x10000  # OZ_NET_FP8, OR-ed into a channels argument
 PRECISIONS = ("bf16", "fp8")
 
@@ -50,6 +52,24 @@ def values_arg(values: str = "reference", solve_leaves: int = 0, scoring: str = 
                          f"drawn final position is not a function of the margin); got values={values!r}, "
                          f"scoring={scoring!r}")
     return VALUES.index(values)
+
+
+def exploration_arg(dirichlet_alpha: float = 0.0, dirichlet_fraction: float = 0.25, sample_moves: int = 0):
+    """The C-ABI arguments of oz_search_set_exploration: (alpha, fraction, M).  dirichlet_alpha = alpha >= 0 (0: no root
+    noise, the default; at most DIRICHLET_ALPHA_MAX) mixes Dirichlet(alpha) noise into each root's priors once, with weight dirichlet_fraction in
+    [0, 1]; sample_moves = M in [0, SAMPLE_MOVES_MAX] plays self-play's first M plies in proportion to the root visit
+    counts.  Non-finite values and anything out of range raise ValueError."""
+    import math
+    for name, x in (("dirichlet_alpha", dirichlet_alpha), ("dirichlet_fraction", dirichlet_fraction)):
+        if isinstance(x, bool) or not isinstance(x, (int, float)) or not math.isfinite(x):
+            raise ValueError(f"{name} must be a finite number, got {x!r}")
+    if not 0 <= dirichlet_alpha <= DIRICHLET_ALPHA_MAX:
+        raise ValueError(f"dirichlet_alpha must be in [0, {DIRICHLET_ALPHA_MAX:g}], got {dirichlet_alpha!r}")
+    if not 0 <= dirichlet_fraction <= 1:
+        raise ValueError(f"dirichlet_fraction must be in [0, 1], got {dirichlet_fraction!r}")
+    if isinstance(sample_moves, bool) or not isinstance(sample_moves, int) or not 0 <= sample_moves <= SAMPLE_MOVES_MAX:
+        raise ValueError(f"sample_moves must be an int in [0, {SAMPLE_MOVES_MAX}], got {sample_moves!r}")
+    return float(dirichlet_alpha), float(dirichlet_fraction), int(sample_moves)
 
 
 def channels_arg(channels: int, precision: str = "bf16") -> int:
@@ -107,6 +127,7 @@ SIGNATURES = {
     "oz_engine_counters": (C.c_int, [vp, u64p]),
     "oz_search_set_values": (C.c_int, [vp, C.c_int32, C.c_int32]),
     "oz_search_solve_counters": (C.c_int, [vp, u64p]),
+    "oz_search_set_exploration": (C.c_int, [vp, C.c_double, C.c_double, C.c_int32]),
     "oz_selfplay_begin": (C.c_int, [vp, C.c_int32, u64p, u64p, i32p, u64p, C.c_int32, C.c_double, C.c_double,
                                     C.c_int32]),
     "oz_selfplay_run": (C.c_int, [vp, C.c_int32, i32p]),

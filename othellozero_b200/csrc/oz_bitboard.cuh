@@ -337,7 +337,8 @@ OZ_HD unsigned pick_index(oz_u64 z, unsigned cnt) { return (unsigned)(((z >> 32)
 OZ_HD oz_u64 stream_key(oz_u64 seed, oz_u64 id) { return sm64(sm64(seed) + id); }
 // Self-play draws of move index p (training.py:48-56, othelo_mcts.py:54-62): value sm64(base + 4p + which).
 constexpr oz_u64 EPISODE_STREAM = 0x5EEDC01Dull;
-enum : unsigned { DRAW_COIN = 0u, DRAW_RANDOM_ACTION = 1u, DRAW_TIE_BREAK = 2u };
+// DRAW_SAMPLE_MOVE: the proportional draw of a sampled opening move (oz_search_set_exploration).
+enum : unsigned { DRAW_COIN = 0u, DRAW_RANDOM_ACTION = 1u, DRAW_TIE_BREAK = 2u, DRAW_SAMPLE_MOVE = 3u };
 OZ_HD oz_u64 episode_key(oz_u64 seed, oz_u64 id) { return stream_key(seed ^ EPISODE_STREAM, id); }
 OZ_HD oz_u64 episode_draw(oz_u64 base, int ply, unsigned which) { return sm64(base + 4ull * (oz_u64)ply + which); }
 

@@ -155,6 +155,19 @@ extern "C" int oz_search_set_values(oz_engine* e, int32_t values, int32_t solve_
     return OZ_OK;
 }
 
+extern "C" int oz_search_set_exploration(oz_engine* e, double alpha, double fraction, int32_t sample_moves) {
+    OZ_REQUIRE(e, "null engine");
+    OZ_REQUIRE(alpha >= 0.0 && alpha <= OZ_DIRICHLET_ALPHA_MAX, "dirichlet alpha must be in [0, %g] (got %g)",
+               OZ_DIRICHLET_ALPHA_MAX, alpha);
+    OZ_REQUIRE(fraction >= 0.0 && fraction <= 1.0, "dirichlet fraction must be in [0, 1] (got %g)", fraction);
+    OZ_REQUIRE(sample_moves >= 0 && sample_moves <= OZ_SAMPLE_MOVES_MAX, "sample_moves must be in [0, %d] (got %d)",
+               OZ_SAMPLE_MOVES_MAX, sample_moves);
+    e->dir_alpha_req = alpha;
+    e->dir_fraction_req = fraction;
+    e->sample_moves_req = sample_moves;
+    return OZ_OK;
+}
+
 extern "C" int oz_search_solve_counters(oz_engine* e, uint64_t* out2) {
     OZ_REQUIRE(e && out2, "null argument");
     OZ_CUDA(cudaSetDevice(e->cfg.device));

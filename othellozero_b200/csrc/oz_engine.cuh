@@ -107,7 +107,7 @@ struct __align__(16) OzNodeHdr {
     int ns;        // _Ns
     int k;
     int vns;       // in-flight (virtual) visits through this node; 0 outside a virtual-loss wave
-    int pad1;
+    int pad1;      // 1: the node has served as a root with exploration on (its noise is mixed in); 0 otherwise
 };
 static_assert(sizeof(OzNodeHdr) == 48, "node header layout");
 
@@ -166,6 +166,9 @@ struct OzTreeParams {
     int solve_leaves;            // K: new child positions below the root with <= K empties are solved, not expanded
     u64 corners, near_corners;   // the leaf solver's move ordering (oz_ordering_masks)
     u64* solve_counters;         // [0] leaves solved, [1] solver positions (oz_search_solve_counters)
+    // root exploration only (appended likewise; oz_search_set_exploration)
+    double dir_alpha, dir_fraction;  // Dirichlet noise mixed into each root's priors once; alpha = 0: none
+    int sample_moves;                // self-play plies p < M play a move drawn in proportion to the root visit counts
 };
 
 struct OzNet;  // oz_net.cu
@@ -176,6 +179,8 @@ struct oz_engine {
     int scoring = SCORING_REFERENCE;
     int values = VALUES_REFERENCE;    // latched from the requested values by oz_tree_reset(clear)
     int values_req = VALUES_REFERENCE, solve_leaves_req = 0;  // oz_search_set_values
+    double dir_alpha_req = 0.0, dir_fraction_req = 0.0;       // oz_search_set_exploration, latched like the values
+    int sample_moves_req = 0;
     cudaStream_t stream = nullptr;
     OzTreeParams tp{};
     int n_games = 0;

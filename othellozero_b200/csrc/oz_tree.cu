@@ -462,6 +462,152 @@ __device__ __noinline__ u64 solve_leaf_call(u64 own, u64 opp, u64 legal, u64 ful
     return ((u64)total << 2) | (u64)(best + 1);
 }
 
+// ---- root exploration (EXPLORE instantiations; oz_search_set_exploration, DESIGN.md 15) ---------------------------------
+// The Dirichlet sampler uses IEEE +, -, *, /, sqrt (each rounded separately: no FMA contraction) and integer operations
+// only, log and exp included, so that the CPU oracle's restatement in C (tests/oracle_explore.py) reproduces every bit.
+// Uniform from a stream word: ((w >> 11) + 1) * 2^-53, in (0, 1].
+__device__ __forceinline__ double x_uniform(u64 w) { return __dmul_rn((double)((w >> 11) + 1ull), 1.0 / 9007199254740992.0); }
+
+// Natural log of a positive normal x: x = m * 2^e with m in [sqrt(1/2), sqrt(2))
+// (f = m - 1 exact, s = f / (2 + f)), log m = 2s + (s z) P(z), z = s^2, P = sum of 2 / (2i + 1) z^(i-1) for i = 1..11 (Horner from i = 11),
+// log x = e * ln2_hi + (log m + e * ln2_lo).
+__device__ __forceinline__ double x_log(double x) {
+    u64 b = (u64)__double_as_longlong(x);
+    int e = (int)((b >> 52) & 0x7ffull) - 1023;
+    b = (b & 0x000FFFFFFFFFFFFFull) | 0x3FF0000000000000ull;
+    if (b > 0x3FF6A09E667F3BCDull) { b -= 0x0010000000000000ull; ++e; }
+    const double f = __dsub_rn(__longlong_as_double((long long)b), 1.0);
+    const double s = __ddiv_rn(f, __dadd_rn(2.0, f));
+    const double z = __dmul_rn(s, s);
+    double p = 0.08695652173913043;
+    p = __dadd_rn(__dmul_rn(p, z), 0.09523809523809523);
+    p = __dadd_rn(__dmul_rn(p, z), 0.10526315789473684);
+    p = __dadd_rn(__dmul_rn(p, z), 0.11764705882352941);
+    p = __dadd_rn(__dmul_rn(p, z), 0.13333333333333333);
+    p = __dadd_rn(__dmul_rn(p, z), 0.15384615384615385);
+    p = __dadd_rn(__dmul_rn(p, z), 0.18181818181818182);
+    p = __dadd_rn(__dmul_rn(p, z), 0.2222222222222222);
+    p = __dadd_rn(__dmul_rn(p, z), 0.2857142857142857);
+    p = __dadd_rn(__dmul_rn(p, z), 0.4);
+    p = __dadd_rn(__dmul_rn(p, z), 0.6666666666666666);
+    const double lm = __dadd_rn(__dmul_rn(2.0, s), __dmul_rn(__dmul_rn(s, z), p));
+    return __dadd_rn(__dmul_rn((double)e, 6.93147180369123816490e-01),
+                     __dadd_rn(lm, __dmul_rn((double)e, 1.90821492927058770002e-10)));
+}
+
+// exp x for x <= 0: k = x / ln2 rounded half away from zero, r = (x - k * ln2_hi) - k * ln2_lo, exp r by its Taylor
+// polynomial to r^13 (Horner), times 2^k (two exact scalings below 2^-1022, so the last product rounds once).  0 below -746.
+__device__ __forceinline__ double x_exp(double x) {
+    if (x < -746.0) return 0.0;
+    const double t = __dmul_rn(x, 1.4426950408889634);
+    const int k = (int)__dadd_rn(t, t < 0.0 ? -0.5 : 0.5);  // truncation
+    const double r = __dsub_rn(__dsub_rn(x, __dmul_rn((double)k, 6.93147180369123816490e-01)),
+                               __dmul_rn((double)k, 1.90821492927058770002e-10));
+    double p = 1.6059043836821613e-10;
+    p = __dadd_rn(__dmul_rn(p, r), 2.08767569878681e-09);
+    p = __dadd_rn(__dmul_rn(p, r), 2.505210838544172e-08);
+    p = __dadd_rn(__dmul_rn(p, r), 2.755731922398589e-07);
+    p = __dadd_rn(__dmul_rn(p, r), 2.7557319223985893e-06);
+    p = __dadd_rn(__dmul_rn(p, r), 2.48015873015873e-05);
+    p = __dadd_rn(__dmul_rn(p, r), 0.0001984126984126984);
+    p = __dadd_rn(__dmul_rn(p, r), 0.001388888888888889);
+    p = __dadd_rn(__dmul_rn(p, r), 0.008333333333333333);
+    p = __dadd_rn(__dmul_rn(p, r), 0.041666666666666664);
+    p = __dadd_rn(__dmul_rn(p, r), 0.16666666666666666);
+    p = __dadd_rn(__dmul_rn(p, r), 0.5);
+    p = __dadd_rn(__dmul_rn(p, r), 1.0);
+    p = __dadd_rn(__dmul_rn(p, r), 1.0);
+    if (k >= -1022) return __dmul_rn(p, __longlong_as_double((long long)((u64)(k + 1023) << 52)));
+    p = __dmul_rn(p, __longlong_as_double((long long)((u64)(k + 600 + 1023) << 52)));
+    return __dmul_rn(p, __longlong_as_double((long long)((u64)(1023 - 600) << 52)));
+}
+
+// One Gamma(alpha) variate from the words sm64(key + t), t = 0, 1, ... (one per uniform, in the order they are used).
+// Marsaglia-Tsang for a = alpha + 1 if alpha < 1 (then times U^(1/alpha) = exp(log U / alpha)), else a = alpha:
+//   d = a - 1/3, c = 1 / sqrt(9d); repeat: z = a Marsaglia-polar normal, v = 1 + c z, rejected if v <= 0, v = (v v) v,
+//   u uniform; accept d v if u < 1 - (0.0331 z^2) z^2 or log u < 0.5 z^2 + d ((1 - v) + log v).
+// The polar normal: x = 2 u1 - 1, y = 2 u2 - 1, s = x x + y y, rejected unless 0 < s < 1, z = x sqrt((-2 log s) / s).
+// Either loop gives up after 256 rejections (probability below 1e-300): the normal as 0, the gamma loop as d.
+__device__ __forceinline__ double x_gamma(double alpha, u64 key) {
+    u64 t = 0;
+    const double a = alpha < 1.0 ? __dadd_rn(alpha, 1.0) : alpha;
+    const double d = __dsub_rn(a, 0.3333333333333333);
+    const double c = __ddiv_rn(1.0, __dsqrt_rn(__dmul_rn(9.0, d)));
+    double g = d;
+#pragma unroll 1
+    for (int it = 0; it < 256; ++it) {
+        double z = 0.0;
+#pragma unroll 1
+        for (int jt = 0; jt < 256; ++jt) {
+            const double x = __dsub_rn(__dmul_rn(2.0, x_uniform(sm64(key + t))), 1.0);
+            const double y = __dsub_rn(__dmul_rn(2.0, x_uniform(sm64(key + t + 1))), 1.0);
+            t += 2;
+            const double s = __dadd_rn(__dmul_rn(x, x), __dmul_rn(y, y));
+            if (s >= 1.0 || s == 0.0) continue;
+            z = __dmul_rn(x, __dsqrt_rn(__ddiv_rn(__dmul_rn(-2.0, x_log(s)), s)));
+            break;
+        }
+        double v = __dadd_rn(1.0, __dmul_rn(c, z));
+        if (v <= 0.0) continue;
+        v = __dmul_rn(__dmul_rn(v, v), v);
+        const double u = x_uniform(sm64(key + t));
+        t += 1;
+        const double z2 = __dmul_rn(z, z);
+        if (u < __dsub_rn(1.0, __dmul_rn(__dmul_rn(0.0331, z2), z2)) ||
+            x_log(u) < __dadd_rn(__dmul_rn(0.5, z2), __dmul_rn(d, __dadd_rn(__dsub_rn(1.0, v), x_log(v))))) {
+            g = __dmul_rn(d, v);
+            break;
+        }
+    }
+    if (alpha < 1.0) g = __dmul_rn(g, x_exp(__ddiv_rn(x_log(x_uniform(sm64(key + t))), alpha)));
+    return g;
+}
+
+// Mixes Dirichlet(alpha) noise into the P row of root `h` (k >= 2 legal moves) and flags it (h->pad1 = 1); k = 1 is only
+// flagged.  Noise stream of the root position (own, opp) of game `base` = episode_key(seed, game id):
+//   rk = sm64(sm64(base ^ own) + opp); the j-th legal move (row-major) draws g_j = Gamma(alpha) from key sm64(rk + j)
+//   (its words sm64(sm64(rk + j) + t)).  S = (((g_0 + g_1) + g_2) + ...) in ascending j; eta_j = g_j / S (1/k if S = 0);
+//   P'_j = (1 - eps) * P_j + eps * eta_j.
+// Lane l draws moves l and l + 32.  A real call (see above): the sampler's code stays out of the descent loop.
+__device__ __noinline__ void root_noise_call(OzNodeHdr* h, int k, u64 base, double alpha, double eps, double* sa) {
+    const int lane = threadIdx.x & 31;
+    if (k > 1) {
+        const u64 rk = sm64(sm64(base ^ h->own) + h->opp);
+        for (int j = lane; j < k; j += 32) sa[j] = x_gamma(alpha, sm64(rk + (u64)j));
+        __syncwarp();
+        double s = sa[0];
+        for (int j = 1; j < k; ++j) s = __dadd_rn(s, sa[j]);
+        const double keep = __dsub_rn(1.0, eps);
+        double* Pp = node_P(h);
+        for (int j = lane; j < k; j += 32) {
+            const double eta = s > 0.0 ? __ddiv_rn(sa[j], s) : __ddiv_rn(1.0, (double)k);
+            Pp[j] = __dadd_rn(__dmul_rn(keep, Pp[j]), __dmul_rn(eps, eta));
+        }
+    }
+    if (lane == 0) h->pad1 = 1;
+    __syncwarp();
+}
+
+// Sampled opening move: the first child slot whose running visit sum (ascending slots) exceeds
+// u = pick_index(draw, sum of the visits); -1 when the root has no visits.  Warp-collective; a real call.
+__device__ __noinline__ int sample_move_call(const int* Np, int k, u64 draw) {
+    const int lane = threadIdx.x & 31;
+    int s0 = lane < k ? (Np[lane] & N_MASK) : 0;
+    int s1 = lane + 32 < k ? (Np[lane + 32] & N_MASK) : 0;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {  // inclusive prefix sums
+        const int a = __shfl_up_sync(FULLW, s0, o), b = __shfl_up_sync(FULLW, s1, o);
+        if (lane >= o) { s0 += a; s1 += b; }
+    }
+    s1 += __shfl_sync(FULLW, s0, 31);
+    const int total = __shfl_sync(FULLW, s1, 31);
+    if (total <= 0) return -1;
+    const u32 u = pick_index(draw, (u32)total);
+    const unsigned b0 = __ballot_sync(FULLW, lane < k && (u32)s0 > u);
+    if (b0) return __ffs(b0) - 1;
+    return 31 + __ffs(__ballot_sync(FULLW, lane + 32 < k && (u32)s1 > u));
+}
+
 // The engine step.  Every warp: (1) finishes the simulations that were waiting for their leaves, (2) keeps simulating
 // until it needs another network evaluation or runs out of work.
 //
@@ -474,7 +620,8 @@ __device__ __noinline__ u64 solve_leaf_call(u64 own, u64 opp, u64 legal, u64 ful
 #ifndef OZ_TREE_MIN_CTAS
 #define OZ_TREE_MIN_CTAS 7
 #endif
-template <int RULES, int SCORING, int VALUES>
+// EXPLORE = 1 (root noise or sampled opening moves requested): the two hooks below; EXPLORE = 0 compiles neither.
+template <int RULES, int SCORING, int VALUES, int EXPLORE>
 __global__ void __launch_bounds__(TREE_WARPS * 32, OZ_TREE_MIN_CTAS) tree_step_kernel(const OzTreeParams P) {
     __shared__ double s_a[TREE_WARPS][72];  // [0,64): masked priors of the node being expanded, [64,72): its partial sums
     const int lane = threadIdx.x & 31;
@@ -598,7 +745,14 @@ __global__ void __launch_bounds__(TREE_WARPS * 32, OZ_TREE_MIN_CTAS) tree_step_k
                 warp_argmax(best, bj);
                 const u64 base = episode_key(P.seed, P.game_id[slot]);
                 int aj = bj;
-                if (P.temperature == 0.0) {
+                bool sampled = false;
+                if constexpr (EXPLORE) {  // an opening ply: the move is drawn in proportion to the visit counts
+                    if (ply < P.sample_moves) {
+                        const int sj = sample_move_call(Np, k, episode_draw(base, ply, DRAW_SAMPLE_MOVE));
+                        if (sj >= 0) { aj = sj; sampled = true; }
+                    }
+                }
+                if (P.temperature == 0.0 && !sampled) {
                     // othelo_mcts.py:54-62: the policy is one-hot on random.choice(arg-max set); a unique maximum needs no
                     // draw, ties are broken by the game's counter RNG over the tied actions in row-major order
                     const unsigned t0 = __ballot_sync(FULLW, lane < k && (double)(Np[lane] & N_MASK) == best);
@@ -682,6 +836,11 @@ __global__ void __launch_bounds__(TREE_WARPS * 32, OZ_TREE_MIN_CTAS) tree_step_k
 
             // ---- one simulation: MCTS.simulate from the canonical root (othelo_mcts.py:22-26) -----------
             int node = P.root_node[slot];
+            if constexpr (EXPLORE) {  // a root's first descent: mix its Dirichlet noise in (once per node)
+                if (node >= 0 && P.dir_alpha > 0.0 && ld_i32(&node_at(arena, ref_off(node))->pad1) == 0)
+                    root_noise_call(node_at(arena, ref_off(node)), ref_k(node), episode_key(P.seed, P.game_id[slot]),
+                                    P.dir_alpha, P.dir_fraction, sa);
+            }
             int depth = 0;
             int outcome = 0;  // 1 = terminal, 2 = leaf, 3 = ran into a leaf of this wave
             int term_val = 0;
@@ -1006,6 +1165,8 @@ int oz_tree_alloc(oz_engine* e) {
     P.next_game = P.n_active + 1;
     P.solve_counters = P.counters + 8;
     P.solve_leaves = 0;
+    P.dir_alpha = P.dir_fraction = 0.0;
+    P.sample_moves = 0;
     oz_ordering_masks(P.n, &P.corners, &P.near_corners);
     P.total_games = 0;
     P.q_black = P.q_white = nullptr; P.q_player = nullptr; P.q_ids = nullptr;
@@ -1135,8 +1296,11 @@ int oz_tree_reset(oz_engine* e, int n_games, const u64* black, const u64* white,
         OZ_CUDA(cudaMemsetAsync(P.table, 0, ((size_t)n_games << P.table_log2) * sizeof(u64), e->stream));
         OZ_CUDA(cudaMemsetAsync(P.counters, 0, 10 * sizeof(u64), e->stream));
         OZ_CUDA(cudaMemsetAsync(P.leaf_count, 0, sizeof(int), e->stream));
-        e->values = e->values_req;  // oz_search_set_values is latched here (search reset / self-play begin)
+        e->values = e->values_req;  // oz_search_set_values is latched here (search reset / self-play begin) ...
         P.solve_leaves = e->solve_leaves_req;
+        P.dir_alpha = e->dir_alpha_req;  // ... and so is oz_search_set_exploration
+        P.dir_fraction = e->dir_fraction_req;
+        P.sample_moves = e->sample_moves_req;
     }
     P.G = n_games;
     tree_init_slots_kernel<<<(G + 255) / 256, 256, 0, e->stream>>>(P, n_games, d_b, d_w, d_p, d_id, clear ? 1 : 0);
@@ -1154,17 +1318,20 @@ int oz_tree_reset(oz_engine* e, int n_games, const u64* black, const u64* white,
 int oz_tree_step(oz_engine* e) {
     OzTreeParams& P = e->tp;
     int blocks = (P.G + TREE_WARPS - 1) / TREE_WARPS;
-    // one instantiation per (rule set, scoring, value convention): [rules][scoring][values]
-    static void (*const kernels[2][2][2])(const OzTreeParams) = {
-        {{tree_step_kernel<RULES_REFERENCE, SCORING_REFERENCE, VALUES_REFERENCE>,
-          tree_step_kernel<RULES_REFERENCE, SCORING_REFERENCE, VALUES_STANDARD>},
-         {tree_step_kernel<RULES_REFERENCE, SCORING_STANDARD, VALUES_REFERENCE>,
-          tree_step_kernel<RULES_REFERENCE, SCORING_STANDARD, VALUES_STANDARD>}},
-        {{tree_step_kernel<RULES_STANDARD, SCORING_REFERENCE, VALUES_REFERENCE>,
-          tree_step_kernel<RULES_STANDARD, SCORING_REFERENCE, VALUES_STANDARD>},
-         {tree_step_kernel<RULES_STANDARD, SCORING_STANDARD, VALUES_REFERENCE>,
-          tree_step_kernel<RULES_STANDARD, SCORING_STANDARD, VALUES_STANDARD>}}};
-    auto kernel = kernels[e->rules == RULES_STANDARD][e->scoring == SCORING_STANDARD][e->values == VALUES_STANDARD];
+    // one instantiation per (rule set, scoring, value convention, exploration): [rules][scoring][values][explore]
+#define OZ_TREE_X(R, S, V) {tree_step_kernel<R, S, V, 0>, tree_step_kernel<R, S, V, 1>}
+    static void (*const kernels[2][2][2][2])(const OzTreeParams) = {
+        {{OZ_TREE_X(RULES_REFERENCE, SCORING_REFERENCE, VALUES_REFERENCE),
+          OZ_TREE_X(RULES_REFERENCE, SCORING_REFERENCE, VALUES_STANDARD)},
+         {OZ_TREE_X(RULES_REFERENCE, SCORING_STANDARD, VALUES_REFERENCE),
+          OZ_TREE_X(RULES_REFERENCE, SCORING_STANDARD, VALUES_STANDARD)}},
+        {{OZ_TREE_X(RULES_STANDARD, SCORING_REFERENCE, VALUES_REFERENCE),
+          OZ_TREE_X(RULES_STANDARD, SCORING_REFERENCE, VALUES_STANDARD)},
+         {OZ_TREE_X(RULES_STANDARD, SCORING_STANDARD, VALUES_REFERENCE),
+          OZ_TREE_X(RULES_STANDARD, SCORING_STANDARD, VALUES_STANDARD)}}};
+#undef OZ_TREE_X
+    const bool explore = P.dir_alpha > 0.0 || P.sample_moves > 0;
+    auto kernel = kernels[e->rules == RULES_STANDARD][e->scoring == SCORING_STANDARD][e->values == VALUES_STANDARD][explore];
     kernel<<<blocks, TREE_WARPS * 32, 0, e->stream>>>(P);
     OZ_CUDA(cudaGetLastError());
     e->launches++;

@@ -8,7 +8,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import (PRIOR_HASH, PRIOR_HOST, PRIOR_NET, SCORINGS, SOLVE_MAX_EMPTIES, SOLVE_NONE, WINNER_DRAW, board_arg,
-                   channels_arg, check, f32p, f64p, i8p, i32p, ptr, u8p, u32p, u64p, values_arg)
+                   channels_arg, check, exploration_arg, f32p, f64p, i8p, i32p, ptr, u8p, u32p, u64p, values_arg)
 
 M64 = (1 << 64) - 1
 
@@ -137,20 +137,26 @@ class Engine:
     "reference" (default) negates a child's value at every ply, as the reference does; "standard" negates it only when
     the move swapped the side to move (a game-ending move is worth its own result, a value crossing a pass keeps its
     sign).  `solve_leaves` = K > 0 (values="standard" and scoring="standard" only) replaces the evaluation of every new
-    leaf below the root with at most K empties by the sign of its perfect-play margin (DESIGN.md 14)."""
+    leaf below the root with at most K empties by the sign of its perfect-play margin (DESIGN.md 14).
+    `dirichlet_alpha` = alpha > 0 mixes Dirichlet(alpha) noise into each root's priors once, with weight
+    `dirichlet_fraction`; `sample_moves` = M > 0 plays self-play's first M plies in proportion to the root visit counts
+    (no effect on the search API).  Both are off by default (DESIGN.md 15)."""
 
     def __init__(self, board_size: int = 8, max_games: int = 1, nodes_per_game: int = 8192,
                  prior_mode: int = PRIOR_HASH, c_puct: float = 1.0, seed: int = 0, device: int = 0,
                  log_visits: bool = False, eval_cache_log2: int = 0, vl_width: int = 1, rules: str = "reference",
-                 scoring: str = "reference", values: str = "reference", solve_leaves: int = 0):
+                 scoring: str = "reference", values: str = "reference", solve_leaves: int = 0,
+                 dirichlet_alpha: float = 0.0, dirichlet_fraction: float = 0.25, sample_moves: int = 0):
         bs = board_arg(board_size, rules, scoring)
         va = values_arg(values, solve_leaves, scoring)
+        xa = exploration_arg(dirichlet_alpha, dirichlet_fraction, sample_moves)
         self._L = _lib.load()
         self.board_size = board_size
         self.rules = rules
         self.precision, self.channels = "bf16", 0  # of the loaded network (load_weights)
         self.scoring = scoring
         self.values, self.solve_leaves = values, solve_leaves
+        self.dirichlet_alpha, self.dirichlet_fraction, self.sample_moves = xa
         self.nsq = board_size * board_size
         self.max_games = max_games
         self.prior_mode = prior_mode
@@ -164,6 +170,7 @@ class Engine:
         check(self._L.oz_engine_create(C.byref(cfg), C.byref(h)))
         self._h = h
         check(self._L.oz_search_set_values(h, va, solve_leaves))
+        check(self._L.oz_search_set_exploration(h, *xa))
         self.n_games = self.n_slots = 0
 
     def close(self):

@@ -50,6 +50,9 @@ class IterationConfig:
     precision: str = "bf16"          # "fp8": self-play and arena nets evaluate conv3/conv4/fc1 in FP8 (training stays fp32)
     values: str = "reference"        # "standard": self-play and arena searches negate a value only when the side swapped
     solve_leaves: int = 0            # > 0: self-play and arena searches solve new leaves with <= this many empties exactly
+    dirichlet_alpha: float = 0.0     # > 0: self-play roots get Dirichlet(alpha) noise once (the arena never explores)
+    dirichlet_fraction: float = 0.25  # ... mixed in with this weight
+    sample_moves: int = 0            # > 0: self-play plays its first this many plies in proportion to the visit counts
 
 
 def unpack_rows(rows: np.ndarray):
@@ -129,9 +132,14 @@ class Trainer:
             sp = selfplay.SelfPlay(n, net_now, cfg.degree_exploration, max_games=min(int(ids.size), cfg.max_concurrent),
                                    num_simulations=cfg.num_simulations, device=self.local, seed=cfg.seed,
                                    rules=cfg.rules, scoring=cfg.scoring, values=cfg.values,
-                                   solve_leaves=cfg.solve_leaves)
+                                   solve_leaves=cfg.solve_leaves, dirichlet_alpha=cfg.dirichlet_alpha,
+                                   dirichlet_fraction=cfg.dirichlet_fraction, sample_moves=cfg.sample_moves)
             rec = sp.play(int(ids.size), cfg.temperature, cfg.e_greedy, game_ids=ids)
             info["selfplay_sims_this_rank"] = sp.engine.counters()["sims"]
+            # how many of this rank's games differ from every other (move sequences): 1 when every game is the same
+            # game (e_greedy = 1 without root exploration), up to the rank's game count
+            nm = np.asarray(rec["n_moves"]).astype(np.int64)
+            info["distinct_this_rank"] = len({rec["action"][g][:nm[g]].tobytes() for g in range(nm.size)})
             sp.close()
         timed("selfplay_s", t0)
         # ---- exact endgame targets: every rank relabels the positions of its own games ---------------------------------
@@ -194,8 +202,12 @@ class Trainer:
             s = torch.tensor([info.get("selfplay_sims_this_rank", 0)], dtype=torch.int64, device=dev)
             dist.all_reduce(s)
             info["selfplay_sims"] = int(s.item())
+            d = torch.tensor([info.get("distinct_this_rank", 0)], dtype=torch.int64, device=dev)
+            dist.all_reduce(d)
+            info["selfplay_distinct_games"] = int(d.item())
         else:
             info["selfplay_sims"] = info.get("selfplay_sims_this_rank", 0)
+            info["selfplay_distinct_games"] = info.get("distinct_this_rank", 0)
         solve = {}
         if cfg.solve_empties > 0:
             counts = info["solve_this_rank"]
@@ -209,7 +221,7 @@ class Trainer:
                     train_steps=cfg.epochs * ((arrays[0].shape[0] + cfg.batch_size - 1) // cfg.batch_size),
                     train_history=hist, arena_new_wins=wins, arena_draws=draws, arena_games=cfg.arena_games,
                     promoted=bool(promoted),
-                    selfplay_sims=info["selfplay_sims"],
+                    selfplay_sims=info["selfplay_sims"], selfplay_distinct_games=info["selfplay_distinct_games"],
                     selfplay_sims_per_s=info["selfplay_sims"] / max(phases["selfplay_s"], 1e-9), **solve)
 
 
@@ -222,7 +234,11 @@ def main(argv=None):
              "solve_leaves": "search: new leaves with <= K empties are solved exactly instead of evaluated by the "
                              "network (needs --values standard --scoring standard; targets unchanged)",
              "values": "search value backup: 'standard' negates a child's value only when the move swapped the side "
-                       "to move"}
+                       "to move",
+             "dirichlet_alpha": "self-play only: Dirichlet(alpha) noise mixed into each root's priors once (0: none)",
+             "dirichlet_fraction": "self-play only: the weight of the root noise, in [0, 1]",
+             "sample_moves": "self-play only: the first M plies are drawn in proportion to the root visit counts "
+                             "(the e_greedy coin still applies)"}
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     for f, v in asdict(IterationConfig()).items():
         ap.add_argument("--" + f.replace("_", "-"), type=type(v), default=v, help=helps.get(f),
@@ -232,9 +248,10 @@ def main(argv=None):
     from ._lib import SOLVE_MAX_EMPTIES
     if not 0 <= args.solve_empties <= SOLVE_MAX_EMPTIES:
         ap.error(f"--solve-empties must be in [0, {SOLVE_MAX_EMPTIES}] (got {args.solve_empties})")
-    from ._lib import values_arg
+    from ._lib import exploration_arg, values_arg
     try:
         values_arg(args.values, args.solve_leaves, args.scoring)
+        exploration_arg(args.dirichlet_alpha, args.dirichlet_fraction, args.sample_moves)
     except ValueError as err:
         ap.error(str(err))
     import torch

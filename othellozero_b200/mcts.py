@@ -16,7 +16,11 @@ Aliases ``search`` / ``getActionProb`` are the alpha-zero-general names used in 
 ``rules="standard"`` searches under standard Othello flipping instead of the reference's flip rule, and
 ``scoring="standard"`` values a drawn terminal as 0 instead of as a BLACK win.  ``values="standard"`` negates a child's
 value only when the move swapped the side to move, and ``solve_leaves=K`` (with standard values and scoring) solves new
-leaves with at most K empties exactly (``engine.Engine``).
+leaves with at most K empties exactly (``engine.Engine``).  ``dirichlet_alpha`` > 0 mixes Dirichlet noise into each
+root's priors once, with weight ``dirichlet_fraction`` (the root exploration of ``engine.Engine``).  The noise stream is
+keyed by (seed, game id, root position); by default every instance takes the process-wide OS-drawn seed and a game id
+nobody has used before (``selfplay.allocate_game_ids``), so a new instance per episode, as the reference's training loop
+builds them, explores differently every time.  Pass ``seed=`` and ``game_id=`` for a reproducible search.
 """
 from __future__ import annotations
 
@@ -40,7 +44,8 @@ class HashPriorNet:
 class OthelloMCTS:
     def __init__(self, board_size, neural_network, degree_exploration, nodes: int = 65536, device: int = 0,
                  rules: str = "reference", scoring: str = "reference", values: str = "reference",
-                 solve_leaves: int = 0):
+                 solve_leaves: int = 0, dirichlet_alpha: float = 0.0, dirichlet_fraction: float = 0.25,
+                 seed: int | None = None, game_id: int | None = None):
         self._board_size = board_size
         self._neural_network = neural_network
         self.degree_explorarion = degree_exploration  # (sic) MCTS/__init__.py:27
@@ -54,13 +59,17 @@ class OthelloMCTS:
         else:
             mode = _e.PRIOR_HOST
         self._mode = mode
+        from . import selfplay  # the process-wide seed and game-id allocator (selfplay imports this module)
+        self.seed = selfplay._PROCESS_SEED if seed is None else int(seed)
+        self.game_id = int(selfplay.allocate_game_ids(1)[0]) if game_id is None else int(game_id)
         self._eng = _e.Engine(board_size, max_games=1, nodes_per_game=nodes, prior_mode=mode,
-                              c_puct=float(degree_exploration), device=device, rules=rules, scoring=scoring,
-                              values=values, solve_leaves=solve_leaves)
+                              c_puct=float(degree_exploration), seed=self.seed, device=device, rules=rules,
+                              scoring=scoring, values=values, solve_leaves=solve_leaves,
+                              dirichlet_alpha=dirichlet_alpha, dirichlet_fraction=dirichlet_fraction)
         self._game = game_class(rules, scoring)
         if mode == _e.PRIOR_NET:
             self._eng.load_weights(neural_network.blob, neural_network.channels, neural_network.precision)
-        self._eng.reset(1)
+        self._eng.reset(1, game_ids=[self.game_id])
         self._root = None
 
     # -- helpers ------------------------------------------------------------------------------------

@@ -13,7 +13,9 @@ and ``scoring="reference"`` (a draw counts as a BLACK win) or ``scoring="standar
 z = 0 for every example of the game).  ``values="standard"`` backs search values up with the standard sign (a child's
 value is negated only when the move swapped the side to move), and ``solve_leaves=K`` (standard values and scoring only)
 solves the search's new leaves with at most K empties exactly; this changes the search, not the targets, and composes
-with ``solve_empties``, which relabels the targets.
+with ``solve_empties``, which relabels the targets.  ``dirichlet_alpha`` > 0 mixes Dirichlet noise into each root's
+priors once (weight ``dirichlet_fraction``), and ``sample_moves=M`` plays each game's first M plies in proportion to
+the root visit counts (the e_greedy coin still applies); both are off by default (``engine.Engine``).
 """
 from __future__ import annotations
 
@@ -54,7 +56,8 @@ class SelfPlay:
     def __init__(self, board_size: int, neural_network, degree_exploration: float = 1.0, max_games: int = 4096,
                  num_simulations: int = 100, device: int = 0, seed: int = 0, log_visits: bool = False,
                  eval_cache_log2: int = 22, rules: str = "reference", scoring: str = "reference",
-                 values: str = "reference", solve_leaves: int = 0):
+                 values: str = "reference", solve_leaves: int = 0, dirichlet_alpha: float = 0.0,
+                 dirichlet_fraction: float = 0.25, sample_moves: int = 0):
         self.board_size = board_size
         self.num_simulations = num_simulations
         if isinstance(neural_network, HashPriorNet):
@@ -70,7 +73,9 @@ class SelfPlay:
                                 # identical positions reached by different games are evaluated once (results unchanged:
                                 # tests/test_gpu_net.py::test_eval_cache_is_results_preserving); 272 B per entry
                                 eval_cache_log2=eval_cache_log2 if mode == _e.PRIOR_NET else 0, rules=rules,
-                                scoring=scoring, values=values, solve_leaves=solve_leaves)
+                                scoring=scoring, values=values, solve_leaves=solve_leaves,
+                                dirichlet_alpha=dirichlet_alpha, dirichlet_fraction=dirichlet_fraction,
+                                sample_moves=sample_moves)
         if mode == _e.PRIOR_NET:
             self.engine.load_weights(neural_network.blob, neural_network.channels, neural_network.precision)
 
@@ -216,14 +221,17 @@ def allocate_game_ids(n: int) -> np.ndarray:
 def execute_episodes(n_episodes, board_size, neural_network, degree_exploration, num_simulations, policy_temperature,
                      e_greedy, device: int = 0, seed: int | None = None, reference_aliasing: bool = False, game_ids=None,
                      max_concurrent: int = 4096, rules: str = "reference", scoring: str = "reference",
-                     solve_empties: int = 0, values: str = "reference", solve_leaves: int = 0):
+                     solve_empties: int = 0, values: str = "reference", solve_leaves: int = 0,
+                     dirichlet_alpha: float = 0.0, dirichlet_fraction: float = 0.25, sample_moves: int = 0):
     """n_episodes x training.execute_episode as one GPU job; returns a list of example lists.  At most `max_concurrent`
     episodes are in flight (node pools are per slot); the others are queued on the device and start as slots free up.
     policy_temperature may be 0 (main.py:73-76 switches to it after `temperature_threshold` iterations).
     solve_empties > 0: the target z of every position with at most that many empties comes from the winner under perfect
     play (solve_record_winners), not from the game's outcome; not available with reference_aliasing.
-    values / solve_leaves: the search's value convention and leaf solving (Engine)."""
+    values / solve_leaves: the search's value convention and leaf solving (Engine).
+    dirichlet_alpha / dirichlet_fraction / sample_moves: root noise and sampled opening moves (Engine)."""
     _e.values_arg(values, solve_leaves, scoring)
+    _e.exploration_arg(dirichlet_alpha, dirichlet_fraction, sample_moves)
     if solve_empties and reference_aliasing:
         raise ValueError("solve_empties > 0 needs per-position targets, which reference_aliasing=True does not have")
     if seed is None:
@@ -232,7 +240,8 @@ def execute_episodes(n_episodes, board_size, neural_network, degree_exploration,
         game_ids = allocate_game_ids(n_episodes)
     sp = SelfPlay(board_size, neural_network, degree_exploration, max_games=min(n_episodes, max_concurrent),
                   num_simulations=num_simulations, device=device, seed=seed, rules=rules, scoring=scoring,
-                  values=values, solve_leaves=solve_leaves)
+                  values=values, solve_leaves=solve_leaves, dirichlet_alpha=dirichlet_alpha,
+                  dirichlet_fraction=dirichlet_fraction, sample_moves=sample_moves)
     try:
         rec = sp.play(n_episodes, policy_temperature, e_greedy, game_ids=game_ids)
     finally:
@@ -284,14 +293,19 @@ class Worker:
 
 
 def make_b200_worker(worker_base=Worker, device: int = 0, seed: int | None = None, rules: str = "reference",
-                     scoring: str = "reference", values: str = "reference", solve_leaves: int = 0):
+                     scoring: str = "reference", values: str = "reference", solve_leaves: int = 0,
+                     dirichlet_alpha: float = 0.0, dirichlet_fraction: float = 0.25, sample_moves: int = 0):
     """Builds a ``B200Worker`` class deriving from ``worker_base`` — pass the reference's ``workers.Worker`` so that
     ``WorkerManager.add_worker``'s isinstance check (workers.py:186-190) accepts it.  seed=None (default): the
     process-wide OS-drawn seed; game ids always come from the process-wide allocator, so every run() of every worker
     plays episodes nobody has played before (see allocate_game_ids).  ``rules``, ``scoring``, ``values`` and
-    ``solve_leaves`` are the rule set, the scoring and the search values of every work type."""
+    ``solve_leaves`` are the rule set, the scoring and the search values of every work type.  ``dirichlet_alpha``,
+    ``dirichlet_fraction`` and ``sample_moves`` (root exploration) apply to episode work only: duels and evaluations
+    never explore."""
     _e.board_arg(8, rules, scoring)  # unknown rule sets / scorings / values fail here, not in the worker thread
     _e.values_arg(values, solve_leaves, scoring)
+    explore_kw = dict(zip(("dirichlet_alpha", "dirichlet_fraction", "sample_moves"),
+                          _e.exploration_arg(dirichlet_alpha, dirichlet_fraction, sample_moves)))
 
     class B200Worker(worker_base):
         def __init__(self):
@@ -301,6 +315,7 @@ def make_b200_worker(worker_base=Worker, device: int = 0, seed: int | None = Non
             self.rules = rules
             self.scoring = scoring
             self.search_kw = dict(values=values, solve_leaves=solve_leaves)
+            self.explore_kw = explore_kw  # episode work only
 
         def _run(self, work_type, iterations, args, kwargs):
             # workers.py:57-65 runs the target once per iteration; here all iterations are one GPU batch and
@@ -310,7 +325,7 @@ def make_b200_worker(worker_base=Worker, device: int = 0, seed: int | None = Non
             if work_type == WorkType.EXECUTE_EPISODE:
                 logging.info(f'Task {work_type}: {iterations} episodes as one GPU job on cuda:{self.device}')
                 results = execute_episodes(iterations, *args, device=self.device, seed=self.seed, rules=self.rules,
-                                           scoring=self.scoring, **self.search_kw, **kwargs)
+                                           scoring=self.scoring, **self.search_kw, **self.explore_kw, **kwargs)
             elif work_type == WorkType.DUEL_BETWEEN_NEURAL_NETWORKS:
                 from . import arena
                 logging.info(f'Task {work_type}: {iterations} duels as one GPU batch on cuda:{self.device}')
@@ -328,7 +343,7 @@ def make_b200_worker(worker_base=Worker, device: int = 0, seed: int | None = Non
 
         def execute_episode(self, *args, **kwargs):
             return execute_episode(*args, device=self.device, seed=self.seed, rules=self.rules, scoring=self.scoring,
-                                   **self.search_kw, **kwargs)
+                                   **self.search_kw, **self.explore_kw, **kwargs)
 
         def duel_between_neural_networks(self, *args, **kwargs):
             from . import arena

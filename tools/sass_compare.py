@@ -6,7 +6,9 @@ bf16 one (OUT_BF16 of conv2_table_gather_kernel); a lone `<0>` is the reference-
 or the bf16 SM-pair GEMM (OP_BF16).  So a kernel that became `template <int RULES>` or `template <int OP>` is compared with
 its pre-template self, `tree_step_kernel<R, 0>` with `tree_step_kernel<R>` and `conv2_table_gather_kernel<NJ, W, X, 0>`
 with `conv2_table_gather_kernel<NJ, W, X>`.  Before that, the reference-values tree kernel `tree_step_kernel<R, S, 0>`
-(VALUES_REFERENCE) becomes `tree_step_kernel<R, S>`, its name before the value convention was a template argument.
+(VALUES_REFERENCE) becomes `tree_step_kernel<R, S>`, its name before the value convention was a template argument, and
+before that the non-exploring tree kernel `tree_step_kernel<R, S, V, 0>` becomes `tree_step_kernel<R, S, V>`, its name
+before root exploration was a template argument.
 Every instantiation of a listed kernel that
 the OLD build has is compared.  Instruction addresses and encodings are ignored; branch and call targets are offsets
 inside the kernel's own section, so identical code gives identical text.  Needs cuobjdump and c++filt, no GPU.
@@ -44,6 +46,7 @@ def functions(so: str) -> dict[str, list[str]]:
 
 def normalize(demangled: str) -> str:
     s = re.sub(r"^void ", "", demangled).replace("(anonymous namespace)::", "")  # oz_net.cu's kernels
+    s = re.sub(r"^(tree_step_kernel<\d+, \d+, \d+), 0>\(", r"\1>(", s)  # the non-exploring tree kernel
     s = re.sub(r"^(tree_step_kernel<\d+, \d+), 0>\(", r"\1>(", s)  # the reference-values tree kernel
     s = re.sub(r", 0>\(", ">(", s)
     return s.replace("<0>(", "(")
